@@ -1,7 +1,7 @@
 #!/usr/bin/env python3
 """bench.py -- headline benchmark of the raytrace path.
 
-    python bench.py --gpus N --steps K --warmup W [--impl reference] [--config 2] [--extra auto|none|3,5,4]
+    python bench.py --gpus N --steps K --warmup W [--impl reference] [--config 2] [--extra auto|none|3,5,4] [--dump-outputs DIR]
 
 One "step" = one pass of the hot path over one frame of the BASELINE.json config-2 workload (6x6 tessellated-sphere grid
 + floor = 101 090 triangles, 1920x1080, 1 light, primary + shadow + 1 diffuse bounce, 1 sample/pixel): every pixel-sample
@@ -26,6 +26,11 @@ One "step" = one pass of the hot path over one frame of the BASELINE.json config
   cpu_baseline  the reference's own C build of the kernel (oracle/_ref, "reference") or the C port ("port") on the host
              cores, on a bounded sample of rows of the same frame; plus RaytraceAll(0, ...) as shipped (1 thread).
 
+--dump-outputs DIR writes the three 16-bit planes the timed path produced in its last timed step as DIR/r.npy, g.npy, b.npy
+(float32, [rows, width]), so that two builds can be compared output for output: the workload is synthetic and seeded, the same
+arguments give the same inputs.  A frame larger than DUMP_LIMIT_BYTES in float32 keeps every k-th row; the rows kept go to
+DIR/rows.npy.
+
 N > 1 (launched by torchrun, one process per GPU): the frame is cut into row bands dealt round-robin to the ranks, the
 scene is replicated, and the planes are assembled by peer stores over NVLink (the path's only exchange step).
 """
@@ -46,6 +51,7 @@ import numpy as np  # noqa: E402
 
 HBM_FALLBACK_GBS = 6650.0     # B200_PROFILING.md fallback when MEASURED_PEAKS.json is absent
 ROW_STEP = 4                  # CPU arms: every 4th row of the WHOLE frame (a quarter of the work, sky and geometry in proportion)
+DUMP_LIMIT_BYTES = 64_000_000  # --dump-outputs: all files together
 
 
 def parse():
@@ -58,6 +64,8 @@ def parse():
     ap.add_argument("--variant", type=int, default=-1)
     ap.add_argument("--band-rows", type=int, default=16)
     ap.add_argument("--extra", default="auto", help="other configs measured into `configs`: auto (3, 5; 4 at 8 GPUs), none, or a list")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the planes of the last timed step of the headline config to DIR/{r,g,b}.npy (float32)")
     return ap.parse_args()
 
 
@@ -99,6 +107,20 @@ def algorithmic_bytes(cnt: dict, rays: int) -> float:
     grid_candidates = cnt["gridCandidates"] + cnt.get("mailboxSkips", 0)     # the reference tests these again in every cell
     return (8.0 * rays + 68.0 * cnt["primCandidates"] + 8.0 * cnt["cells"] + 68.0 * grid_candidates + 212.0 * cnt["shadedHits"] +
             44.0 * cnt["occluderLookups"] + 12.0 * rays)
+
+
+def dump_outputs(out_dir, planes):
+    """--dump-outputs: the uint16 planes (r, g, b) as float32 .npy files, every k-th row when the whole frame exceeds the limit."""
+    h, w = planes[0].shape
+    step = 1
+    while 3 * len(range(0, h, step)) * w * 4 > DUMP_LIMIT_BYTES:
+        step += 1
+    rows = np.arange(0, h, step)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, plane in zip("rgb", planes):
+        np.save(os.path.join(out_dir, f"{name}.npy"), plane[rows].astype(np.float32))
+    if step > 1:
+        np.save(os.path.join(out_dir, "rows.npy"), rows.astype(np.float64))
 
 
 def hbm_peak():
@@ -325,6 +347,8 @@ def measure_config(run: Run, cfg_id: int, steps: int, warmup: int, primary: bool
             launches += n
         torch.cuda.synchronize()
     run.barrier()
+    if primary and args.dump_outputs and rank == 0:      # before anything below renders into the frame again
+        dump_outputs(args.dump_outputs, assembled.cpu().numpy().view(np.uint16) if world > 1 else fr.read())
     ms_total, ms_render = run.max_over_ranks([sum(a.elapsed_time(b) for a, b, _ in events), sum(a.elapsed_time(c) for a, _, c in events)])
     ms_step = ms_total / steps
     res = {"workload": cfg["name"], "triangles": int(sc.triangle_count), "width": w, "height": h, "samples": S,

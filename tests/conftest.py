@@ -36,16 +36,6 @@ def pytest_collection_modifyitems(config, items):
 
 
 @pytest.fixture(scope="session")
-def ref():
-    """The unmodified reference, compiled by oracle/build_ref.py (prebuilt .so on the GPU box)."""
-    import ref as _ref
-    if not _ref.available():
-        pytest.skip("oracle/_ref not built and /root/reference absent")
-    _ref.load()
-    return _ref
-
-
-@pytest.fixture(scope="session")
 def port():
     import port as _port
     _port.load()

@@ -1,7 +1,7 @@
 /* helpers_kat.c -- test driver (not product code): calls the eight host helpers of source/opencl/raytrace.h:37-44 in the shared
  * library given on the command line -- by value, through include/oclr_abi.h's types -- on a fixed pseudo-random + boundary input
  * set and writes every result to stdout as raw 32-bit words.  tests/test_abi_c.py runs it against libopencl_render_b200.so and
- * against the reference build (oracle/_ref) and compares the two streams. */
+ * compares the stream with the reference build's, stored in tests/golden/reference_values.json. */
 #include <dlfcn.h>
 #include <math.h>
 #include <stdint.h>
