@@ -337,6 +337,44 @@ void oclr_frame_device_planes(oclr_frame* frame, void** red, void** green, void*
  * One kernel on cudaStream; the caller orders a cross-GPU barrier behind it.  The reference has no counterpart (one device). */
 int oclr_frame_push_rows(oclr_frame* frame, cl_uint bandRows, int rank, int worldSize, void* const* peerPlanes, void* cudaStream);
 
+/* Batched ray queries on a resident scene, with the reference's own semantics.  The reference has no such door: its only caller of
+ * RayIntersectsTriangles is the Raytrace kernel.  A query runs on the scene's device.
+ *
+ * Rays: origin4[i] = (ox, oy, oz, minD), direction4[i] = (dx, dy, dz, maxD) -- the reference's cl_float3 layout with the range in the
+ * unused 4th component.  The direction is not normalised: t is in its units.  `excluded` = cl_uint[count] (the triangle the ray
+ * starts on, RayIntersectsTriangles' `excludeTriangle`), or NULL = 0xFFFFFFFF for every ray.  The caller's input arrays are never
+ * written.  count == 0 is accepted.
+ *
+ * oclr_scene_intersect: RayIntersectsTriangles (raytrace_opencl.c:324-401) exactly.  The first grid cell along the ray that holds any
+ * hit with minD < t < maxD wins; inside it the smallest t, and on equal t the earliest entry of the cell's list.
+ *   hit4[i] = (as_float(triangle), t, abL, acL); a miss is (as_float(0xFFFFFFFF), maxD, 0, 0).
+ * oclr_scene_transmittance: the shadow loop of raytrace_opencl.c:608-627.  att = (1,1,1); closest hit with the same excluded triangle;
+ * at each blocker att *= its TRANSPARENCY texel at (abL, acL) (0 without that channel) and the query continues from minD = t while all
+ * three components are > 0 -- the loop stops as soon as ANY component reaches 0 and the others are returned as they are.
+ *   att4[i] = (r, g, b, as_float(last triangle met, or 0xFFFFFFFF)).
+ *
+ * Preconditions.  The trace kernel orders the hits of a ray by the bit pattern of t, which requires t > 0 and so minD >= 0 (-0.0 is
+ * allowed).  A ray with minD < 0, a NaN minD or maxD, or a non-finite origin or direction component is NOT traced: its result is
+ * (0xFFFFFFFF, NaN, 0, 0), transmittance (NaN, NaN, NaN, 0xFFFFFFFF).  A real miss never has a NaN t.  A ray with !(minD < maxD) or a
+ * zero direction is not traced either; no t can pass minD < t < maxD, so it gets the ordinary miss (0xFFFFFFFF, maxD, 0, 0) and att
+ * (1, 1, 1).
+ *
+ * memory: OCLR_QUERY_HOST_MEMORY -- host arrays, staged through the library (the call synchronises).  OCLR_QUERY_DEVICE_MEMORY --
+ * device memory of the scene's device; origin4 / direction4 / hit4 / att4 16-byte aligned, excluded 4-byte aligned; any other pointer
+ * fails the call with a message.  Inputs are read in place.
+ * Rays are processed in internal batches of 2^21 (2 097 152); scratch is allocated per call, stream-ordered on cudaStream (up to about
+ * 190 MB for closest hit, 270 MB for transmittance, plus 110 MB of staging for host memory), so queries on one scene from different
+ * streams share no state.
+ * `stats` as in oclr_frame_render: NULL = no synchronisation for a device-memory closest-hit query; host-memory queries and transmittance
+ * always synchronise (the loop reads its ray count back once per chunk of rounds).  stats->deviceMs is the whole call;
+ * stats->traceLaunches the trace rounds enqueued; with countEvents, counters.gridRays counts every closest-hit trace (transmittance: of
+ * every round).  Returns 1 on success. */
+enum { OCLR_QUERY_HOST_MEMORY = 0, OCLR_QUERY_DEVICE_MEMORY = 1 };
+int oclr_scene_intersect(oclr_scene* scene, size_t count, const cl_float* origin4, const cl_float* direction4, const cl_uint* excluded,
+                         cl_float* hit4, int memory, int countEvents, void* cudaStream, oclr_render_stats* stats);
+int oclr_scene_transmittance(oclr_scene* scene, size_t count, const cl_float* origin4, const cl_float* direction4, const cl_uint* excluded,
+                             cl_float* att4, int memory, int countEvents, void* cudaStream, oclr_render_stats* stats);
+
 /* Rows of a W x H image owned by `rank` of `worldSize` when the image is cut into bands of `bandRows` rows dealt
  * round-robin (SURVEY.md section 8e; band height 128 = the reference's tile height, raytrace.c:507).  Writes up to
  * `maxBands` [begin,end) pairs to `rows` and returns the number of bands owned. */

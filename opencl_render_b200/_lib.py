@@ -80,6 +80,8 @@ EXPORTS = [
     "oclr_frame_render_samples", "oclr_frame_render_bands_samples", "oclr_frame_write", "oclr_frame_set_accumulation", "oclr_frame_read_accum",
     "oclr_frame_write_accum", "oclr_frame_progress", "oclr_estimated_seconds_left", "oclr_write_bmp", "oclr_write_ppm16", "oclr_write_png16",
     "oclr_set_option", "oclr_frame_push_rows",
+    # batched ray queries on a resident scene
+    "oclr_scene_intersect", "oclr_scene_transmittance",
 ]
 
 _lib = None
@@ -182,6 +184,10 @@ def load() -> C.CDLL:
     lib.oclr_write_bmp.argtypes = [C.c_char_p, C.c_uint32, C.c_uint32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int]
     lib.oclr_frame_push_rows.restype = C.c_int
     lib.oclr_frame_push_rows.argtypes = [C.c_void_p, C.c_uint32, C.c_int, C.c_int, C.POINTER(C.c_void_p), C.c_void_p]
+    for name in ("oclr_scene_intersect", "oclr_scene_transmittance"):
+        getattr(lib, name).restype = C.c_int
+        getattr(lib, name).argtypes = [C.c_void_p, C.c_size_t, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_void_p,
+                                       C.POINTER(RenderStats)]
     lib.oclr_set_option.restype = C.c_int
     lib.oclr_set_option.argtypes = [C.c_char_p, C.c_int]
     lib.InitOpenCL.restype = None

@@ -24,6 +24,8 @@ LIGHT_OMNI, LIGHT_SPOT, LIGHT_SPOTRECT, LIGHT_DISTANT, LIGHT_PARALLEL, LIGHT_PAR
 KERNEL_SIMPLE, KERNEL_PIPE, KERNEL_DEFAULT = 0, 2, -1
 ACCUMULATE_REFERENCE_16BIT, ACCUMULATE_FLOAT = 0, 1
 NO_TRIANGLE = 0xFFFFFFFF
+QUERY_HOST_MEMORY, QUERY_DEVICE_MEMORY = 0, 1
+QUERY_BATCH = 1 << 21        # rays per internal batch of a query (runtime.h kQueryBatch)
 
 
 class OclrError(RuntimeError):
@@ -281,6 +283,72 @@ class DeviceScene:
         self._lib.oclr_scene_debug_read(self.handle, which, _ptr(out), n)
         return out[:n]
 
+    def intersect(self, origins, directions, t_min=None, t_max=None, exclude=None, stream=None, count: bool = False):
+        """Closest hit of every ray, RayIntersectsTriangles exactly (raytrace_opencl.c:324-401; semantics and preconditions in
+        include/oclr_abi.h).  origins / directions: [N,3], or [N,4] with minD / maxD in column 3; t_min / t_max (scalars or [N]) give the
+        range of [N,3] rays (default 0 and +inf) and may not be combined with [N,4] inputs; exclude: [N] triangle ids or None.
+        numpy inputs run through host memory and return numpy; CUDA torch tensors on the scene's device run in place (contiguous [N,4]
+        float32 inputs are not copied) on `stream` (torch stream or cudaStream_t handle; default: torch's current stream) and return
+        tensors.  Returns (ids uint32[N], t float32[N], abL float32[N], acL float32[N]) -- a miss is (NO_TRIANGLE, maxD, 0, 0), a ray
+        that breaks the preconditions (minD < 0, NaN range, non-finite component) (NO_TRIANGLE, NaN, 0, 0) -- plus the counters dict
+        when count=True."""
+        out, cnt = self._query("oclr_scene_intersect", origins, directions, t_min, t_max, exclude, stream, count)
+        res = (self._ids(out[:, 0]), out[:, 1], out[:, 2], out[:, 3])
+        return res + (cnt,) if count else res
+
+    def transmittance(self, origins, directions, t_min=None, t_max=None, exclude=None, stream=None, count: bool = False):
+        """Transmittance along every ray: the shadow loop of raytrace_opencl.c:608-627 (att starts at (1,1,1) and is multiplied by the
+        TRANSPARENCY texel of each blocker, 0 without that channel, until a component reaches 0 or the ray is clear).  Arguments as in
+        intersect().  Returns (att float32[N,3], last blocker uint32[N] or NO_TRIANGLE) (+ counters dict when count=True)."""
+        out, cnt = self._query("oclr_scene_transmittance", origins, directions, t_min, t_max, exclude, stream, count)
+        res = (out[:, :3], self._ids(out[:, 3]))
+        return res + (cnt,) if count else res
+
+    @staticmethod
+    def _ids(col):
+        if isinstance(col, np.ndarray):
+            return np.ascontiguousarray(col).view(np.uint32)
+        import torch
+        return col.contiguous().view(torch.uint32)
+
+    def _query(self, entry, origins, directions, t_min, t_max, exclude, stream, count):
+        torch = _torch_if_tensor(origins)
+        if torch is None:
+            o, d, ex = _query_rays_numpy(origins, directions, t_min, t_max, exclude)
+            out = np.empty((o.shape[0], 4), np.float32)
+            stats = _lib.RenderStats()
+            if not getattr(self._lib, entry)(self.handle, o.shape[0], _ptr(o), _ptr(d), _ptr(ex), _ptr(out), QUERY_HOST_MEMORY,
+                                              1 if count else 0, None, C.byref(stats) if count else None):
+                raise OclrError(_lib.last_error())
+            return out, (stats.counters.as_dict() if count else None)
+        dev = torch.device("cuda", self.device)
+        for name, a in (("origins", origins), ("directions", directions), ("exclude", exclude), ("t_min", t_min), ("t_max", t_max)):
+            if isinstance(a, torch.Tensor) and a.device != dev:
+                raise ValueError(f"{name} is on {a.device}, the scene is on {dev}")
+            if isinstance(a, np.ndarray) and a.ndim > 0:
+                raise ValueError(f"{name} is a numpy array: a query takes numpy or torch inputs, not both")
+        if isinstance(stream, torch.cuda.Stream):
+            ts = stream
+        elif stream:
+            ts = torch.cuda.ExternalStream(int(stream), device=dev)
+        else:
+            ts = torch.cuda.current_stream(dev)
+        with torch.cuda.device(dev), torch.cuda.stream(ts):
+            o, d, ex = _query_rays_torch(torch, dev, origins, directions, t_min, t_max, exclude)
+            out = torch.empty((o.shape[0], 4), dtype=torch.float32, device=dev)
+            stats = _lib.RenderStats()
+            sync = count
+            if not getattr(self._lib, entry)(self.handle, o.shape[0], C.c_void_p(o.data_ptr()), C.c_void_p(d.data_ptr()),
+                                              C.c_void_p(ex.data_ptr()) if ex is not None else None, C.c_void_p(out.data_ptr()),
+                                              QUERY_DEVICE_MEMORY, 1 if count else 0, C.c_void_p(ts.cuda_stream),
+                                              C.byref(stats) if sync else None):
+                raise OclrError(_lib.last_error())
+        cur = torch.cuda.current_stream(dev)
+        if cur != ts:   # results are used on the caller's current stream
+            cur.wait_stream(ts)
+            out.record_stream(cur)
+        return out, (stats.counters.as_dict() if count else None)
+
     def close(self):
         if getattr(self, "handle", None):
             self._lib.oclr_scene_destroy(self.handle)
@@ -288,6 +356,99 @@ class DeviceScene:
 
     def __del__(self):
         self.close()
+
+
+def _torch_if_tensor(a):
+    """The torch module when `a` is a torch tensor (torch is imported only then), else None."""
+    mod = type(a).__module__
+    if mod.startswith("torch"):
+        import torch
+        if isinstance(a, torch.Tensor):
+            if not a.is_cuda:
+                raise ValueError("torch inputs of a query must be CUDA tensors (numpy arrays take the host path)")
+            return torch
+    return None
+
+
+def _ray_shape(name, shape):
+    if len(shape) != 2 or shape[1] not in (3, 4):
+        raise ValueError(f"{name} must be [N,3] or [N,4], got {tuple(shape)}")
+
+
+def _query_range(name, v, n):
+    a = np.asarray(v)
+    if a.dtype.kind not in "fiu" or (a.ndim != 0 and a.shape != (n,)):
+        raise ValueError(f"{name} must be a real scalar or [N={n}] array, got {a.dtype} {a.shape}")
+    return a
+
+
+def _query_rays_numpy(origins, directions, t_min, t_max, exclude):
+    """Validated contiguous (origin4, direction4, excluded | None) host arrays."""
+    o, d = np.asarray(origins), np.asarray(directions)
+    for name, a in (("origins", o), ("directions", d)):
+        _ray_shape(name, a.shape)
+        if a.dtype.kind != "f":
+            raise ValueError(f"{name} must be floating point, got {a.dtype}")
+    n = o.shape[0]
+    if d.shape[0] != n:
+        raise ValueError(f"origins has {n} rays, directions {d.shape[0]}")
+    rays = []
+    for name, a, rng, dflt in (("origins", o, t_min, 0.0), ("directions", d, t_max, np.inf)):
+        if a.shape[1] == 4:
+            if rng is not None:
+                raise ValueError(f"{name} is [N,4] (range in column 3): {'t_min' if dflt == 0.0 else 't_max'} cannot be given too")
+            rays.append(np.ascontiguousarray(a, np.float32))
+        else:
+            r = _query_range("t_min" if dflt == 0.0 else "t_max", dflt if rng is None else rng, n)
+            a4 = np.empty((n, 4), np.float32)
+            a4[:, :3] = a
+            a4[:, 3] = r
+            rays.append(a4)
+    ex = None
+    if exclude is not None:
+        e = np.asarray(exclude)
+        if e.dtype.kind not in "iu" or e.shape != (n,):
+            raise ValueError(f"exclude must be an integer [N={n}] array, got {e.dtype} {e.shape}")
+        ex = np.ascontiguousarray(e.astype(np.int64) & 0xFFFFFFFF, np.uint32) if e.dtype != np.uint32 else np.ascontiguousarray(e)
+    return rays[0], rays[1], ex
+
+
+def _query_rays_torch(torch, dev, origins, directions, t_min, t_max, exclude):
+    """Validated contiguous (origin4, direction4, excluded | None) CUDA tensors; contiguous [N,4] float32 inputs are used as they are."""
+    if not isinstance(directions, torch.Tensor):
+        raise ValueError("directions must be a torch tensor like origins")
+    for name, a in (("origins", origins), ("directions", directions)):
+        _ray_shape(name, a.shape)
+        if not a.dtype.is_floating_point:
+            raise ValueError(f"{name} must be floating point, got {a.dtype}")
+    n = origins.shape[0]
+    if directions.shape[0] != n:
+        raise ValueError(f"origins has {n} rays, directions {directions.shape[0]}")
+    rays = []
+    for name, a, rng, dflt in (("origins", origins, t_min, 0.0), ("directions", directions, t_max, float("inf"))):
+        rname = "t_min" if dflt == 0.0 else "t_max"
+        if a.shape[1] == 4:
+            if rng is not None:
+                raise ValueError(f"{name} is [N,4] (range in column 3): {rname} cannot be given too")
+            rays.append(a.to(torch.float32).contiguous())
+        else:
+            rng = dflt if rng is None else rng
+            if isinstance(rng, torch.Tensor):
+                if rng.ndim != 0 and tuple(rng.shape) != (n,):
+                    raise ValueError(f"{rname} must be a scalar or [N={n}] tensor, got {tuple(rng.shape)}")
+            else:
+                rng = _query_range(rname, rng, n)
+                rng = float(rng) if rng.ndim == 0 else torch.as_tensor(rng, device=dev)
+            a4 = torch.empty((n, 4), dtype=torch.float32, device=dev)
+            a4[:, :3] = a
+            a4[:, 3] = rng
+            rays.append(a4)
+    ex = None
+    if exclude is not None:
+        if not isinstance(exclude, torch.Tensor) or exclude.dtype not in (torch.int32, torch.uint32, torch.int64) or tuple(exclude.shape) != (n,):
+            raise ValueError(f"exclude must be an int32 / uint32 / int64 [N={n}] CUDA tensor")
+        ex = exclude.contiguous() if exclude.dtype != torch.int64 else (exclude & 0xFFFFFFFF).to(torch.int32).contiguous()
+    return rays[0], rays[1], ex
 
 
 class DeviceFrame:

@@ -328,6 +328,40 @@ int oclr_frame_render(oclr_frame* frame, cl_uint sampleCount, cl_uint rowBegin, 
     return oclr_frame_render_samples(frame, sampleCount, 0, sampleCount, rowBegin, rowEnd, kernelVariant, countEvents, cudaStream, stats);
 }
 
+static int scene_query_entry(const char* name, bool transmit, oclr_scene* scene, size_t count, const cl_float* origin4, const cl_float* direction4,
+                             const cl_uint* excluded, cl_float* out4, int memory, int countEvents, void* cudaStream, oclr_render_stats* stats) {
+    if (!scene) {
+        fail(std::string(name) + ": null scene");
+        return 0;
+    }
+    if (memory != OCLR_QUERY_HOST_MEMORY && memory != OCLR_QUERY_DEVICE_MEMORY) {
+        fail(std::string(name) + ": unknown memory kind " + std::to_string(memory));
+        return 0;
+    }
+    std::string err;
+    RenderStats rs;
+    const bool dev = memory == OCLR_QUERY_DEVICE_MEMORY;
+    const bool ok = transmit ? scene_transmittance(scene->impl, count, origin4, direction4, excluded, out4, dev, countEvents != 0, cudaStream,
+                                                   stats ? &rs : nullptr, err)
+                             : scene_intersect(scene->impl, count, origin4, direction4, excluded, out4, dev, countEvents != 0, cudaStream,
+                                               stats ? &rs : nullptr, err);
+    if (!ok) {
+        fail(std::string(name) + ": " + err);
+        return 0;
+    }
+    if (stats) copy_stats(stats, rs);
+    return 1;
+}
+int oclr_scene_intersect(oclr_scene* scene, size_t count, const cl_float* origin4, const cl_float* direction4, const cl_uint* excluded,
+                         cl_float* hit4, int memory, int countEvents, void* cudaStream, oclr_render_stats* stats) {
+    return scene_query_entry("oclr_scene_intersect", false, scene, count, origin4, direction4, excluded, hit4, memory, countEvents, cudaStream, stats);
+}
+int oclr_scene_transmittance(oclr_scene* scene, size_t count, const cl_float* origin4, const cl_float* direction4, const cl_uint* excluded,
+                             cl_float* att4, int memory, int countEvents, void* cudaStream, oclr_render_stats* stats) {
+    return scene_query_entry("oclr_scene_transmittance", true, scene, count, origin4, direction4, excluded, att4, memory, countEvents, cudaStream,
+                             stats);
+}
+
 int oclr_frame_render_bands_samples(oclr_frame* frame, cl_uint sampleCount, cl_uint sampleBegin, cl_uint sampleEnd, cl_uint bandRows, int rank,
                                     int worldSize, int kernelVariant, int countEvents, void* cudaStream, oclr_render_stats* stats) {
     if (!frame || rank < 0 || worldSize < 1) {

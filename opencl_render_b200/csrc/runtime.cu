@@ -22,6 +22,7 @@
 #include "grid_builder.cuh"
 #include "pack_kernels.cuh"
 #include "rt_kernels.cuh"
+#include "rt_query.cuh"
 #include "rt_tail.cuh"
 #include "rt_trace.cuh"
 #include "rt_wavefront.cuh"
@@ -1570,6 +1571,92 @@ static std::string cam_check_message(uint32_t flag);
 static int slice_count_for(uint32_t rows, uint32_t width);
 static bool resumes_prelaunch(const Frame* f, const FrameView& F);
 
+// ---- the trace stage (rt_trace.cuh), shared by frames and ray queries --------------------------------------------------------------
+// Scheduling knobs of wf_pipe_kernel.
+static const TraceTuning& trace_tuning() {
+    // (function-local static built by a lambda: initialised once, thread-safe -- RaytraceAll's all-devices mode launches from one
+    // host thread per GPU)
+    static const TraceTuning tune = [] {
+        auto env = [](const char* k, int d) { const char* v = getenv(k); return v && atoi(v) > 0 ? atoi(v) : d; };
+        TraceTuning t = {0, 1, 0, 0, 0, 0, 0, 0, 0, 0, 1, 16, 12};
+        t.refillMin = env("OCLR_REFILL_MIN", 4);
+        t.hierarchical = getenv("OCLR_HIERARCHICAL") ? atoi(getenv("OCLR_HIERARCHICAL")) : 2;
+        t.drainMin = std::min(env("OCLR_DRAIN_MIN", 64), (int)kCellQCap - 31);   // (round 2 sweep: 64 is ~1 % faster than 48 on configs 2 and 3)
+        t.walkMin3 = env("OCLR_WALK_MIN3", 8);
+        t.switchMin = env("OCLR_SWITCH_MIN", 6);
+        t.tailDrain = env("OCLR_TAIL_DRAIN", 8);
+        t.splitMin = getenv("OCLR_SPLIT_MIN") ? atoi(getenv("OCLR_SPLIT_MIN")) : 0;   // 0: never cut a walk (default, see rt_trace.cuh)
+        t.splitPart = env("OCLR_SPLIT_PART", 16);
+        t.splitEarly = getenv("OCLR_SPLIT_EARLY") ? atoi(getenv("OCLR_SPLIT_EARLY")) : 0;
+        t.handoffAfter = getenv("OCLR_HANDOFF_AFTER") ? atoi(getenv("OCLR_HANDOFF_AFTER")) : 2;
+        t.handoffMode = getenv("OCLR_HANDOFF_MODE") ? atoi(getenv("OCLR_HANDOFF_MODE")) : 1;
+        if (t.handoffMode == 1 && getenv("OCLR_TAIL_BRICKS") && atoi(getenv("OCLR_TAIL_BRICKS")) == 0) t.handoffMode = 3;   // cell-plane bursts
+        t.handoffLanes = getenv("OCLR_HANDOFF_LANES") ? atoi(getenv("OCLR_HANDOFF_LANES")) : (t.handoffMode == 2 ? 16 : 32);
+        t.handoffBurst = env("OCLR_HANDOFF_BURST", 12);
+        return t;
+    }();
+    return tune;
+}
+
+// Persistent grid of the trace kernel: as many CTAs as are resident on the device at once.
+static bool trace_grid(const SceneView& S, int smCount, bool counting, unsigned& grid, std::string& err) {
+    const size_t shBytes = sizeof(float) * 3 * (S.n + 1);
+    int perSm = 0;
+    if (counting)
+        OCLR_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&perSm, wf_pipe_kernel<true, false>, 128, shBytes));
+    else
+        OCLR_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&perSm, wf_pipe_kernel<false, false>, 128, shBytes));
+    if (perSm < 1) perSm = 1;
+    if (getenv("OCLR_TRACE_CTAS") && atoi(getenv("OCLR_TRACE_CTAS")) > 0) perSm = std::min(perSm, atoi(getenv("OCLR_TRACE_CTAS")));
+    grid = (unsigned)(smCount * perSm);
+    return true;
+}
+
+// Enqueues one round of the trace stage on `ks`: walk records of the rays queued in w (wf_setup_kernel), the trace (wf_pipe_kernel,
+// instantiation chosen from the tuning), and the hand-off of its tail when `tq` has room (tq.capacity != 0).  Every kernel reads the ray
+// count from device memory, so a round with nothing queued costs only its launches.
+static void enqueue_trace(const SceneView& S, const WfState& w, const WalkRecords& rec, const TailQueue& tq, unsigned setupGrid, unsigned traceGrid,
+                          int smCount, Counters* dcnt, cudaStream_t ks, uint32_t& launches) {
+    const TraceTuning& tune = trace_tuning();
+    const size_t shBytes = sizeof(float) * 3 * (S.n + 1);
+    wf_setup_kernel<<<setupGrid, 256, shBytes, ks>>>(S, w, rec);
+    ++launches;
+    // (the run-time split of long walks is an instantiation of its own: compiled into the production kernel it cost
+    // 10 % through register pressure even when switched off)
+    // (so is the hand-off of the tail to wf_tail_kernel: only the launches of small domains run that instantiation)
+    const bool handoff = tq.capacity != 0 && tune.splitMin <= 0;
+    if (dcnt && tune.splitMin > 0)
+        wf_pipe_kernel<true, true><<<traceGrid, 128, shBytes, ks>>>(S, w, rec, tune, dcnt, tq);
+    else if (dcnt && handoff)
+        wf_pipe_kernel<true, false, true><<<traceGrid, 128, shBytes, ks>>>(S, w, rec, tune, dcnt, tq);
+    else if (dcnt)
+        wf_pipe_kernel<true, false><<<traceGrid, 128, shBytes, ks>>>(S, w, rec, tune, dcnt, tq);
+    else if (tune.splitMin > 0)
+        wf_pipe_kernel<false, true><<<traceGrid, 128, shBytes, ks>>>(S, w, rec, tune, dcnt, tq);
+    else if (handoff)
+        wf_pipe_kernel<false, false, true><<<traceGrid, 128, shBytes, ks>>>(S, w, rec, tune, dcnt, tq);
+    else
+        wf_pipe_kernel<false, false><<<traceGrid, 128, shBytes, ks>>>(S, w, rec, tune, dcnt, tq);
+    if (handoff && tune.handoffMode == 2) {   // second pass: the same kernel over the rays given up, as their own little queue
+        WfState w2 = w;
+        w2.queueCount = tq.count;
+        w2.queueCursor = tq.cursor;
+        WalkRecords rec2 = {tq.o, tq.d, tq.s0, tq.s1, tq.order, tq.count, tq.capacity};
+        if (dcnt)
+            wf_pipe_kernel<true, false><<<traceGrid, 128, shBytes, ks>>>(S, w2, rec2, tune, dcnt, tq);
+        else
+            wf_pipe_kernel<false, false><<<traceGrid, 128, shBytes, ks>>>(S, w2, rec2, tune, dcnt, tq);
+        ++launches;
+    } else if (handoff) {   // one ray per warp: bursts over brick planes (default) or over cell planes (OCLR_TAIL_BRICKS=0)
+        if (tune.handoffMode == 1)
+            wf_tail_brick_kernel<<<(unsigned)(smCount * 4), 128, shBytes, ks>>>(S, w, tq);
+        else
+            wf_tail_kernel<<<(unsigned)(smCount * 4), 128, shBytes, ks>>>(S, w, tq);
+        ++launches;
+    }
+    ++launches;
+}
+
 // Wavefront driver: alternate the logic and trace kernels until no path is waiting for a ray (rt_wavefront.cuh).
 // `prelaunchOnly`: allocate the path state and enqueue nothing but the first logic round of the first sample, on the frame's own
 // stream behind everything already enqueued on `st` (frame_prelaunch).  A later normal call with the same view finds
@@ -1695,36 +1782,8 @@ static bool launch_wavefront(Frame* f, const SceneView& S, const FrameView& Fall
         return false;
     }
 
-    const size_t shBytes = sizeof(float) * 3 * (S.n + 1);
-    int perSm = 0;
-    if (dcnt)
-        OCLR_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&perSm, wf_pipe_kernel<true, false>, 128, shBytes));
-    else
-        OCLR_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&perSm, wf_pipe_kernel<false, false>, 128, shBytes));
-    if (perSm < 1) perSm = 1;
-    // (function-local static built by a lambda: initialised once, thread-safe -- RaytraceAll's all-devices mode launches from one
-    // host thread per GPU)
-    static const TraceTuning tune = [] {
-        auto env = [](const char* k, int d) { const char* v = getenv(k); return v && atoi(v) > 0 ? atoi(v) : d; };
-        TraceTuning t = {0, 1, 0, 0, 0, 0, 0, 0, 0, 0, 1, 16, 12};
-        t.refillMin = env("OCLR_REFILL_MIN", 4);
-        t.hierarchical = getenv("OCLR_HIERARCHICAL") ? atoi(getenv("OCLR_HIERARCHICAL")) : 2;
-        t.drainMin = std::min(env("OCLR_DRAIN_MIN", 64), (int)kCellQCap - 31);   // (round 2 sweep: 64 is ~1 % faster than 48 on configs 2 and 3)
-        t.walkMin3 = env("OCLR_WALK_MIN3", 8);
-        t.switchMin = env("OCLR_SWITCH_MIN", 6);
-        t.tailDrain = env("OCLR_TAIL_DRAIN", 8);
-        t.splitMin = getenv("OCLR_SPLIT_MIN") ? atoi(getenv("OCLR_SPLIT_MIN")) : 0;   // 0: never cut a walk (default, see rt_trace.cuh)
-        t.splitPart = env("OCLR_SPLIT_PART", 16);
-        t.splitEarly = getenv("OCLR_SPLIT_EARLY") ? atoi(getenv("OCLR_SPLIT_EARLY")) : 0;
-        t.handoffAfter = getenv("OCLR_HANDOFF_AFTER") ? atoi(getenv("OCLR_HANDOFF_AFTER")) : 2;
-        t.handoffMode = getenv("OCLR_HANDOFF_MODE") ? atoi(getenv("OCLR_HANDOFF_MODE")) : 1;
-        if (t.handoffMode == 1 && getenv("OCLR_TAIL_BRICKS") && atoi(getenv("OCLR_TAIL_BRICKS")) == 0) t.handoffMode = 3;   // cell-plane bursts
-        t.handoffLanes = getenv("OCLR_HANDOFF_LANES") ? atoi(getenv("OCLR_HANDOFF_LANES")) : (t.handoffMode == 2 ? 16 : 32);
-        t.handoffBurst = env("OCLR_HANDOFF_BURST", 12);
-        return t;
-    }();
-    if (getenv("OCLR_TRACE_CTAS") && atoi(getenv("OCLR_TRACE_CTAS")) > 0) perSm = std::min(perSm, atoi(getenv("OCLR_TRACE_CTAS")));
-    const unsigned traceGrid = (unsigned)(smCount * perSm);
+    unsigned traceGrid = 0;
+    if (!trace_grid(S, smCount, dcnt != nullptr, traceGrid, err)) return false;
     if (Fall.flagOut && !resumePre) OCLR_CUDA(cudaMemsetAsync(Fall.flagOut, 0, (size_t)Fall.cam.width * Fall.cam.height, st));
     if (prelaunchOnly) {
         if (!f->preStream) {
@@ -1803,49 +1862,14 @@ static bool launch_wavefront(Frame* f, const SceneView& S, const FrameView& Fall
                         }
                         OCLR_CUDA(cudaEventRecord(sl.traceEvents[sl.traceEventsUsed], ks));
                     }
-                    wf_setup_kernel<<<setupGrid[k], 256, shBytes, ks>>>(S, w[k], rec[k]);
-                    ++launches;
-                    // (the run-time split of long walks is an instantiation of its own: compiled into the production kernel it cost
-                    // 10 % through register pressure even when switched off)
-                    // (so is the hand-off of the tail to wf_tail_kernel: only the launches of small domains run that instantiation)
                     TailQueue tq = {(uint4*)sl.tailEntries.p, w[k].queueCount + 2 + kLengthClasses, w[k].queueCount + 6 + kLengthClasses,
                                     sl.tailCapacity, (float4*)sl.tailO.p, (float4*)sl.tailD.p, (float4*)sl.tailS0.p, (uint4*)sl.tailS1.p,
                                     (uint32_t*)sl.tailOrder.p};
-                    const bool handoff = sl.tailCapacity != 0 && tune.splitMin <= 0;
-                    if (dcnt && tune.splitMin > 0)
-                        wf_pipe_kernel<true, true><<<traceGrid, 128, shBytes, ks>>>(S, w[k], rec[k], tune, dcnt, tq);
-                    else if (dcnt && handoff)
-                        wf_pipe_kernel<true, false, true><<<traceGrid, 128, shBytes, ks>>>(S, w[k], rec[k], tune, dcnt, tq);
-                    else if (dcnt)
-                        wf_pipe_kernel<true, false><<<traceGrid, 128, shBytes, ks>>>(S, w[k], rec[k], tune, dcnt, tq);
-                    else if (tune.splitMin > 0)
-                        wf_pipe_kernel<false, true><<<traceGrid, 128, shBytes, ks>>>(S, w[k], rec[k], tune, dcnt, tq);
-                    else if (handoff)
-                        wf_pipe_kernel<false, false, true><<<traceGrid, 128, shBytes, ks>>>(S, w[k], rec[k], tune, dcnt, tq);
-                    else
-                        wf_pipe_kernel<false, false><<<traceGrid, 128, shBytes, ks>>>(S, w[k], rec[k], tune, dcnt, tq);
-                    if (handoff && tune.handoffMode == 2) {   // second pass: the same kernel over the rays given up, as their own little queue
-                        WfState w2 = w[k];
-                        w2.queueCount = tq.count;
-                        w2.queueCursor = tq.cursor;
-                        WalkRecords rec2 = {tq.o, tq.d, tq.s0, tq.s1, tq.order, tq.count, tq.capacity};
-                        if (dcnt)
-                            wf_pipe_kernel<true, false><<<traceGrid, 128, shBytes, ks>>>(S, w2, rec2, tune, dcnt, tq);
-                        else
-                            wf_pipe_kernel<false, false><<<traceGrid, 128, shBytes, ks>>>(S, w2, rec2, tune, dcnt, tq);
-                        ++launches;
-                    } else if (handoff) {   // one ray per warp: bursts over brick planes (default) or over cell planes (OCLR_TAIL_BRICKS=0)
-                        if (tune.handoffMode == 1)
-                            wf_tail_brick_kernel<<<(unsigned)(smCount * 4), 128, shBytes, ks>>>(S, w[k], tq);
-                        else
-                            wf_tail_kernel<<<(unsigned)(smCount * 4), 128, shBytes, ks>>>(S, w[k], tq);
-                        ++launches;
-                    }
+                    enqueue_trace(S, w[k], rec[k], tq, setupGrid[k], traceGrid, smCount, dcnt, ks, launches);
                     if (timeTrace) {
                         OCLR_CUDA(cudaEventRecord(sl.traceEvents[sl.traceEventsUsed + 1], ks));
                         sl.traceEventsUsed += 2;
                     }
-                    ++launches;
                     ++round[k];
                 }
             }
@@ -2395,6 +2419,190 @@ void frame_device_planes(Frame* f, void** r, void** g, void** b) {
     *r = d;
     *g = d + P;
     *b = d + 2 * P;
+}
+
+// ---- batched ray queries (rt_query.cuh) ------------------------------------------------------------------------------------------------
+// A device pointer the trace stage may read with 16-byte loads: device memory of the scene's device, aligned to `align`.
+static bool query_pointer_ok(const Scene* s, const void* p, size_t align, const char* what, std::string& err) {
+    if ((uintptr_t)p % align != 0) {
+        err = std::string(what) + " is not " + std::to_string(align) + "-byte aligned";
+        return false;
+    }
+    cudaPointerAttributes a;
+    if (cudaPointerGetAttributes(&a, p) != cudaSuccess) {
+        cudaGetLastError();
+        err = std::string(what) + " is not a CUDA pointer";
+        return false;
+    }
+    if ((a.type != cudaMemoryTypeDevice && a.type != cudaMemoryTypeManaged) || a.device != s->device) {
+        err = std::string(what) + " is not device memory of the scene's device (" + std::to_string(s->device) + ")";
+        return false;
+    }
+    return true;
+}
+
+// Scratch of one query call: stream-ordered allocations, released on the query's stream whichever way the call ends, so that queries
+// on one scene from different streams share nothing.
+struct QueryScratch {
+    DeviceBuffer recO, recD, recS0, recS1, order, queue, excl, counters, stats, hit, rayO, inO, inD, inExcl, out;
+    cudaStream_t st = nullptr;
+    int device = 0;
+    cudaEvent_t ev0 = nullptr, ev1 = nullptr;
+    uint32_t* pinned = nullptr;   // transmittance: rays the last enqueued round queued again, read back once per chunk
+    ~QueryScratch() {
+        for (DeviceBuffer* b : {&recO, &recD, &recS0, &recS1, &order, &queue, &excl, &counters, &stats, &hit, &rayO, &inO, &inD, &inExcl, &out})
+            b->release(st);
+        drop_event(device, ev0, true);
+        drop_event(device, ev1, true);
+        pinned_release(pinned);
+    }
+};
+
+static bool scene_query(Scene* s, bool transmit, size_t count, const float* origin4, const float* direction4, const uint32_t* excluded,
+                        float* out4, bool deviceMemory, bool counting, void* stream, RenderStats* stats, std::string& err) {
+    if (!s) {
+        err = "null scene";
+        return false;
+    }
+    if (stats) *stats = RenderStats();
+    if (count == 0) return true;
+    if (!origin4 || !direction4 || !out4) {
+        err = "null origin, direction or output array";
+        return false;
+    }
+    OCLR_CUDA(cudaSetDevice(s->device));
+    if (deviceMemory && (!query_pointer_ok(s, origin4, 16, "origin", err) || !query_pointer_ok(s, direction4, 16, "direction", err) ||
+                         !query_pointer_ok(s, out4, 16, transmit ? "att" : "hit", err) ||
+                         (excluded && !query_pointer_ok(s, excluded, 4, "excluded", err))))
+        return false;
+    const SceneView& S = s->view;
+    if (S.n > 1024) {
+        err = "axesDivCount > 1024 is not supported by the packed walk";
+        return false;
+    }
+    cudaStream_t st = (cudaStream_t)stream;
+    QueryScratch q;
+    q.st = st;
+    q.device = s->device;
+    const uint32_t B = (uint32_t)std::min<size_t>(count, kQueryBatch);
+    const size_t b = B;
+    if (!q.recO.alloc(sizeof(float4) * b, err, st) || !q.recD.alloc(sizeof(float4) * b, err, st) || !q.recS0.alloc(sizeof(float4) * b, err, st) ||
+        !q.recS1.alloc(sizeof(uint4) * b, err, st) || !q.order.alloc(sizeof(uint32_t) * b * kLengthClasses, err, st) ||
+        !q.queue.alloc(sizeof(uint32_t) * b * (transmit ? 2 : 1), err, st) || !q.excl.alloc(sizeof(uint32_t) * b, err, st) ||
+        !q.counters.alloc(sizeof(uint32_t) * (2 * kCounterStride + kRoundLogSize), err, st) ||
+        (counting && !q.stats.alloc(sizeof(Counters), err, st)) ||
+        (transmit && (!q.hit.alloc(sizeof(float4) * b, err, st) || !q.rayO.alloc(sizeof(float4) * b, err, st))) ||
+        (!deviceMemory && (!q.inO.alloc(sizeof(float4) * b, err, st) || !q.inD.alloc(sizeof(float4) * b, err, st) ||
+                           (excluded && !q.inExcl.alloc(sizeof(uint32_t) * b, err, st)) || !q.out.alloc(sizeof(float4) * b, err, st))))
+        return false;
+    Counters* dcnt = counting ? (Counters*)q.stats.p : nullptr;
+    if (dcnt) OCLR_CUDA(cudaMemsetAsync(dcnt, 0, sizeof(Counters), st));
+    if (stats) {
+        OCLR_CUDA(make_event(s->device, &q.ev0, true));
+        OCLR_CUDA(make_event(s->device, &q.ev1, true));
+        OCLR_CUDA(cudaEventRecord(q.ev0, st));
+    }
+    unsigned traceGrid = 0;
+    if (!trace_grid(S, s->smCount, counting, traceGrid, err)) return false;
+    const unsigned setupGrid = (unsigned)std::min<uint64_t>((uint64_t)s->smCount * 8, (b + 255) / 256);
+    const unsigned rayGrid = (unsigned)std::min<uint64_t>((uint64_t)s->smCount * 16, (b + 127) / 128);
+    uint32_t* counters = (uint32_t*)q.counters.p;
+    const uint32_t cstride = kCounterStride;
+    if (transmit && !(q.pinned = (uint32_t*)pinned_block())) {
+        err = "out of pinned host memory";
+        return false;
+    }
+    uint32_t launches = 0, rounds = 0;
+    for (size_t off = 0; off < count; off += b) {
+        const uint32_t n = (uint32_t)std::min<size_t>(b, count - off);
+        QueryBatch qb;
+        qb.count = n;
+        qb.excl = (uint32_t*)q.excl.p;
+        if (deviceMemory) {
+            qb.origin = (const float4*)origin4 + off;
+            qb.direction = (const float4*)direction4 + off;
+            qb.excluded = excluded ? excluded + off : nullptr;
+        } else {
+            if (!host_to_device(q.inO.p, origin4 + 4 * off, sizeof(float4) * n, st, err) ||
+                !host_to_device(q.inD.p, direction4 + 4 * off, sizeof(float4) * n, st, err) ||
+                (excluded && !host_to_device(q.inExcl.p, excluded + off, sizeof(uint32_t) * n, st, err)))
+                return false;
+            qb.origin = (const float4*)q.inO.p;
+            qb.direction = (const float4*)q.inD.p;
+            qb.excluded = excluded ? (const uint32_t*)q.inExcl.p : nullptr;
+        }
+        float4* result = deviceMemory ? (float4*)out4 + off : (float4*)q.out.p;
+        qb.hit = transmit ? (float4*)q.hit.p : result;
+        qb.rayO = transmit ? (float4*)q.rayO.p : nullptr;
+        qb.att = transmit ? result : nullptr;
+        WfState w = {};
+        w.Q = B;
+        w.rayO = transmit ? qb.rayO : (float4*)qb.origin;   // (the trace stage only reads rayO / rayD / rayExcl)
+        w.rayD = (float4*)qb.direction;
+        w.rayExcl = qb.excl;
+        w.hit = qb.hit;
+        w.roundLog = counters + 2 * cstride;
+        WalkRecords rec = {(float4*)q.recO.p, (float4*)q.recD.p, (float4*)q.recS0.p, (uint4*)q.recS1.p, (uint32_t*)q.order.p, nullptr, B};
+        auto use_set = [&](WfState& v, uint32_t r) {
+            v.queue = (uint32_t*)q.queue.p + (transmit ? (size_t)(r & 1u) * b : 0);
+            v.queueCount = counters + cstride * (r & 1u);
+            v.queueCursor = v.queueCount + 1;
+        };
+        use_set(w, 0);
+        OCLR_CUDA(cudaMemsetAsync(w.queueCount, 0, sizeof(uint32_t) * cstride, st));
+        query_screen_kernel<<<rayGrid, 128, 0, st>>>(qb, w);
+        ++launches;
+        // Rounds (trace -> transmit) are enqueued ahead in chunks without a host round trip, as frames do (launch_wavefront): every kernel
+        // reads its ray count from device memory and returns at once when there is nothing to do.  One read per chunk: the count the last
+        // transmit round queued.
+        for (uint32_t r = 0;;) {
+            const uint32_t chunk = transmit ? 3u : 1u;
+            for (uint32_t c = 0; c < chunk; ++c, ++r) {
+                use_set(w, r);
+                w.roundIndex = r;
+                rec.classCount = w.queueCount + 2;
+                const TailQueue tq = {nullptr, w.queueCount + 2 + kLengthClasses, w.queueCount + 6 + kLengthClasses, 0u,
+                                      nullptr, nullptr, nullptr, nullptr, nullptr};
+                enqueue_trace(S, w, rec, tq, setupGrid, traceGrid, s->smCount, dcnt, st, launches);
+                ++rounds;
+                if (!transmit) break;
+                WfState next = w;
+                use_set(next, r + 1);
+                OCLR_CUDA(cudaMemsetAsync(next.queueCount, 0, sizeof(uint32_t) * cstride, st));
+                query_transmit_kernel<<<rayGrid, 128, 0, st>>>(S, qb, w.queue, w.queueCount, next);
+                ++launches;
+            }
+            if (!transmit) break;
+            OCLR_CUDA(cudaMemcpyAsync(q.pinned, counters + cstride * (r & 1u), sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
+            OCLR_CUDA(cudaStreamSynchronize(st));
+            if (*q.pinned == 0) break;
+            if (r > 100000) {
+                err = "transmittance did not converge";
+                return false;
+            }
+        }
+        OCLR_CUDA(cudaGetLastError());
+        if (!deviceMemory && !device_to_host(out4 + 4 * off, q.out.p, sizeof(float4) * n, st, err)) return false;
+    }
+    if (stats) {
+        OCLR_CUDA(cudaEventRecord(q.ev1, st));
+        OCLR_CUDA(cudaEventSynchronize(q.ev1));
+        OCLR_CUDA(cudaEventElapsedTime(&stats->deviceMs, q.ev0, q.ev1));
+        stats->launches = launches;
+        stats->traceLaunches = rounds;
+        if (dcnt) OCLR_CUDA(cudaMemcpy(&stats->counters, dcnt, sizeof(Counters), cudaMemcpyDeviceToHost));
+    }
+    return true;
+}
+
+bool scene_intersect(Scene* s, size_t count, const float* origin4, const float* direction4, const uint32_t* excluded, float* hit4,
+                     bool deviceMemory, bool counting, void* stream, RenderStats* stats, std::string& err) {
+    return scene_query(s, false, count, origin4, direction4, excluded, hit4, deviceMemory, counting, stream, stats, err);
+}
+
+bool scene_transmittance(Scene* s, size_t count, const float* origin4, const float* direction4, const uint32_t* excluded, float* att4,
+                         bool deviceMemory, bool counting, void* stream, RenderStats* stats, std::string& err) {
+    return scene_query(s, true, count, origin4, direction4, excluded, att4, deviceMemory, counting, stream, stats, err);
 }
 
 }  // namespace oclr

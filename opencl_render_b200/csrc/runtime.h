@@ -170,4 +170,17 @@ bool frame_push_rows(Frame* f, uint32_t bandRows, uint32_t rank, uint32_t world,
 // Device pointers of the planes (for NCCL gathers done by the host layer) and of the id plane.
 void frame_device_planes(Frame* f, void** r, void** g, void** b);
 
+// Batched ray queries on a resident scene (rt_query.cuh; semantics and preconditions in include/oclr_abi.h): closest hit
+// (RayIntersectsTriangles) into hit4 = (as_float(tri), t, abL, acL), and the shadow loop's transmittance into att4 = (rgb,
+// as_float(last blocker)).  origin4 / direction4 / hit4 / att4 are 4 floats per ray; excluded may be null.  Rays are processed in
+// batches of kQueryBatch: the call's scratch (walk records 64 B, class order 16 B, queue 4 B, excluded triangle 4 B per ray of a batch;
+// transmittance adds a second queue, hits and an origin copy, 36 B; host-memory inputs add staging, 52 B) stays below 300 MB.
+// deviceMemory: the arrays are device memory of the scene's device, 16-byte aligned (excluded: 4).  Synchronous when `stats` is given,
+// for host memory and for transmittance.
+enum { kQueryBatch = 1 << 21 };
+bool scene_intersect(Scene* s, size_t count, const float* origin4, const float* direction4, const uint32_t* excluded, float* hit4,
+                     bool deviceMemory, bool counting, void* stream, RenderStats* stats, std::string& err);
+bool scene_transmittance(Scene* s, size_t count, const float* origin4, const float* direction4, const uint32_t* excluded, float* att4,
+                         bool deviceMemory, bool counting, void* stream, RenderStats* stats, std::string& err);
+
 }  // namespace oclr
