@@ -375,6 +375,33 @@ int oclr_scene_intersect(oclr_scene* scene, size_t count, const cl_float* origin
 int oclr_scene_transmittance(oclr_scene* scene, size_t count, const cl_float* origin4, const cl_float* direction4, const cl_uint* excluded,
                              cl_float* att4, int memory, int countEvents, void* cudaStream, oclr_render_stats* stats);
 
+/* Radiance along caller rays: the colour the reference computes for a pixel-sample (raytrace_opencl.c:452-725 -- shading, lights and
+ * their shadow loops, the ring of diffuse / mirror / glass segments, the RNG draw order), with the camera segment replaced by the
+ * caller's ray.  For light baking, light probes and projections the pinhole camera cannot express (panoramas, stereo, orthographic).
+ *
+ * Rays as for the queries above, with maxD = direction4[i].w = +inf (ring segments have no far limit).  Ring slot 0 is {o, d, minD,
+ * excluded, weight (1,1,1), 12 bounces}, an ordinary grid segment: its closest hit is RayIntersectsTriangles, never a camera-list scan,
+ * and so is that of its glass continuation.  There are no jitter draws: sample s of ray i starts from rng = (indexBase + i) *
+ * sampleCount + s + 1 (64-bit), the frame's pixel * S + s + 1 rule with the ray's global index for the pixel, so a job split across
+ * calls (indexBase = index of the call's first ray) gives the same results.  sampleCount >= 1; a call renders all samples.
+ *   rgb4[i] = (R, G, B, as_float(tri0)): R = (colour_0 + colour_1 + ... ) / (float)sampleCount, an fp32 sum in sample order and one
+ *   IEEE division, where colour_s is the value the reference converts at :726-741 (before its * 65535 / S truncation); tri0 = the
+ *   triangle the ray itself hits in sample 0, or 0xFFFFFFFF.
+ * A ray with minD < 0, a NaN minD, a maxD other than +inf, or a non-finite origin or direction component is not traced: (NaN, NaN,
+ * NaN, 0xFFFFFFFF), which no real result has.  A zero direction or minD = +inf meets nothing: (0, 0, 0, 0xFFFFFFFF) without a trace.
+ * flags: NULL or cl_uchar[count]; bit 0 = the reference's own result is undefined for this ray, as in oclr_frame_read_flags (every
+ * caller ray is a non-camera segment, so this can happen on its very first hit).
+ * camera: bump-mapped normals read its leftToRight, topToBottom and pixelSizeInv (raytrace_opencl.c:195-263), nothing else of it.
+ * It may be NULL only if no material has a BUMP channel; otherwise the call fails.
+ * memory, alignment (rgb4 16 bytes, flags 1), pointer checks, countEvents and cudaStream as for the queries above.  Rays go in
+ * internal batches of 2^20 (1 048 576) with about 1 KB of path state per ray of a batch (about 1.1 GB stream-ordered scratch; host
+ * memory adds about 55 MB of staging).  The call always synchronises (it reads each sample's round count back).  With countEvents,
+ * counters.segments / shadedHits / gridRays / occluderLookups count ring segments, shaded hits, grid walks (closest hits and every
+ * walk of the shadow loops) and transparency lookups of blockers.  Returns 1 on success. */
+int oclr_scene_radiance(oclr_scene* scene, const oclr_camera* camera, size_t count, const cl_float* origin4, const cl_float* direction4,
+                        const cl_uint* excluded, unsigned long long indexBase, cl_uint sampleCount, cl_float* rgb4, cl_uchar* flags,
+                        int memory, int countEvents, void* cudaStream, oclr_render_stats* stats);
+
 /* Rows of a W x H image owned by `rank` of `worldSize` when the image is cut into bands of `bandRows` rows dealt
  * round-robin (SURVEY.md section 8e; band height 128 = the reference's tile height, raytrace.c:507).  Writes up to
  * `maxBands` [begin,end) pairs to `rows` and returns the number of bands owned. */

@@ -81,7 +81,7 @@ EXPORTS = [
     "oclr_frame_write_accum", "oclr_frame_progress", "oclr_estimated_seconds_left", "oclr_write_bmp", "oclr_write_ppm16", "oclr_write_png16",
     "oclr_set_option", "oclr_frame_push_rows",
     # batched ray queries on a resident scene
-    "oclr_scene_intersect", "oclr_scene_transmittance",
+    "oclr_scene_intersect", "oclr_scene_transmittance", "oclr_scene_radiance",
 ]
 
 _lib = None
@@ -188,6 +188,9 @@ def load() -> C.CDLL:
         getattr(lib, name).restype = C.c_int
         getattr(lib, name).argtypes = [C.c_void_p, C.c_size_t, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_void_p,
                                        C.POINTER(RenderStats)]
+    lib.oclr_scene_radiance.restype = C.c_int
+    lib.oclr_scene_radiance.argtypes = [C.c_void_p, C.POINTER(Camera), C.c_size_t, C.c_void_p, C.c_void_p, C.c_void_p, C.c_ulonglong, C.c_uint32,
+                                        C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.POINTER(RenderStats)]
     lib.oclr_set_option.restype = C.c_int
     lib.oclr_set_option.argtypes = [C.c_char_p, C.c_int]
     lib.InitOpenCL.restype = None

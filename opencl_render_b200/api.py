@@ -26,6 +26,7 @@ ACCUMULATE_REFERENCE_16BIT, ACCUMULATE_FLOAT = 0, 1
 NO_TRIANGLE = 0xFFFFFFFF
 QUERY_HOST_MEMORY, QUERY_DEVICE_MEMORY = 0, 1
 QUERY_BATCH = 1 << 21        # rays per internal batch of a query (runtime.h kQueryBatch)
+RADIANCE_BATCH = 1 << 20     # rays per internal batch of a radiance query (runtime.h kRadianceBatch)
 
 
 class OclrError(RuntimeError):
@@ -292,7 +293,7 @@ class DeviceScene:
         tensors.  Returns (ids uint32[N], t float32[N], abL float32[N], acL float32[N]) -- a miss is (NO_TRIANGLE, maxD, 0, 0), a ray
         that breaks the preconditions (minD < 0, NaN range, non-finite component) (NO_TRIANGLE, NaN, 0, 0) -- plus the counters dict
         when count=True."""
-        out, cnt = self._query("oclr_scene_intersect", origins, directions, t_min, t_max, exclude, stream, count)
+        out, _, cnt = self._query(self._entry("oclr_scene_intersect"), origins, directions, t_min, t_max, exclude, stream, count)
         res = (self._ids(out[:, 0]), out[:, 1], out[:, 2], out[:, 3])
         return res + (cnt,) if count else res
 
@@ -300,8 +301,36 @@ class DeviceScene:
         """Transmittance along every ray: the shadow loop of raytrace_opencl.c:608-627 (att starts at (1,1,1) and is multiplied by the
         TRANSPARENCY texel of each blocker, 0 without that channel, until a component reaches 0 or the ray is clear).  Arguments as in
         intersect().  Returns (att float32[N,3], last blocker uint32[N] or NO_TRIANGLE) (+ counters dict when count=True)."""
-        out, cnt = self._query("oclr_scene_transmittance", origins, directions, t_min, t_max, exclude, stream, count)
+        out, _, cnt = self._query(self._entry("oclr_scene_transmittance"), origins, directions, t_min, t_max, exclude, stream, count)
         res = (out[:, :3], self._ids(out[:, 3]))
+        return res + (cnt,) if count else res
+
+    def radiance(self, origins, directions, t_min=None, exclude=None, samples: int = 1, index_base: int = 0, camera: CameraSetup | None = None,
+                 stream=None, flags: bool = False, count: bool = False):
+        """Colour arriving along every ray: the reference's pixel-sample loop (raytrace_opencl.c:452-725) with the camera segment replaced by
+        the ray (semantics in include/oclr_abi.h, oclr_scene_radiance).  origins / directions as in intersect(), but a ray has no far
+        limit: [N,4] directions carry +inf in column 3 (a finite one is refused per ray, with a NaN result).  Sample s of ray i is seeded
+        (index_base + i) * samples + s + 1, so a job split over calls gives the same colours.  `camera` (CameraSetup): its pixel step
+        vectors are what bump-mapped normals read; required when a material has a BUMP channel.  Returns (rgb float32[N,3] = mean over
+        the samples, first-hit ids uint32[N] = the ray's own hit in sample 0), plus flags uint8[N] (bit 0: the reference's result is
+        undefined for the ray) when flags=True and the counters dict when count=True."""
+        if isinstance(samples, bool) or not isinstance(samples, (int, np.integer)) or samples < 1:
+            raise ValueError(f"samples must be an integer >= 1, got {samples!r}")
+        if isinstance(index_base, bool) or not isinstance(index_base, (int, np.integer)) or not 0 <= index_base < 1 << 64:
+            raise ValueError(f"index_base must be an integer in [0, 2^64), got {index_base!r}")
+        if camera is not None and not isinstance(camera, CameraSetup):
+            raise ValueError("camera must be a CameraSetup (set_camera) or None")
+        host = getattr(self, "host", None)
+        if camera is None and host is not None and host.material_count and (host.mat_size[CH_BUMP::MATERIAL_CHANNEL_COUNT, 0] > 0).any():
+            raise ValueError("the scene has bump-mapped materials, whose normals read the camera's pixel step vectors: pass camera=")
+        cam = C.byref(camera.c()) if camera is not None else None
+
+        def native(n, o, d, ex, out, fl, memory, cnt, st, stats):
+            return self._lib.oclr_scene_radiance(self.handle, cam, n, o, d, ex, int(index_base), int(samples), out, fl, memory, cnt, st, stats)
+        out, fl, cnt = self._query(native, origins, directions, t_min, None, exclude, stream, count, flags)
+        res = (out[:, :3], self._ids(out[:, 3]))
+        if flags:
+            res += (fl,)
         return res + (cnt,) if count else res
 
     @staticmethod
@@ -311,16 +340,27 @@ class DeviceScene:
         import torch
         return col.contiguous().view(torch.uint32)
 
-    def _query(self, entry, origins, directions, t_min, t_max, exclude, stream, count):
+    def _entry(self, name):
+        """The native call of oclr_scene_intersect / oclr_scene_transmittance in _query's argument order."""
+        def native(n, o, d, ex, out, fl, memory, cnt, st, stats):
+            return getattr(self._lib, name)(self.handle, n, o, d, ex, out, memory, cnt, st, stats)
+        return native
+
+    def _query(self, native, origins, directions, t_min, t_max, exclude, stream, count, flags=False):
+        """Runs native(n, origin4, direction4, excluded, out4, flags, memory, countEvents, stream, stats) on validated rays: numpy inputs
+        through host memory, CUDA torch tensors in place on `stream`.  Returns (out [N,4], flags uint8 [N] or None, counters dict or None)."""
         torch = _torch_if_tensor(origins)
         if torch is None:
+            if _torch_if_tensor(directions) is not None:
+                raise ValueError("directions is a torch tensor, origins a numpy array: a query takes numpy or torch inputs, not both")
             o, d, ex = _query_rays_numpy(origins, directions, t_min, t_max, exclude)
             out = np.empty((o.shape[0], 4), np.float32)
+            fl = np.zeros(o.shape[0], np.uint8) if flags else None
             stats = _lib.RenderStats()
-            if not getattr(self._lib, entry)(self.handle, o.shape[0], _ptr(o), _ptr(d), _ptr(ex), _ptr(out), QUERY_HOST_MEMORY,
-                                              1 if count else 0, None, C.byref(stats) if count else None):
+            if not native(o.shape[0], _ptr(o), _ptr(d), _ptr(ex), _ptr(out), _ptr(fl), QUERY_HOST_MEMORY, 1 if count else 0, None,
+                          C.byref(stats) if count else None):
                 raise OclrError(_lib.last_error())
-            return out, (stats.counters.as_dict() if count else None)
+            return out, fl, (stats.counters.as_dict() if count else None)
         dev = torch.device("cuda", self.device)
         for name, a in (("origins", origins), ("directions", directions), ("exclude", exclude), ("t_min", t_min), ("t_max", t_max)):
             if isinstance(a, torch.Tensor) and a.device != dev:
@@ -336,18 +376,19 @@ class DeviceScene:
         with torch.cuda.device(dev), torch.cuda.stream(ts):
             o, d, ex = _query_rays_torch(torch, dev, origins, directions, t_min, t_max, exclude)
             out = torch.empty((o.shape[0], 4), dtype=torch.float32, device=dev)
+            fl = torch.zeros(o.shape[0], dtype=torch.uint8, device=dev) if flags else None
             stats = _lib.RenderStats()
-            sync = count
-            if not getattr(self._lib, entry)(self.handle, o.shape[0], C.c_void_p(o.data_ptr()), C.c_void_p(d.data_ptr()),
-                                              C.c_void_p(ex.data_ptr()) if ex is not None else None, C.c_void_p(out.data_ptr()),
-                                              QUERY_DEVICE_MEMORY, 1 if count else 0, C.c_void_p(ts.cuda_stream),
-                                              C.byref(stats) if sync else None):
+            if not native(o.shape[0], C.c_void_p(o.data_ptr()), C.c_void_p(d.data_ptr()), C.c_void_p(ex.data_ptr()) if ex is not None else None,
+                          C.c_void_p(out.data_ptr()), C.c_void_p(fl.data_ptr()) if fl is not None else None, QUERY_DEVICE_MEMORY,
+                          1 if count else 0, C.c_void_p(ts.cuda_stream), C.byref(stats) if count else None):
                 raise OclrError(_lib.last_error())
         cur = torch.cuda.current_stream(dev)
         if cur != ts:   # results are used on the caller's current stream
             cur.wait_stream(ts)
             out.record_stream(cur)
-        return out, (stats.counters.as_dict() if count else None)
+            if fl is not None:
+                fl.record_stream(cur)
+        return out, fl, (stats.counters.as_dict() if count else None)
 
     def close(self):
         if getattr(self, "handle", None):

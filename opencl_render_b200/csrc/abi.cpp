@@ -361,6 +361,29 @@ int oclr_scene_transmittance(oclr_scene* scene, size_t count, const cl_float* or
     return scene_query_entry("oclr_scene_transmittance", true, scene, count, origin4, direction4, excluded, att4, memory, countEvents, cudaStream,
                              stats);
 }
+int oclr_scene_radiance(oclr_scene* scene, const oclr_camera* camera, size_t count, const cl_float* origin4, const cl_float* direction4,
+                        const cl_uint* excluded, unsigned long long indexBase, cl_uint sampleCount, cl_float* rgb4, cl_uchar* flags, int memory,
+                        int countEvents, void* cudaStream, oclr_render_stats* stats) {
+    if (!scene) {
+        fail("oclr_scene_radiance: null scene");
+        return 0;
+    }
+    if (memory != OCLR_QUERY_HOST_MEMORY && memory != OCLR_QUERY_DEVICE_MEMORY) {
+        fail("oclr_scene_radiance: unknown memory kind " + std::to_string(memory));
+        return 0;
+    }
+    std::string err;
+    RenderStats rs;
+    Camera cam;
+    if (camera) cam = to_camera(camera);
+    if (!scene_radiance(scene->impl, camera ? &cam : nullptr, count, origin4, direction4, excluded, indexBase, sampleCount, rgb4, flags,
+                        memory == OCLR_QUERY_DEVICE_MEMORY, countEvents != 0, cudaStream, stats ? &rs : nullptr, err)) {
+        fail("oclr_scene_radiance: " + err);
+        return 0;
+    }
+    if (stats) copy_stats(stats, rs);
+    return 1;
+}
 
 int oclr_frame_render_bands_samples(oclr_frame* frame, cl_uint sampleCount, cl_uint sampleBegin, cl_uint sampleEnd, cl_uint bandRows, int rank,
                                     int worldSize, int kernelVariant, int countEvents, void* cudaStream, oclr_render_stats* stats) {

@@ -658,6 +658,7 @@ struct Scene {
     // (or only all-black ones, the plugin's 1x1 fallback) never touches slot 2, so its frames allocate 2 slots (96 B per path)
     // instead of kRingSize (576 B)
     int ringSlots = kRingSize;
+    bool hasBump = false;   // some material has a BUMP channel: its normals read the camera vectors (radiance queries need a camera)
 };
 
 // Wavefront path state of one slice of a launch domain (launch_wavefront): its own buffers, queue counters and stream, so
@@ -1045,6 +1046,8 @@ static bool scene_upload(Scene* s, const HostScene& h, std::string& err, const s
             if (!black) s->ringSlots = kRingSize;
         }
     if (const char* v = getenv("OCLR_RING_SLOTS")) s->ringSlots = std::max(s->ringSlots, std::min(atoi(v), (int)kRingSize));   // (test knob: more, never fewer)
+    s->hasBump = false;
+    for (uint32_t m = 0; m < h.materialCount; ++m) s->hasBump |= h.matSize[kMaterialChannels * m + kChBump].x > 0u;
     uint32_t total = buildGrid ? 0u : h.gridStart[cells];
     if (total && !h.gridList) {
         err = "scenePixelTriangleList missing";
@@ -2603,6 +2606,221 @@ bool scene_intersect(Scene* s, size_t count, const float* origin4, const float* 
 bool scene_transmittance(Scene* s, size_t count, const float* origin4, const float* direction4, const uint32_t* excluded, float* att4,
                          bool deviceMemory, bool counting, void* stream, RenderStats* stats, std::string& err) {
     return scene_query(s, true, count, origin4, direction4, excluded, att4, deviceMemory, counting, stream, stats, err);
+}
+
+// ---- radiance along caller rays (rt_query.cuh radiance_start_kernel, then the frame's wf_logic_kernel) ---------------------------------
+// Scratch of one radiance call: the path state of one batch, stream-ordered like QueryScratch.
+struct RadianceScratch {
+    DeviceBuffer ctl, rng, colour, ring, carry, rayO, rayD, rayExcl, hit, queue, recO, recD, recS0, recS1, order, counters, stats;
+    DeviceBuffer accum, firstHit, inO, inD, inExcl, out, flags;
+    cudaStream_t st = nullptr;
+    int device = 0;
+    cudaEvent_t ev0 = nullptr, ev1 = nullptr;
+    uint32_t* pinned = nullptr;   // the round log, read back once per chunk of rounds
+    ~RadianceScratch() {
+        for (DeviceBuffer* b : {&ctl, &rng, &colour, &ring, &carry, &rayO, &rayD, &rayExcl, &hit, &queue, &recO, &recD, &recS0, &recS1, &order,
+                                &counters, &stats, &accum, &firstHit, &inO, &inD, &inExcl, &out, &flags})
+            b->release(st);
+        drop_event(device, ev0, true);
+        drop_event(device, ev1, true);
+        pinned_release(pinned);
+    }
+};
+
+bool scene_radiance(Scene* s, const Camera* cam, size_t count, const float* origin4, const float* direction4, const uint32_t* excluded,
+                    unsigned long long indexBase, uint32_t sampleCount, float* rgb4, uint8_t* flags, bool deviceMemory, bool counting,
+                    void* stream, RenderStats* stats, std::string& err) {
+    if (!s) {
+        err = "null scene";
+        return false;
+    }
+    if (stats) *stats = RenderStats();
+    if (sampleCount < 1) {
+        err = "sampleCount must be at least 1";
+        return false;
+    }
+    if (!cam && s->hasBump) {
+        err = "null camera: the scene has bump-mapped materials, whose normals read the camera's leftToRight / topToBottom / pixelSizeInv";
+        return false;
+    }
+    if (count == 0) return true;
+    if (!origin4 || !direction4 || !rgb4) {
+        err = "null origin, direction or output array";
+        return false;
+    }
+    OCLR_CUDA(cudaSetDevice(s->device));
+    if (deviceMemory && (!query_pointer_ok(s, origin4, 16, "origin", err) || !query_pointer_ok(s, direction4, 16, "direction", err) ||
+                         !query_pointer_ok(s, rgb4, 16, "rgb", err) || (excluded && !query_pointer_ok(s, excluded, 4, "excluded", err)) ||
+                         (flags && !query_pointer_ok(s, flags, 1, "flags", err))))
+        return false;
+    const SceneView& S = s->view;
+    if (S.n > 1024) {
+        err = "axesDivCount > 1024 is not supported by the packed walk";
+        return false;
+    }
+    cudaStream_t st = (cudaStream_t)stream;
+    RadianceScratch q;
+    q.st = st;
+    q.device = s->device;
+    const uint32_t B = (uint32_t)std::min<size_t>(count, kRadianceBatch);
+    const size_t b = B;
+    const uint32_t W = kRadianceRowWidth, Q = (B + W - 1) / W * W;   // paths: the batch as a W-wide image (rt_query.cuh)
+    const size_t qn = Q;
+    if (!q.ctl.alloc(sizeof(uint32_t) * qn, err, st) || !q.rng.alloc(sizeof(uint64_t) * qn, err, st) || !q.colour.alloc(sizeof(float4) * qn, err, st) ||
+        !q.ring.alloc(sizeof(float4) * qn * (size_t)s->ringSlots * kRingParts, err, st) || !q.carry.alloc(sizeof(float4) * qn * kCarryParts, err, st) ||
+        // two ray slots per path (rt_wavefront.cuh: the next segment's closest hit is traced one round ahead)
+        !q.rayO.alloc(sizeof(float4) * 2 * qn, err, st) || !q.rayD.alloc(sizeof(float4) * 2 * qn, err, st) ||
+        !q.rayExcl.alloc(sizeof(uint32_t) * 2 * qn, err, st) || !q.hit.alloc(sizeof(float4) * 2 * qn, err, st) ||
+        !q.queue.alloc(sizeof(uint32_t) * 2 * qn, err, st) || !q.recO.alloc(sizeof(float4) * 2 * qn, err, st) ||
+        !q.recD.alloc(sizeof(float4) * 2 * qn, err, st) || !q.recS0.alloc(sizeof(float4) * 2 * qn, err, st) ||
+        !q.recS1.alloc(sizeof(uint4) * 2 * qn, err, st) || !q.order.alloc(sizeof(uint32_t) * 2 * qn * kLengthClasses, err, st) ||
+        !q.counters.alloc(sizeof(uint32_t) * (2 * kCounterStride + kRoundLogSize), err, st) ||
+        !q.accum.alloc(sizeof(float4) * qn, err, st) || !q.firstHit.alloc(sizeof(uint32_t) * qn, err, st) ||
+        (counting && !q.stats.alloc(sizeof(Counters), err, st)) ||
+        (!deviceMemory && (!q.inO.alloc(sizeof(float4) * b, err, st) || !q.inD.alloc(sizeof(float4) * b, err, st) ||
+                           (excluded && !q.inExcl.alloc(sizeof(uint32_t) * b, err, st)) || !q.out.alloc(sizeof(float4) * b, err, st) ||
+                           (flags && !q.flags.alloc(b, err, st)))))
+        return false;
+    if (!(q.pinned = (uint32_t*)pinned_block())) {
+        err = "out of pinned host memory";
+        return false;
+    }
+    Counters* dcnt = counting ? (Counters*)q.stats.p : nullptr;
+    if (dcnt) OCLR_CUDA(cudaMemsetAsync(dcnt, 0, sizeof(Counters), st));
+    if (stats) {
+        OCLR_CUDA(make_event(s->device, &q.ev0, true));
+        OCLR_CUDA(make_event(s->device, &q.ev1, true));
+        OCLR_CUDA(cudaEventRecord(q.ev0, st));
+    }
+    unsigned traceGrid = 0;
+    if (!trace_grid(S, s->smCount, counting, traceGrid, err)) return false;
+    const unsigned setupGrid = (unsigned)std::min<uint64_t>((uint64_t)s->smCount * 8, (2 * qn + 255) / 256);
+    const int aheadMode = ahead_mode_for(Q);   // (no camera segments: modes 1 and 2 coincide)
+    uint32_t* counters = (uint32_t*)q.counters.p;
+    const uint32_t cstride = kCounterStride;
+    WfState w = {};
+    w.Q = Q;
+    w.ctl = (uint32_t*)q.ctl.p;
+    w.rng = (uint64_t*)q.rng.p;
+    w.colour = (float4*)q.colour.p;
+    w.ring = (float4*)q.ring.p;
+    w.ringSlots = (uint32_t)s->ringSlots;
+    w.carry = (float4*)q.carry.p;
+    w.rayO = (float4*)q.rayO.p;
+    w.rayD = (float4*)q.rayD.p;
+    w.rayExcl = (uint32_t*)q.rayExcl.p;
+    w.hit = (float4*)q.hit.p;
+    w.queue = (uint32_t*)q.queue.p;
+    w.roundLog = counters + 2 * cstride;
+    WalkRecords rec = {(float4*)q.recO.p, (float4*)q.recD.p, (float4*)q.recS0.p, (uint4*)q.recS1.p, (uint32_t*)q.order.p, nullptr, 2 * Q};
+    FrameView F = {};   // the logic kernel's view of a batch: camera vectors, sample count, accumulator, flags (rt_query.cuh)
+    if (cam) F.cam = *cam;
+    F.cam.width = W;
+    F.sampleCount = sampleCount;
+    F.accum = (float4*)q.accum.p;
+    uint32_t launches = 0, rounds = 0, lastRounds = 4;
+    for (size_t off = 0; off < count; off += b) {
+        const uint32_t n = (uint32_t)std::min<size_t>(b, count - off);
+        RayBatch R;
+        R.count = n;
+        R.indexBase = indexBase + off;
+        if (deviceMemory) {
+            R.origin = (const float4*)origin4 + off;
+            R.direction = (const float4*)direction4 + off;
+            R.excluded = excluded ? excluded + off : nullptr;
+        } else {
+            if (!host_to_device(q.inO.p, origin4 + 4 * off, sizeof(float4) * n, st, err) ||
+                !host_to_device(q.inD.p, direction4 + 4 * off, sizeof(float4) * n, st, err) ||
+                (excluded && !host_to_device(q.inExcl.p, excluded + off, sizeof(uint32_t) * n, st, err)))
+                return false;
+            R.origin = (const float4*)q.inO.p;
+            R.direction = (const float4*)q.inD.p;
+            R.excluded = excluded ? (const uint32_t*)q.inExcl.p : nullptr;
+        }
+        float4* result = deviceMemory ? (float4*)rgb4 + off : (float4*)q.out.p;
+        F.flagOut = flags ? (deviceMemory ? flags + off : (uint8_t*)q.flags.p) : nullptr;
+        if (F.flagOut) OCLR_CUDA(cudaMemsetAsync(F.flagOut, 0, n, st));
+        const uint32_t rows = (n + W - 1) / W;
+        F.cam.height = rows;
+        F.rowBegin = 0;
+        F.rowEnd = rows;
+        const dim3 logicGrid(1, (rows + 7) / 8);
+        const unsigned startGrid = (rows * W + 127) / 128, rayGrid = (n + 127) / 128;
+        // Rounds (entry or logic kernel -> setup -> trace) are enqueued ahead in chunks and ended by the round log, as frames do
+        // (launch_wavefront); round 0's entry is radiance_start_kernel instead of the logic kernel's kWfNew.
+        for (uint32_t smp = 0; smp < sampleCount; ++smp) {
+            for (uint32_t r = 0;;) {
+                const uint32_t chunk = r == 0 ? std::max<uint32_t>(lastRounds, 2) : 2u;
+                for (uint32_t c = 0; c < chunk; ++c, ++r) {
+                    w.queueCount = counters + cstride * (r & 1u);
+                    w.queueCursor = w.queueCount + 1;
+                    w.roundIndex = r;
+                    rec.classCount = w.queueCount + 2;
+                    const uint32_t* prev = r ? counters + cstride * ((r - 1) & 1u) : nullptr;
+                    OCLR_CUDA(cudaMemsetAsync(w.queueCount, 0, sizeof(uint32_t) * cstride, st));
+                    if (r == 0) {
+                        if (dcnt)
+                            radiance_start_kernel<true><<<startGrid, 128, 0, st>>>(R, w, smp, sampleCount, dcnt);
+                        else
+                            radiance_start_kernel<false><<<startGrid, 128, 0, st>>>(R, w, smp, sampleCount, dcnt);
+                    } else {
+                        if (r == 1 && smp == 0)   // the trace of round 0 holds each ray's own closest hit
+                            radiance_first_hit_kernel<<<rayGrid, 128, 0, st>>>(n, w.hit, (uint32_t*)q.firstHit.p);
+                        if (dcnt)
+                            wf_logic_kernel<true><<<logicGrid, 128, 0, st>>>(S, F, w, smp, 0u, prev, dcnt, aheadMode);
+                        else
+                            wf_logic_kernel<false><<<logicGrid, 128, 0, st>>>(S, F, w, smp, 0u, prev, dcnt, aheadMode);
+                    }
+                    ++launches;
+                    const TailQueue tq = {nullptr, w.queueCount + 2 + kLengthClasses, w.queueCount + 6 + kLengthClasses, 0u,
+                                          nullptr, nullptr, nullptr, nullptr, nullptr};
+                    enqueue_trace(S, w, rec, tq, setupGrid, traceGrid, s->smCount, dcnt, st, launches);
+                    ++rounds;
+                }
+                OCLR_CUDA(cudaMemcpyAsync(q.pinned, counters + 2 * cstride, sizeof(uint32_t) * std::min<uint32_t>(r, kRoundLogSize),
+                                          cudaMemcpyDeviceToHost, st));
+                if (r > kRoundLogSize)   // beyond the log: the live counter of the last enqueued round
+                    OCLR_CUDA(cudaMemcpyAsync(q.pinned + kRoundLogSize, counters + cstride * ((r - 1) & 1u), sizeof(uint32_t),
+                                              cudaMemcpyDeviceToHost, st));
+                OCLR_CUDA(cudaStreamSynchronize(st));
+                bool finished = false;
+                uint32_t needed = r;
+                if (r <= kRoundLogSize) {
+                    finished = q.pinned[r - 1] == 0;
+                    for (uint32_t k = 0; k < r; ++k)
+                        if (q.pinned[k] == 0) {   // the first round that queued no ray is the last one that had anything to do
+                            needed = k + 1;
+                            break;
+                        }
+                } else {
+                    finished = q.pinned[kRoundLogSize] == 0;
+                }
+                if (finished) {
+                    lastRounds = needed;
+                    break;
+                }
+                if (r > 100000) {
+                    err = "radiance query did not converge";
+                    return false;
+                }
+            }
+        }
+        radiance_resolve_kernel<<<rayGrid, 128, 0, st>>>(R, (const float4*)q.accum.p, (const uint32_t*)q.firstHit.p, sampleCount, result);
+        ++launches;
+        OCLR_CUDA(cudaGetLastError());
+        if (!deviceMemory && (!device_to_host(rgb4 + 4 * off, q.out.p, sizeof(float4) * n, st, err) ||
+                              (flags && !device_to_host(flags + off, q.flags.p, n, st, err))))
+            return false;
+    }
+    if (stats) {
+        OCLR_CUDA(cudaEventRecord(q.ev1, st));
+        OCLR_CUDA(cudaEventSynchronize(q.ev1));
+        OCLR_CUDA(cudaEventElapsedTime(&stats->deviceMs, q.ev0, q.ev1));
+        stats->launches = launches;
+        stats->traceLaunches = rounds;
+        if (dcnt) OCLR_CUDA(cudaMemcpy(&stats->counters, dcnt, sizeof(Counters), cudaMemcpyDeviceToHost));
+    }
+    return true;
 }
 
 }  // namespace oclr

@@ -182,5 +182,14 @@ bool scene_intersect(Scene* s, size_t count, const float* origin4, const float* 
                      bool deviceMemory, bool counting, void* stream, RenderStats* stats, std::string& err);
 bool scene_transmittance(Scene* s, size_t count, const float* origin4, const float* direction4, const uint32_t* excluded, float* att4,
                          bool deviceMemory, bool counting, void* stream, RenderStats* stats, std::string& err);
+// Radiance along caller rays (rt_query.cuh radiance_start_kernel + the frame's logic kernel; semantics in include/oclr_abi.h): the reference's pixel-sample loop
+// with the camera segment replaced by the ray, sampleCount samples, rgb4 = (mean rgb, as_float(first hit of sample 0)), flags optional
+// (cl_uchar per ray).  `cam` may be null when no material has a BUMP channel.  Rays are processed in batches of kRadianceBatch; the
+// call's path state is about 1 KB per ray of a batch with a 12-slot ring (432 B + 48 B per ring slot: ring, shading carry, two ray
+// slots, walk records, accumulator), about 1.1 GB for a full batch; host-memory inputs add 53 B per ray of staging.  Synchronous.
+enum { kRadianceBatch = 1 << 20 };
+bool scene_radiance(Scene* s, const Camera* cam, size_t count, const float* origin4, const float* direction4, const uint32_t* excluded,
+                    unsigned long long indexBase, uint32_t sampleCount, float* rgb4, uint8_t* flags, bool deviceMemory, bool counting,
+                    void* stream, RenderStats* stats, std::string& err);
 
 }  // namespace oclr

@@ -10,7 +10,12 @@ Defaults are the dialog's: 1024x768, 100 samples per pixel (render.cpp:176-182);
 The scene is uploaded once; camera lists and -- unless `--host-builders` -- the 256^3 grid are built on the device.  Samples are
 rendered in passes of `--pass-samples`; after every pass the dialog's three lines are printed (progress, estimated time left,
 rendering time) and, with `--preview`, the picture so far is written.  `--checkpoint FILE` saves the planes and the number of
-finished samples after every pass and resumes from the file when it exists."""
+finished samples after every pass and resumes from the file when it exists.
+
+`--projection equirect` renders a 360 x 180 degree panorama around the eye instead (what Cinema4D's spherical camera renders): one
+radiance query per pixel (DeviceScene.radiance), in chunks of rows, with `--samples` samples per pixel.  The panorama is level: `--up`
+is its pole, and longitude 0 looks towards the look-at point (projected onto the horizon).  The options of the pass loop (`--pass-samples`,
+`--preview`, `--checkpoint`, `--float-accum`) belong to the pinhole path and are refused with it."""
 from __future__ import annotations
 
 import argparse
@@ -57,6 +62,64 @@ def _time_str(seconds: float) -> str:
     return f"{s}s"
 
 
+def equirect_basis(eye, look_at, up):
+    """Orthonormal (right, up, forward) in float32 for a level panorama: up = unit(--up) is the pole, forward = the view direction with its
+    component along the pole removed, right = up x forward (the pinhole camera's left-to-right direction, builders.cpp set_camera)."""
+    f32 = lambda v: np.asarray(v, np.float32)[:3]
+    norm = lambda v: np.float32(np.sqrt(np.float32((v * v).sum())))
+    pole = f32(up) / norm(f32(up))
+    view = f32(look_at) - f32(eye)
+    horizontal = view - np.float32((view * pole).sum()) * pole
+    if not norm(horizontal) > np.float32(1e-6) * norm(view):
+        raise ValueError("the view direction is parallel to --up: the panorama has no horizontal reference direction")
+    forward = horizontal / norm(horizontal)
+    right = np.cross(pole, forward).astype(np.float32)
+    return right / norm(right), pole, forward
+
+
+def equirect_directions(basis, width: int, height: int, rows=None):
+    """Directions of rows [rows[0], rows[1]) of a width x height equirectangular panorama, float32 [n*W,3] row-major.  Pixel (x, y) has
+    longitude phi = 2 pi (x + 0.5) / W - pi and latitude theta = pi / 2 - pi (y + 0.5) / H; its direction is
+    cos(theta) sin(phi) right + sin(theta) up + cos(theta) cos(phi) forward.  The angle tables cover the whole image, so a chunk's
+    directions are bit for bit those of the whole panorama."""
+    right, up, forward = (np.asarray(v, np.float32) for v in basis)
+    y0, y1 = rows if rows is not None else (0, height)
+    x = np.arange(width, dtype=np.float32)
+    y = np.arange(height, dtype=np.float32)
+    phi = np.float32(2 * np.pi) * (x + np.float32(0.5)) / np.float32(width) - np.float32(np.pi)
+    theta = np.float32(np.pi / 2) - np.float32(np.pi) * (y + np.float32(0.5)) / np.float32(height)
+    ct, st = np.cos(theta)[y0:y1, None, None], np.sin(theta)[y0:y1, None, None]
+    cp, sp = np.cos(phi)[None, :, None], np.sin(phi)[None, :, None]
+    d = ct * sp * right + st * up + ct * cp * forward
+    return np.ascontiguousarray(d.reshape(-1, 3), np.float32)
+
+
+def planes_from_mean(rgb, width: int, rows: int):
+    """(int)(mean * 65535) clamped to 16 bits -- the frame's float-accumulation conversion -- as three uint16 [rows,W] planes."""
+    v = np.nan_to_num(np.asarray(rgb, np.float32) * np.float32(65535), nan=0.0, posinf=0.0, neginf=0.0)
+    v = np.clip(np.trunc(v), 0, 65535).astype(np.uint16)
+    return tuple(np.ascontiguousarray(v[:, c].reshape(rows, width)) for c in range(3))
+
+
+def render_equirect(ds: api.DeviceScene, cam: api.CameraSetup, basis, width: int, height: int, samples: int, say=lambda *x: None):
+    """The panorama's planes (r, g, b) uint16 [H,W]; sample s of pixel p = y * W + x is seeded p * samples + s + 1."""
+    planes = tuple(np.zeros((height, width), np.uint16) for _ in range(3))
+    chunk = max(1, api.RADIANCE_BATCH // width)
+    t0 = time.monotonic()
+    eye = np.asarray(cam.eye[:3], np.float32)
+    for y0 in range(0, height, chunk):
+        y1 = min(height, y0 + chunk)
+        d = equirect_directions(basis, width, height, (y0, y1))
+        o = np.broadcast_to(eye, d.shape)
+        rgb, _ = ds.radiance(o, d, samples=samples, index_base=y0 * width, camera=cam)
+        for p, q in zip(planes, planes_from_mean(rgb, width, y1 - y0)):
+            p[y0:y1] = q
+        el = time.monotonic() - t0
+        say(f"Rendering Progress {100 * y1 / height:.1f} %   Estimated Time Left {_time_str(el / y1 * (height - y1))}   "
+            f"Rendering Time {_time_str(el)}")
+    return planes
+
+
 def main(argv=None) -> int:
     ap = argparse.ArgumentParser(prog="python -m opencl_render_b200.render", description=__doc__.split("\n\n")[0])
     ap.add_argument("scene", nargs="?", help="OBJ / PLY file or config1..config4")
@@ -76,9 +139,16 @@ def main(argv=None) -> int:
     ap.add_argument("--preview", action="store_true", help="write --out after every pass")
     ap.add_argument("--checkpoint", help="file the job state is saved to after every pass / resumed from")
     ap.add_argument("--bmp-reference-cast", action="store_true", help="BMP bytes = low byte, like writebmp3s (writebmp.cpp:136-141)")
+    ap.add_argument("--projection", choices=["pinhole", "equirect"], default="pinhole",
+                    help="pinhole: the camera's own image; equirect: a 360 x 180 degree panorama around --eye")
     ap.add_argument("--quiet", action="store_true")
     a = ap.parse_args(argv)
     say = (lambda *x: None) if a.quiet else (lambda *x: print(*x, file=sys.stderr, flush=True))
+    if a.projection == "equirect":
+        for flag, given in (("--checkpoint", a.checkpoint), ("--float-accum", a.float_accum), ("--pass-samples", a.pass_samples),
+                            ("--preview", a.preview)):
+            if given:
+                ap.error(f"{flag} belongs to the pinhole pass loop and is not supported with --projection equirect")
 
     names = api.computation_types()
     if a.list_devices:
@@ -112,9 +182,20 @@ def main(argv=None) -> int:
     cam = api.set_camera(cm["eye"], cm["look_at"], cm["up"], cm["fov"], w, h)
     lists = None
     if a.host_builders:
-        lists = api.camera_triangle_list(cam, sc)
+        if a.projection == "pinhole":   # (a panorama reads no camera lists)
+            lists = api.camera_triangle_list(cam, sc)
         api.scene_triangle_list(sc, api.AXES_DIVISION)
     ds = api.DeviceScene(sc, a.device - 1)
+    if a.projection == "equirect":
+        say(f"{sc.name}: {sc.triangle_count} triangles, {sc.material_count} materials, {sc.light_count} lights on {names[a.device]}; "
+            f"scene & device prepare time {_time_str(time.monotonic() - t_prepare)} ({time.monotonic() - t_prepare:.2f} s)")
+        t0 = time.monotonic()
+        img = render_equirect(ds, cam, equirect_basis(cm["eye"], cm["look_at"], cm["up"]), w, h, a.samples, say)
+        el = time.monotonic() - t0
+        api.write_image(a.out, img, bmp_reference_cast=a.bmp_reference_cast)
+        say(f"{a.out}: {w}x{h} equirect, {a.samples} samples; {w * h * a.samples / max(el, 1e-9) / 1e6:.1f} Mpaths/s over {el:.2f} s")
+        ds.close()
+        return 0
     fr = api.DeviceFrame(ds, cam, lists)
     if a.float_accum:
         fr.set_accumulation(api.ACCUMULATE_FLOAT)
