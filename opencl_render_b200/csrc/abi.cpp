@@ -328,16 +328,21 @@ int oclr_frame_render(oclr_frame* frame, cl_uint sampleCount, cl_uint rowBegin, 
     return oclr_frame_render_samples(frame, sampleCount, 0, sampleCount, rowBegin, rowEnd, kernelVariant, countEvents, cudaStream, stats);
 }
 
-static int scene_query_entry(const char* name, bool transmit, oclr_scene* scene, size_t count, const cl_float* origin4, const cl_float* direction4,
-                             const cl_uint* excluded, cl_float* out4, int memory, int countEvents, void* cudaStream, oclr_render_stats* stats) {
+// What every query entry checks before the runtime does: a scene and a known memory kind.
+static bool query_entry_ok(const char* name, oclr_scene* scene, int memory) {
     if (!scene) {
         fail(std::string(name) + ": null scene");
-        return 0;
+        return false;
     }
     if (memory != OCLR_QUERY_HOST_MEMORY && memory != OCLR_QUERY_DEVICE_MEMORY) {
         fail(std::string(name) + ": unknown memory kind " + std::to_string(memory));
-        return 0;
+        return false;
     }
+    return true;
+}
+static int scene_query_entry(const char* name, bool transmit, oclr_scene* scene, size_t count, const cl_float* origin4, const cl_float* direction4,
+                             const cl_uint* excluded, cl_float* out4, int memory, int countEvents, void* cudaStream, oclr_render_stats* stats) {
+    if (!query_entry_ok(name, scene, memory)) return 0;
     std::string err;
     RenderStats rs;
     const bool dev = memory == OCLR_QUERY_DEVICE_MEMORY;
@@ -364,14 +369,7 @@ int oclr_scene_transmittance(oclr_scene* scene, size_t count, const cl_float* or
 int oclr_scene_radiance(oclr_scene* scene, const oclr_camera* camera, size_t count, const cl_float* origin4, const cl_float* direction4,
                         const cl_uint* excluded, unsigned long long indexBase, cl_uint sampleCount, cl_float* rgb4, cl_uchar* flags, int memory,
                         int countEvents, void* cudaStream, oclr_render_stats* stats) {
-    if (!scene) {
-        fail("oclr_scene_radiance: null scene");
-        return 0;
-    }
-    if (memory != OCLR_QUERY_HOST_MEMORY && memory != OCLR_QUERY_DEVICE_MEMORY) {
-        fail("oclr_scene_radiance: unknown memory kind " + std::to_string(memory));
-        return 0;
-    }
+    if (!query_entry_ok("oclr_scene_radiance", scene, memory)) return 0;
     std::string err;
     RenderStats rs;
     Camera cam;

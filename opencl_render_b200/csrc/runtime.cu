@@ -8,6 +8,7 @@
 #include <string.h>
 
 #include <algorithm>
+#include <array>
 #include <atomic>
 #include <chrono>
 #include <condition_variable>
@@ -661,30 +662,67 @@ struct Scene {
     bool hasBump = false;   // some material has a BUMP channel: its normals read the camera vectors (radiance queries need a camera)
 };
 
-// Wavefront path state of one slice of a launch domain (launch_wavefront): its own buffers, queue counters and stream, so
-// the rounds of different slices overlap on the GPU.
-enum { kMaxSlices = 8 };
-// per-round counters of a slice: {ray count, cursor, class counts[4], hand-off count, 0, 0, 0, hand-off cursor}, two sets alternating
-// between rounds ({hand-off count, 0, 0, 0} doubles as the class counts of the second pass over the rays given up, rt_tail.cuh)
+// per-round counters of a launch domain: {ray count, cursor, class counts[4], hand-off count, 0, 0, 0, hand-off cursor}, two sets
+// alternating between rounds ({hand-off count, 0, 0, 0} doubles as the class counts of the second pass over the rays given up, rt_tail.cuh)
 enum { kCounterStride = 2 + kLengthClasses + 5 };
-struct WfSlice {
+// Wavefront path state of one launch domain (rt_wavefront.cuh WfState, rt_trace.cuh WalkRecords) and its queue counters: stream-ordered
+// buffers for up to `capacity` paths, reallocated only when a domain of more paths comes along.
+struct PathState {
     DeviceBuffer ctl, rng, colour, ring, carry, rayO, rayD, rayExcl, hit, queue;
     DeviceBuffer recO, recD, recS0, recS1, recOrder;   // walk records in queue order + class order (rt_trace.cuh)
-    DeviceBuffer workCounter;                          // kCounterStride counters x 2, alternating between rounds; then the round log
+    DeviceBuffer counters;                             // kCounterStride counters x 2, alternating between rounds; then the round log
+    uint32_t capacity = 0;
+    std::array<DeviceBuffer*, 16> buffers() {
+        return {&ctl, &rng, &colour, &ring, &carry, &rayO, &rayD, &rayExcl, &hit, &queue, &recO, &recD, &recS0, &recS1, &recOrder, &counters};
+    }
+    bool reserve(uint32_t Q, int ringSlots, cudaStream_t st, std::string& err) {
+        if (Q <= capacity) return true;
+        release(st);
+        const size_t q = Q;
+        if (!ctl.alloc(sizeof(uint32_t) * q, err, st) || !rng.alloc(sizeof(uint64_t) * q, err, st) || !colour.alloc(sizeof(float4) * q, err, st) ||
+            !ring.alloc(sizeof(float4) * q * (size_t)ringSlots * kRingParts, err, st) || !carry.alloc(sizeof(float4) * q * kCarryParts, err, st) ||
+            // two ray slots per path (rt_wavefront.cuh: the next segment's closest hit is traced one round ahead)
+            !rayO.alloc(sizeof(float4) * 2 * q, err, st) || !rayD.alloc(sizeof(float4) * 2 * q, err, st) ||
+            !rayExcl.alloc(sizeof(uint32_t) * 2 * q, err, st) || !hit.alloc(sizeof(float4) * 2 * q, err, st) ||
+            !queue.alloc(sizeof(uint32_t) * 2 * q, err, st) || !recO.alloc(sizeof(float4) * 2 * q, err, st) ||
+            !recD.alloc(sizeof(float4) * 2 * q, err, st) || !recS0.alloc(sizeof(float4) * 2 * q, err, st) ||
+            !recS1.alloc(sizeof(uint4) * 2 * q, err, st) || !recOrder.alloc(sizeof(uint32_t) * 2 * q * kLengthClasses, err, st) ||
+            !counters.alloc(sizeof(uint32_t) * (2 * kCounterStride + kRoundLogSize), err, st))
+            return false;
+        capacity = Q;
+        return true;
+    }
+    void release(cudaStream_t st) {
+        for (DeviceBuffer* b : buffers()) b->release(st);
+        capacity = 0;
+    }
+    size_t bytes() {
+        size_t n = 0;
+        for (DeviceBuffer* b : buffers()) n += b->bytes;
+        return n;
+    }
+    uint32_t* counter_set(uint32_t round) const { return (uint32_t*)counters.p + kCounterStride * (round & 1u); }
+    // A domain of Q <= capacity paths; the queue counters are set per round (RoundDriver).
+    void bind(uint32_t Q, int ringSlots, WfState& w, WalkRecords& rec) const {
+        w = {Q, (uint32_t*)ctl.p, (uint64_t*)rng.p, (float4*)colour.p, (float4*)ring.p, (uint32_t)ringSlots, (float4*)carry.p, (float4*)rayO.p,
+             (float4*)rayD.p, (uint32_t*)rayExcl.p, (float4*)hit.p, (uint32_t*)queue.p, nullptr, nullptr, (uint32_t*)counters.p + 2 * kCounterStride, 0};
+        rec = {(float4*)recO.p, (float4*)recD.p, (float4*)recS0.p, (uint4*)recS1.p, (uint32_t*)recOrder.p, nullptr, 2 * Q};   // (two rays per path at most)
+    }
+};
+
+// One slice of a launch domain (launch_wavefront): its own path state and stream, so the rounds of different slices overlap on the GPU.
+enum { kMaxSlices = 8 };
+struct WfSlice {
+    PathState ps;
     DeviceBuffer tailEntries;                          // hand-off list of a small launch's trace tail (rt_tail.cuh); unallocated for large domains
     DeviceBuffer tailO, tailD, tailS0, tailS1, tailOrder;   // ... as walk records, for the second pass (hand-off mode 2)
     uint32_t tailCapacity = 0;
-    uint32_t capacity = 0;
     uint32_t lastRounds = 4;          // rounds the previous sample needed (first chunk of the next one)
     cudaStream_t stream = nullptr;    // internal stream (slice 0 runs on the caller's stream)
     cudaEvent_t done = nullptr;
     std::vector<cudaEvent_t> traceEvents;   // pairs around the trace launches of the last timed render
     uint32_t traceEventsUsed = 0;
-    DeviceBuffer* buffers(int i) {
-        DeviceBuffer* all[] = {&ctl, &rng, &colour, &ring, &carry, &rayO, &rayD, &rayExcl, &hit, &queue, &recO, &recD, &recS0, &recS1,
-                               &recOrder, &workCounter, &tailEntries, &tailO, &tailD, &tailS0, &tailS1, &tailOrder};
-        return i < 22 ? all[i] : nullptr;
-    }
+    std::array<DeviceBuffer*, 6> tail_buffers() { return {&tailEntries, &tailO, &tailD, &tailS0, &tailS1, &tailOrder}; }
 };
 
 struct Frame {
@@ -1263,8 +1301,10 @@ size_t scene_device_bytes(const Scene* s) { return s->bytes; }
 // of `capacity` paths costs; 0 before the first render.
 size_t frame_state_bytes(Frame* f) {
     size_t n = 0;
-    for (WfSlice& sl : f->slices)
-        for (int i = 0; sl.buffers(i); ++i) n += sl.buffers(i)->bytes;
+    for (WfSlice& sl : f->slices) {
+        n += sl.ps.bytes();
+        for (DeviceBuffer* b : sl.tail_buffers()) n += b->bytes;
+    }
     return n;
 }
 
@@ -1510,7 +1550,8 @@ void frame_destroy(Frame* f) {
     drop_event(f->device, f->preReady, false);
     drop_event(f->device, f->preDone, false);
     for (WfSlice& sl : f->slices) {
-        for (int i = 0; sl.buffers(i); ++i) sl.buffers(i)->release();
+        sl.ps.release(0);
+        for (DeviceBuffer* b : sl.tail_buffers()) b->release();
         drop_stream(f->device, sl.stream);
         drop_event(f->device, sl.done, false);
         for (cudaEvent_t e : sl.traceEvents) drop_event(f->device, e, true);
@@ -1660,6 +1701,146 @@ static void enqueue_trace(const SceneView& S, const WfState& w, const WalkRecord
     ++launches;
 }
 
+// Every walk of the trace stage is the packed walk (rt_walk.h).
+static bool packed_walk_ok(const SceneView& S, std::string& err) {
+    if (S.n > 1024) {
+        err = "axesDivCount > 1024 is not supported by the packed walk";
+        return false;
+    }
+    return true;
+}
+
+// ---- the round driver of the path state machine (rt_wavefront.cuh), shared by frames and radiance queries ---------------------------
+// One launch domain: its bound path state, stream and round history.
+struct RoundDomain {
+    const PathState* ps = nullptr;
+    WfState w = {};       // ps bound (PathState::bind); the driver points the queue counters at each round's set
+    WalkRecords rec = {};
+    TailQueue tail = {};  // hand-off buffers of the trace tail (capacity 0: none); the driver points its counters at each round's set
+    cudaStream_t st = nullptr;
+    uint32_t* lastRounds = nullptr;                    // rounds the previous sample needed: the length of the next one's first chunk
+    std::vector<cudaEvent_t>* traceEvents = nullptr;   // set: a timing event pair around every round's trace stage
+    uint32_t* traceEventsUsed = nullptr;
+};
+// Enqueues the entry kernel(s) of round r of domain k on `ks`, behind the clearing of the round's counter set; `prev` is the previous
+// round's set (null at r = 0).  Counted as one launch.
+using RoundEntry = std::function<void(int k, uint32_t r, const WfState& w, const uint32_t* prev, cudaStream_t ks)>;
+struct RoundDriver {
+    const SceneView& S;
+    int device, smCount;
+    unsigned traceGrid;
+    Counters* dcnt;
+    uint32_t* host;           // pinned: per domain kRoundLogSize + 1 words, then the camera-check word
+    const uint32_t* camBad;   // optional device word read back with every chunk's round logs (FrameView::camBad)
+    const char* what;         // "<what> did not converge"
+    int K = 0;
+    RoundDomain dom[kMaxSlices];
+    uint32_t launches = 0, rounds = 0;
+    bool run(cudaEvent_t resume, const RoundEntry& entry, std::string& err);
+};
+static_assert(sizeof(uint32_t) * (kMaxSlices * (kRoundLogSize + 1) + 1) <= 4096, "round logs + camera-check word fit one pinned block");
+
+// Rounds of one sample (entry -> setup -> trace) until no path of any domain waits for a ray.  Rounds are enqueued ahead in chunks
+// without a host round trip: every kernel reads the ray count of its round from device memory and returns at once when there is
+// nothing to do.  The host reads the round log once per chunk; the first chunk is as long as the previous sample needed.  Domains are
+// enqueued round by round, alternating, so that their launches interleave on the device.  `resume`: round 0 of domain 0 was enqueued
+// ahead (frame_prelaunch) and has already queued its rays; the stream waits for it instead of clearing the counters and entering again.
+bool RoundDriver::run(cudaEvent_t resume, const RoundEntry& entry, std::string& err) {
+    uint32_t round[kMaxSlices] = {0};
+    bool live[kMaxSlices];
+    unsigned setupGrid[kMaxSlices];
+    for (int k = 0; k < K; ++k) {
+        live[k] = true;
+        setupGrid[k] = (unsigned)std::min<uint64_t>((uint64_t)smCount * 8, (2 * (uint64_t)dom[k].w.Q + 255) / 256);
+    }
+    for (;;) {
+        uint32_t chunk[kMaxSlices], maxChunk = 0;
+        for (int k = 0; k < K; ++k) {
+            chunk[k] = !live[k] ? 0u : (round[k] == 0 ? std::max<uint32_t>(*dom[k].lastRounds, 2) : 2u);
+            maxChunk = std::max(maxChunk, chunk[k]);
+        }
+        if (maxChunk == 0) return true;
+        for (uint32_t c = 0; c < maxChunk; ++c) {
+            for (int k = 0; k < K; ++k) {
+                if (c >= chunk[k]) continue;
+                RoundDomain& d = dom[k];
+                const uint32_t r = round[k];
+                d.w.queueCount = d.ps->counter_set(r);
+                d.w.queueCursor = d.w.queueCount + 1;
+                d.w.roundIndex = r;
+                d.rec.classCount = d.w.queueCount + 2;
+                d.tail.count = d.w.queueCount + 2 + kLengthClasses;
+                d.tail.cursor = d.w.queueCount + 6 + kLengthClasses;
+                if (resume && k == 0 && r == 0) {
+                    OCLR_CUDA(cudaStreamWaitEvent(d.st, resume, 0));
+                } else {
+                    OCLR_CUDA(cudaMemsetAsync(d.w.queueCount, 0, sizeof(uint32_t) * kCounterStride, d.st));
+                    entry(k, r, d.w, r ? d.ps->counter_set(r - 1) : nullptr, d.st);
+                    ++launches;
+                }
+                if (d.traceEvents) {
+                    while (d.traceEvents->size() < (size_t)*d.traceEventsUsed + 2) {
+                        cudaEvent_t e;
+                        OCLR_CUDA(make_event(device, &e, true));
+                        d.traceEvents->push_back(e);
+                    }
+                    OCLR_CUDA(cudaEventRecord((*d.traceEvents)[*d.traceEventsUsed], d.st));
+                }
+                enqueue_trace(S, d.w, d.rec, d.tail, setupGrid[k], traceGrid, smCount, dcnt, d.st, launches);
+                if (d.traceEvents) {
+                    OCLR_CUDA(cudaEventRecord((*d.traceEvents)[*d.traceEventsUsed + 1], d.st));
+                    *d.traceEventsUsed += 2;
+                }
+                ++round[k];
+                ++rounds;
+            }
+        }
+        // one read per chunk: the round log (rays queued by every round so far; the last enqueued round decides) and, beyond the log,
+        // the live counter of the last enqueued round
+        for (int k = 0; k < K; ++k) {
+            if (!chunk[k]) continue;
+            uint32_t* log = host + k * (kRoundLogSize + 1);
+            OCLR_CUDA(cudaMemcpyAsync(log, dom[k].w.roundLog, sizeof(uint32_t) * std::min<uint32_t>(round[k], kRoundLogSize),
+                                      cudaMemcpyDeviceToHost, dom[k].st));
+            if (round[k] > kRoundLogSize)
+                OCLR_CUDA(cudaMemcpyAsync(log + kRoundLogSize, dom[k].ps->counter_set(round[k] - 1), sizeof(uint32_t), cudaMemcpyDeviceToHost,
+                                          dom[k].st));
+        }
+        uint32_t* camFlag = host + kMaxSlices * (kRoundLogSize + 1);
+        *camFlag = 0;
+        if (camBad) OCLR_CUDA(cudaMemcpyAsync(camFlag, camBad, sizeof(uint32_t), cudaMemcpyDeviceToHost, dom[0].st));
+        for (int k = 0; k < K; ++k)
+            if (chunk[k]) OCLR_CUDA(cudaStreamSynchronize(dom[k].st));
+        if (*camFlag) {
+            err = cam_check_message(*camFlag);
+            return false;
+        }
+        for (int k = 0; k < K; ++k) {
+            if (!chunk[k]) continue;
+            const uint32_t* log = host + k * (kRoundLogSize + 1);
+            bool finished = false;
+            uint32_t needed = round[k];
+            if (round[k] <= kRoundLogSize) {
+                finished = log[round[k] - 1] == 0;
+                for (uint32_t r = 0; r < round[k]; ++r)
+                    if (log[r] == 0) {   // the first round that queued no ray is the last one that had anything to do
+                        needed = r + 1;
+                        break;
+                    }
+            } else {
+                finished = log[kRoundLogSize] == 0;
+            }
+            if (finished) {
+                live[k] = false;
+                *dom[k].lastRounds = needed;
+            } else if (round[k] > 100000) {
+                err = std::string(what) + " did not converge";
+                return false;
+            }
+        }
+    }
+}
+
 // Wavefront driver: alternate the logic and trace kernels until no path is waiting for a ray (rt_wavefront.cuh).
 // `prelaunchOnly`: allocate the path state and enqueue nothing but the first logic round of the first sample, on the frame's own
 // stream behind everything already enqueued on `st` (frame_prelaunch).  A later normal call with the same view finds
@@ -1674,10 +1855,7 @@ static bool handoff_domain(uint32_t Q) {
 static bool launch_wavefront(Frame* f, const SceneView& S, const FrameView& Fall, int smCount, Counters* dcnt, cudaStream_t st,
                              uint32_t& launches, bool timeTrace, std::string& err, bool prelaunchOnly = false) {
     const uint32_t W = Fall.cam.width;
-    if (S.n > 1024) {
-        err = "axesDivCount > 1024 is not supported by the packed walk";
-        return false;
-    }
+    if (!packed_walk_ok(S, err)) return false;
     // ---- cut the launch domain into slices -------------------------------------------------------------------------------------------
     const uint32_t rowsAll = launch_rows(Fall);
     int K = slice_count_for(rowsAll, W);
@@ -1711,12 +1889,10 @@ static bool launch_wavefront(Frame* f, const SceneView& S, const FrameView& Fall
     }
     if (prelaunchOnly && K != 1) return true;   // (only the one-slice case is started ahead)
 
-    WfState w[kMaxSlices];
-    WalkRecords rec[kMaxSlices];
+    RoundDriver drv = {S, f->device, smCount, 0u, dcnt, nullptr, Fall.camBad, "wavefront"};
+    drv.K = K;
     dim3 logicGrid[kMaxSlices];
-    unsigned setupGrid[kMaxSlices];
     int aheadMode[kMaxSlices];
-    cudaStream_t stream[kMaxSlices];
     for (int k = 0; k < K; ++k) {
         WfSlice& sl = f->slices[k];
         const uint32_t rows = launch_rows(FV[k]);
@@ -1726,67 +1902,45 @@ static bool launch_wavefront(Frame* f, const SceneView& S, const FrameView& Fall
             return false;
         }
         const uint32_t Q = (uint32_t)Q64;
-        if (Q > sl.capacity) {
-            for (int i = 0; sl.buffers(i); ++i) sl.buffers(i)->release(st);
-            const size_t q = Q;
-            if (!sl.ctl.alloc(sizeof(uint32_t) * q, err, st) || !sl.rng.alloc(sizeof(uint64_t) * q, err, st) ||
-                !sl.colour.alloc(sizeof(float4) * q, err, st) || !sl.ring.alloc(sizeof(float4) * q * (size_t)f->scene->ringSlots * kRingParts, err, st) ||
-                !sl.carry.alloc(sizeof(float4) * q * kCarryParts, err, st) ||
-                // two ray slots per path (rt_wavefront.cuh: the next segment's closest hit is traced one round ahead)
-                !sl.rayO.alloc(sizeof(float4) * 2 * q, err, st) || !sl.rayD.alloc(sizeof(float4) * 2 * q, err, st) ||
-                !sl.rayExcl.alloc(sizeof(uint32_t) * 2 * q, err, st) || !sl.hit.alloc(sizeof(float4) * 2 * q, err, st) ||
-                !sl.queue.alloc(sizeof(uint32_t) * 2 * q, err, st) || !sl.recO.alloc(sizeof(float4) * 2 * q, err, st) ||
-                !sl.recD.alloc(sizeof(float4) * 2 * q, err, st) || !sl.recS0.alloc(sizeof(float4) * 2 * q, err, st) ||
-                !sl.recS1.alloc(sizeof(uint4) * 2 * q, err, st) || !sl.recOrder.alloc(sizeof(uint32_t) * 2 * q * kLengthClasses, err, st) ||
-                !sl.workCounter.alloc(sizeof(uint32_t) * (2 * kCounterStride + kRoundLogSize), err, st))
-                return false;
+        if (Q > sl.ps.capacity) {
+            for (DeviceBuffer* b : sl.tail_buffers()) b->release(st);
+            if (!sl.ps.reserve(Q, f->scene->ringSlots, st, err)) return false;
             sl.tailCapacity = 0;
             if (handoff_domain(Q)) {   // small launch domain: its trace tail is handed to wf_tail_kernel (rt_tail.cuh)
-                sl.tailCapacity = (uint32_t)(2 * q);   // (every ray of a round could be given up: the list cannot overflow)
+                sl.tailCapacity = 2 * Q;   // (every ray of a round could be given up: the list cannot overflow)
                 const size_t c = sl.tailCapacity;
                 if (!sl.tailEntries.alloc(sizeof(uint4) * c, err, st) || !sl.tailO.alloc(sizeof(float4) * c, err, st) ||
                     !sl.tailD.alloc(sizeof(float4) * c, err, st) || !sl.tailS0.alloc(sizeof(float4) * c, err, st) ||
                     !sl.tailS1.alloc(sizeof(uint4) * c, err, st) || !sl.tailOrder.alloc(sizeof(uint32_t) * c, err, st))
                     return false;
             }
-            sl.capacity = Q;
         }
         if (k > 0 && !sl.stream) OCLR_CUDA(make_stream(f->device, &sl.stream));
         if (!sl.done) OCLR_CUDA(make_event(f->device, &sl.done, false));
-        stream[k] = k == 0 ? st : sl.stream;
         sl.traceEventsUsed = 0;
-        w[k].Q = Q;
-        w[k].ctl = (uint32_t*)sl.ctl.p;
-        w[k].rng = (uint64_t*)sl.rng.p;
-        w[k].colour = (float4*)sl.colour.p;
-        w[k].ring = (float4*)sl.ring.p;
-        w[k].ringSlots = (uint32_t)f->scene->ringSlots;
-        w[k].carry = (float4*)sl.carry.p;
-        w[k].rayO = (float4*)sl.rayO.p;
-        w[k].rayD = (float4*)sl.rayD.p;
-        w[k].rayExcl = (uint32_t*)sl.rayExcl.p;
-        w[k].hit = (float4*)sl.hit.p;
-        w[k].queue = (uint32_t*)sl.queue.p;
-        rec[k].o = (float4*)sl.recO.p;
-        rec[k].d = (float4*)sl.recD.p;
-        rec[k].s0 = (float4*)sl.recS0.p;
-        rec[k].s1 = (uint4*)sl.recS1.p;
-        rec[k].order = (uint32_t*)sl.recOrder.p;
-        rec[k].Q = 2 * Q;   // queue slots (two rays per path at most)
+        RoundDomain& d = drv.dom[k];
+        d.ps = &sl.ps;
+        sl.ps.bind(Q, f->scene->ringSlots, d.w, d.rec);
+        d.tail = {(uint4*)sl.tailEntries.p, nullptr, nullptr, sl.tailCapacity, (float4*)sl.tailO.p, (float4*)sl.tailD.p, (float4*)sl.tailS0.p,
+                  (uint4*)sl.tailS1.p, (uint32_t*)sl.tailOrder.p};
+        d.st = k == 0 ? st : sl.stream;
+        d.lastRounds = &sl.lastRounds;
+        if (timeTrace) {
+            d.traceEvents = &sl.traceEvents;
+            d.traceEventsUsed = &sl.traceEventsUsed;
+        }
         aheadMode[k] = ahead_mode_for(Q);
         logicGrid[k] = dim3((W + 15) / 16, (rows + 7) / 8);
-        setupGrid[k] = (unsigned)std::min<uint64_t>((uint64_t)smCount * 8, (2 * (uint64_t)Q + 255) / 256);
     }
     for (int k = K; k < kMaxSlices; ++k) f->slices[k].traceEventsUsed = 0;
-    static_assert(sizeof(uint32_t) * (kMaxSlices * kRoundLogSize + 1) <= 4096, "round logs + camera-check word fit one pinned block");
     if (!f->hostCount) f->hostCount = (uint32_t*)pinned_block();
     if (!f->hostCount) {
         err = "out of pinned host memory";
         return false;
     }
+    drv.host = f->hostCount;
 
-    unsigned traceGrid = 0;
-    if (!trace_grid(S, smCount, dcnt != nullptr, traceGrid, err)) return false;
+    if (!trace_grid(S, smCount, dcnt != nullptr, drv.traceGrid, err)) return false;
     if (Fall.flagOut && !resumePre) OCLR_CUDA(cudaMemsetAsync(Fall.flagOut, 0, (size_t)Fall.cam.width * Fall.cam.height, st));
     if (prelaunchOnly) {
         if (!f->preStream) {
@@ -1794,16 +1948,13 @@ static bool launch_wavefront(Frame* f, const SceneView& S, const FrameView& Fall
             OCLR_CUDA(make_event(f->device, &f->preReady, false));
             OCLR_CUDA(make_event(f->device, &f->preDone, false));
         }
-        WfSlice& sl = f->slices[0];
-        uint32_t* counters = (uint32_t*)sl.workCounter.p;
-        w[0].queueCount = counters;
-        w[0].queueCursor = counters + 1;
-        w[0].roundLog = counters + 2 * kCounterStride;
-        w[0].roundIndex = 0;
+        WfState& w = drv.dom[0].w;
+        w.queueCount = f->slices[0].ps.counter_set(0);
+        w.queueCursor = w.queueCount + 1;
         OCLR_CUDA(cudaEventRecord(f->preReady, st));
         OCLR_CUDA(cudaStreamWaitEvent(f->preStream, f->preReady, 0));
-        OCLR_CUDA(cudaMemsetAsync(w[0].queueCount, 0, sizeof(uint32_t) * kCounterStride, f->preStream));
-        wf_logic_kernel<false><<<logicGrid[0], 128, 0, f->preStream>>>(S, FV[0], w[0], Fall.sampleBegin, 1u, nullptr, nullptr, aheadMode[0]);
+        OCLR_CUDA(cudaMemsetAsync(w.queueCount, 0, sizeof(uint32_t) * kCounterStride, f->preStream));
+        wf_logic_kernel<false><<<logicGrid[0], 128, 0, f->preStream>>>(S, FV[0], w, Fall.sampleBegin, 1u, nullptr, nullptr, aheadMode[0]);
         OCLR_CUDA(cudaGetLastError());
         OCLR_CUDA(cudaEventRecord(f->preDone, f->preStream));
         f->prelaunched = true;
@@ -1814,113 +1965,24 @@ static bool launch_wavefront(Frame* f, const SceneView& S, const FrameView& Fall
     // fork: the internal streams start after everything already enqueued on the caller's stream
     if (K > 1) {
         OCLR_CUDA(cudaEventRecord(f->evFork, st));
-        for (int k = 1; k < K; ++k) OCLR_CUDA(cudaStreamWaitEvent(stream[k], f->evFork, 0));
+        for (int k = 1; k < K; ++k) OCLR_CUDA(cudaStreamWaitEvent(drv.dom[k].st, f->evFork, 0));
     }
-    // Rounds (logic -> setup -> trace) are enqueued ahead in chunks without a host round trip: every kernel reads the ray count
-    // of its round from device memory and returns at once when there is nothing to do.  The host looks at the count of the last
-    // enqueued round once per chunk; the first chunk is as long as the previous sample / frame needed.  Slices are enqueued round
-    // by round, alternating, so that their launches interleave on the device.
-    const uint32_t cstride = kCounterStride;
     for (uint32_t s = Fall.sampleBegin; s < Fall.sampleEnd; ++s) {
-        uint32_t round[kMaxSlices] = {0};
-        bool live[kMaxSlices];
-        for (int k = 0; k < K; ++k) live[k] = true;
-        for (;;) {
-            uint32_t chunk[kMaxSlices], maxChunk = 0;
-            for (int k = 0; k < K; ++k) {
-                chunk[k] = !live[k] ? 0u : (round[k] == 0 ? std::max<uint32_t>(f->slices[k].lastRounds, 2) : 2u);
-                maxChunk = std::max(maxChunk, chunk[k]);
-            }
-            if (maxChunk == 0) break;
-            for (uint32_t c = 0; c < maxChunk; ++c) {
-                for (int k = 0; k < K; ++k) {
-                    if (c >= chunk[k]) continue;
-                    WfSlice& sl = f->slices[k];
-                    cudaStream_t ks = stream[k];
-                    uint32_t* counters = (uint32_t*)sl.workCounter.p;
-                    const uint32_t r = round[k];
-                    w[k].queueCount = counters + cstride * (r & 1u);
-                    w[k].queueCursor = w[k].queueCount + 1;
-                    rec[k].classCount = w[k].queueCount + 2;
-                    w[k].roundLog = counters + 2 * cstride;
-                    w[k].roundIndex = r;
-                    const uint32_t* prev = r ? counters + cstride * ((r - 1) & 1u) : nullptr;
-                    if (resumePre && f->prelaunched && s == Fall.sampleBegin && r == 0) {
-                        // this round's logic kernel is already running (or done) on the frame's own stream: frame_prelaunch
-                        OCLR_CUDA(cudaStreamWaitEvent(ks, f->preDone, 0));
-                        f->prelaunched = false;
-                    } else {
-                        OCLR_CUDA(cudaMemsetAsync(w[k].queueCount, 0, sizeof(uint32_t) * cstride, ks));
-                        if (dcnt)
-                            wf_logic_kernel<true><<<logicGrid[k], 128, 0, ks>>>(S, FV[k], w[k], s, r == 0 ? 1u : 0u, prev, dcnt, aheadMode[k]);
-                        else
-                            wf_logic_kernel<false><<<logicGrid[k], 128, 0, ks>>>(S, FV[k], w[k], s, r == 0 ? 1u : 0u, prev, dcnt, aheadMode[k]);
-                        ++launches;
-                    }
-                    if (timeTrace) {
-                        while (sl.traceEvents.size() < (size_t)sl.traceEventsUsed + 2) {
-                            cudaEvent_t e;
-                            OCLR_CUDA(make_event(f->device, &e, true));
-                            sl.traceEvents.push_back(e);
-                        }
-                        OCLR_CUDA(cudaEventRecord(sl.traceEvents[sl.traceEventsUsed], ks));
-                    }
-                    TailQueue tq = {(uint4*)sl.tailEntries.p, w[k].queueCount + 2 + kLengthClasses, w[k].queueCount + 6 + kLengthClasses,
-                                    sl.tailCapacity, (float4*)sl.tailO.p, (float4*)sl.tailD.p, (float4*)sl.tailS0.p, (uint4*)sl.tailS1.p,
-                                    (uint32_t*)sl.tailOrder.p};
-                    enqueue_trace(S, w[k], rec[k], tq, setupGrid[k], traceGrid, smCount, dcnt, ks, launches);
-                    if (timeTrace) {
-                        OCLR_CUDA(cudaEventRecord(sl.traceEvents[sl.traceEventsUsed + 1], ks));
-                        sl.traceEventsUsed += 2;
-                    }
-                    ++round[k];
-                }
-            }
-            // one read per chunk: the round log (rays queued by every round so far; the last enqueued round decides)
-            for (int k = 0; k < K; ++k)
-                if (chunk[k])
-                    OCLR_CUDA(cudaMemcpyAsync(f->hostCount + k * kRoundLogSize, (uint32_t*)f->slices[k].workCounter.p + 2 * cstride,
-                                              sizeof(uint32_t) * std::min<uint32_t>(round[k], kRoundLogSize), cudaMemcpyDeviceToHost, stream[k]));
-            uint32_t* camFlag = f->hostCount + kMaxSlices * kRoundLogSize;   // (same pinned block, behind the round logs)
-            *camFlag = 0;
-            if (Fall.camBad) OCLR_CUDA(cudaMemcpyAsync(camFlag, Fall.camBad, sizeof(uint32_t), cudaMemcpyDeviceToHost, stream[0]));
-            for (int k = 0; k < K; ++k)
-                if (chunk[k]) OCLR_CUDA(cudaStreamSynchronize(stream[k]));
-            if (*camFlag) {
-                err = cam_check_message(*camFlag);
-                return false;
-            }
-            for (int k = 0; k < K; ++k) {
-                if (!chunk[k]) continue;
-                const uint32_t* log = f->hostCount + k * kRoundLogSize;
-                bool finished = false;
-                uint32_t needed = round[k];
-                if (round[k] <= kRoundLogSize) {
-                    finished = log[round[k] - 1] == 0;
-                    for (uint32_t r = 0; r < round[k]; ++r)
-                        if (log[r] == 0) {   // the first round that queued no ray is the last one that had anything to do
-                            needed = r + 1;
-                            break;
-                        }
-                } else {   // beyond the log: fall back to the live counter of the last enqueued round
-                    uint32_t last = 1;
-                    OCLR_CUDA(cudaMemcpy(&last, (uint32_t*)f->slices[k].workCounter.p + cstride * ((round[k] - 1) & 1u), sizeof(uint32_t),
-                                         cudaMemcpyDeviceToHost));
-                    finished = last == 0;
-                }
-                if (finished) {
-                    live[k] = false;
-                    f->slices[k].lastRounds = needed;
-                } else if (round[k] > 100000) {
-                    err = "wavefront did not converge";
-                    return false;
-                }
-            }
-        }
+        const RoundEntry logic = [&](int k, uint32_t r, const WfState& w, const uint32_t* prev, cudaStream_t ks) {
+            if (dcnt)
+                wf_logic_kernel<true><<<logicGrid[k], 128, 0, ks>>>(S, FV[k], w, s, r == 0 ? 1u : 0u, prev, dcnt, aheadMode[k]);
+            else
+                wf_logic_kernel<false><<<logicGrid[k], 128, 0, ks>>>(S, FV[k], w, s, r == 0 ? 1u : 0u, prev, dcnt, aheadMode[k]);
+        };
+        // the first logic round of the request may already be running (or done) on the frame's own stream: frame_prelaunch
+        const cudaEvent_t resume = resumePre && s == Fall.sampleBegin ? f->preDone : nullptr;
+        if (resume) f->prelaunched = false;
+        if (!drv.run(resume, logic, err)) return false;
     }
+    launches += drv.launches;
     // join: later work on the caller's stream (plane reads, gathers) follows every slice
     for (int k = 1; k < K; ++k) {
-        OCLR_CUDA(cudaEventRecord(f->slices[k].done, stream[k]));
+        OCLR_CUDA(cudaEventRecord(f->slices[k].done, drv.dom[k].st));
         OCLR_CUDA(cudaStreamWaitEvent(st, f->slices[k].done, 0));
     }
     return true;
@@ -2444,74 +2506,137 @@ static bool query_pointer_ok(const Scene* s, const void* p, size_t align, const 
     return true;
 }
 
-// Scratch of one query call: stream-ordered allocations, released on the query's stream whichever way the call ends, so that queries
-// on one scene from different streams share nothing.
-struct QueryScratch {
-    DeviceBuffer recO, recD, recS0, recS1, order, queue, excl, counters, stats, hit, rayO, inO, inD, inExcl, out;
-    cudaStream_t st = nullptr;
-    int device = 0;
+// Caller rays of one query call (scene_query, scene_radiance): the argument checks, the host-memory staging of each batch, the result
+// download and the call's statistics.  Buffers are stream-ordered and released on the call's stream whichever way the call ends, so that
+// calls on one scene from different streams share nothing.
+struct CallerRays {
+    Scene* s;
+    size_t count;
+    const float* origin4;
+    const float* direction4;
+    const uint32_t* excluded;
+    float* out4;
+    uint8_t* flags;   // radiance's optional per-ray flags
+    bool deviceMemory;
+    cudaStream_t st;
+    DeviceBuffer inO, inD, inExcl, out, outFlags, counters;
+    Counters* dcnt = nullptr;
     cudaEvent_t ev0 = nullptr, ev1 = nullptr;
-    uint32_t* pinned = nullptr;   // transmittance: rays the last enqueued round queued again, read back once per chunk
-    ~QueryScratch() {
-        for (DeviceBuffer* b : {&recO, &recD, &recS0, &recS1, &order, &queue, &excl, &counters, &stats, &hit, &rayO, &inO, &inD, &inExcl, &out})
-            b->release(st);
-        drop_event(device, ev0, true);
-        drop_event(device, ev1, true);
+    uint32_t* pinned = nullptr;   // read-back words of the call's rounds
+    ~CallerRays() {
+        for (DeviceBuffer* b : {&inO, &inD, &inExcl, &out, &outFlags, &counters}) b->release(st);
+        if (s) {
+            drop_event(s->device, ev0, true);
+            drop_event(s->device, ev1, true);
+        }
         pinned_release(pinned);
+    }
+    // True with nothing checked beyond the scene when there are no rays.
+    bool check(const char* outName, RenderStats* stats, std::string& err) {
+        if (!s) {
+            err = "null scene";
+            return false;
+        }
+        if (stats) *stats = RenderStats();
+        if (count == 0) return true;
+        if (!origin4 || !direction4 || !out4) {
+            err = "null origin, direction or output array";
+            return false;
+        }
+        OCLR_CUDA(cudaSetDevice(s->device));
+        if (deviceMemory && (!query_pointer_ok(s, origin4, 16, "origin", err) || !query_pointer_ok(s, direction4, 16, "direction", err) ||
+                             !query_pointer_ok(s, out4, 16, outName, err) || (excluded && !query_pointer_ok(s, excluded, 4, "excluded", err)) ||
+                             (flags && !query_pointer_ok(s, flags, 1, "flags", err))))
+            return false;
+        return packed_walk_ok(s->view, err);
+    }
+    // Staging for batches of up to b rays and the counters block, then the start of the call's timing.
+    bool begin(size_t b, bool counting, RenderStats* stats, std::string& err) {
+        if ((counting && !counters.alloc(sizeof(Counters), err, st)) ||
+            (!deviceMemory && (!inO.alloc(sizeof(float4) * b, err, st) || !inD.alloc(sizeof(float4) * b, err, st) ||
+                               (excluded && !inExcl.alloc(sizeof(uint32_t) * b, err, st)) || !out.alloc(sizeof(float4) * b, err, st) ||
+                               (flags && !outFlags.alloc(b, err, st)))))
+            return false;
+        dcnt = counting ? (Counters*)counters.p : nullptr;
+        if (dcnt) OCLR_CUDA(cudaMemsetAsync(dcnt, 0, sizeof(Counters), st));
+        if (stats) {
+            OCLR_CUDA(make_event(s->device, &ev0, true));
+            OCLR_CUDA(make_event(s->device, &ev1, true));
+            OCLR_CUDA(cudaEventRecord(ev0, st));
+        }
+        return true;
+    }
+    // The rays of batch [off, off + n) as device arrays (host memory: uploaded into the staging buffers).
+    bool rays(size_t off, uint32_t n, const float4*& origin, const float4*& direction, const uint32_t*& excl, std::string& err) {
+        if (deviceMemory) {
+            origin = (const float4*)origin4 + off;
+            direction = (const float4*)direction4 + off;
+            excl = excluded ? excluded + off : nullptr;
+            return true;
+        }
+        if (!host_to_device(inO.p, origin4 + 4 * off, sizeof(float4) * n, st, err) ||
+            !host_to_device(inD.p, direction4 + 4 * off, sizeof(float4) * n, st, err) ||
+            (excluded && !host_to_device(inExcl.p, excluded + off, sizeof(uint32_t) * n, st, err)))
+            return false;
+        origin = (const float4*)inO.p;
+        direction = (const float4*)inD.p;
+        excl = excluded ? (const uint32_t*)inExcl.p : nullptr;
+        return true;
+    }
+    float4* result(size_t off) const { return deviceMemory ? (float4*)out4 + off : (float4*)out.p; }
+    uint8_t* flag_out(size_t off) const { return !flags ? nullptr : deviceMemory ? flags + off : (uint8_t*)outFlags.p; }
+    // Results of batch [off, off + n) back to host memory (device memory is written in place).
+    bool download(size_t off, uint32_t n, std::string& err) {
+        return deviceMemory || (device_to_host(out4 + 4 * off, out.p, sizeof(float4) * n, st, err) &&
+                                (!flags || device_to_host(flags + off, outFlags.p, n, st, err)));
+    }
+    bool finish(RenderStats* stats, uint32_t launches, uint32_t rounds, std::string& err) {
+        if (!stats) return true;
+        OCLR_CUDA(cudaEventRecord(ev1, st));
+        OCLR_CUDA(cudaEventSynchronize(ev1));
+        OCLR_CUDA(cudaEventElapsedTime(&stats->deviceMs, ev0, ev1));
+        stats->launches = launches;
+        stats->traceLaunches = rounds;
+        if (dcnt) OCLR_CUDA(cudaMemcpy(&stats->counters, dcnt, sizeof(Counters), cudaMemcpyDeviceToHost));
+        return true;
+    }
+};
+
+// Scratch of one query call besides its caller rays, stream-ordered like them.
+struct QueryScratch {
+    DeviceBuffer recO, recD, recS0, recS1, order, queue, excl, counters, hit, rayO;
+    cudaStream_t st = nullptr;
+    ~QueryScratch() {
+        for (DeviceBuffer* b : {&recO, &recD, &recS0, &recS1, &order, &queue, &excl, &counters, &hit, &rayO}) b->release(st);
     }
 };
 
 static bool scene_query(Scene* s, bool transmit, size_t count, const float* origin4, const float* direction4, const uint32_t* excluded,
                         float* out4, bool deviceMemory, bool counting, void* stream, RenderStats* stats, std::string& err) {
-    if (!s) {
-        err = "null scene";
-        return false;
-    }
-    if (stats) *stats = RenderStats();
-    if (count == 0) return true;
-    if (!origin4 || !direction4 || !out4) {
-        err = "null origin, direction or output array";
-        return false;
-    }
-    OCLR_CUDA(cudaSetDevice(s->device));
-    if (deviceMemory && (!query_pointer_ok(s, origin4, 16, "origin", err) || !query_pointer_ok(s, direction4, 16, "direction", err) ||
-                         !query_pointer_ok(s, out4, 16, transmit ? "att" : "hit", err) ||
-                         (excluded && !query_pointer_ok(s, excluded, 4, "excluded", err))))
-        return false;
-    const SceneView& S = s->view;
-    if (S.n > 1024) {
-        err = "axesDivCount > 1024 is not supported by the packed walk";
-        return false;
-    }
     cudaStream_t st = (cudaStream_t)stream;
+    CallerRays rays = {s, count, origin4, direction4, excluded, out4, nullptr, deviceMemory, st};
+    if (!rays.check(transmit ? "att" : "hit", stats, err)) return false;
+    if (count == 0) return true;
+    const SceneView& S = s->view;
     QueryScratch q;
     q.st = st;
-    q.device = s->device;
     const uint32_t B = (uint32_t)std::min<size_t>(count, kQueryBatch);
     const size_t b = B;
     if (!q.recO.alloc(sizeof(float4) * b, err, st) || !q.recD.alloc(sizeof(float4) * b, err, st) || !q.recS0.alloc(sizeof(float4) * b, err, st) ||
         !q.recS1.alloc(sizeof(uint4) * b, err, st) || !q.order.alloc(sizeof(uint32_t) * b * kLengthClasses, err, st) ||
         !q.queue.alloc(sizeof(uint32_t) * b * (transmit ? 2 : 1), err, st) || !q.excl.alloc(sizeof(uint32_t) * b, err, st) ||
         !q.counters.alloc(sizeof(uint32_t) * (2 * kCounterStride + kRoundLogSize), err, st) ||
-        (counting && !q.stats.alloc(sizeof(Counters), err, st)) ||
         (transmit && (!q.hit.alloc(sizeof(float4) * b, err, st) || !q.rayO.alloc(sizeof(float4) * b, err, st))) ||
-        (!deviceMemory && (!q.inO.alloc(sizeof(float4) * b, err, st) || !q.inD.alloc(sizeof(float4) * b, err, st) ||
-                           (excluded && !q.inExcl.alloc(sizeof(uint32_t) * b, err, st)) || !q.out.alloc(sizeof(float4) * b, err, st))))
+        !rays.begin(b, counting, stats, err))
         return false;
-    Counters* dcnt = counting ? (Counters*)q.stats.p : nullptr;
-    if (dcnt) OCLR_CUDA(cudaMemsetAsync(dcnt, 0, sizeof(Counters), st));
-    if (stats) {
-        OCLR_CUDA(make_event(s->device, &q.ev0, true));
-        OCLR_CUDA(make_event(s->device, &q.ev1, true));
-        OCLR_CUDA(cudaEventRecord(q.ev0, st));
-    }
+    Counters* dcnt = rays.dcnt;
     unsigned traceGrid = 0;
     if (!trace_grid(S, s->smCount, counting, traceGrid, err)) return false;
     const unsigned setupGrid = (unsigned)std::min<uint64_t>((uint64_t)s->smCount * 8, (b + 255) / 256);
     const unsigned rayGrid = (unsigned)std::min<uint64_t>((uint64_t)s->smCount * 16, (b + 127) / 128);
     uint32_t* counters = (uint32_t*)q.counters.p;
     const uint32_t cstride = kCounterStride;
-    if (transmit && !(q.pinned = (uint32_t*)pinned_block())) {
+    if (transmit && !(rays.pinned = (uint32_t*)pinned_block())) {
         err = "out of pinned host memory";
         return false;
     }
@@ -2521,20 +2646,8 @@ static bool scene_query(Scene* s, bool transmit, size_t count, const float* orig
         QueryBatch qb;
         qb.count = n;
         qb.excl = (uint32_t*)q.excl.p;
-        if (deviceMemory) {
-            qb.origin = (const float4*)origin4 + off;
-            qb.direction = (const float4*)direction4 + off;
-            qb.excluded = excluded ? excluded + off : nullptr;
-        } else {
-            if (!host_to_device(q.inO.p, origin4 + 4 * off, sizeof(float4) * n, st, err) ||
-                !host_to_device(q.inD.p, direction4 + 4 * off, sizeof(float4) * n, st, err) ||
-                (excluded && !host_to_device(q.inExcl.p, excluded + off, sizeof(uint32_t) * n, st, err)))
-                return false;
-            qb.origin = (const float4*)q.inO.p;
-            qb.direction = (const float4*)q.inD.p;
-            qb.excluded = excluded ? (const uint32_t*)q.inExcl.p : nullptr;
-        }
-        float4* result = deviceMemory ? (float4*)out4 + off : (float4*)q.out.p;
+        if (!rays.rays(off, n, qb.origin, qb.direction, qb.excluded, err)) return false;
+        float4* result = rays.result(off);
         qb.hit = transmit ? (float4*)q.hit.p : result;
         qb.rayO = transmit ? (float4*)q.rayO.p : nullptr;
         qb.att = transmit ? result : nullptr;
@@ -2555,7 +2668,7 @@ static bool scene_query(Scene* s, bool transmit, size_t count, const float* orig
         OCLR_CUDA(cudaMemsetAsync(w.queueCount, 0, sizeof(uint32_t) * cstride, st));
         query_screen_kernel<<<rayGrid, 128, 0, st>>>(qb, w);
         ++launches;
-        // Rounds (trace -> transmit) are enqueued ahead in chunks without a host round trip, as frames do (launch_wavefront): every kernel
+        // Rounds (trace -> transmit) are enqueued ahead in chunks without a host round trip, as frames do (RoundDriver): every kernel
         // reads its ray count from device memory and returns at once when there is nothing to do.  One read per chunk: the count the last
         // transmit round queued.
         for (uint32_t r = 0;;) {
@@ -2576,26 +2689,18 @@ static bool scene_query(Scene* s, bool transmit, size_t count, const float* orig
                 ++launches;
             }
             if (!transmit) break;
-            OCLR_CUDA(cudaMemcpyAsync(q.pinned, counters + cstride * (r & 1u), sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
+            OCLR_CUDA(cudaMemcpyAsync(rays.pinned, counters + cstride * (r & 1u), sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
             OCLR_CUDA(cudaStreamSynchronize(st));
-            if (*q.pinned == 0) break;
+            if (*rays.pinned == 0) break;
             if (r > 100000) {
                 err = "transmittance did not converge";
                 return false;
             }
         }
         OCLR_CUDA(cudaGetLastError());
-        if (!deviceMemory && !device_to_host(out4 + 4 * off, q.out.p, sizeof(float4) * n, st, err)) return false;
+        if (!rays.download(off, n, err)) return false;
     }
-    if (stats) {
-        OCLR_CUDA(cudaEventRecord(q.ev1, st));
-        OCLR_CUDA(cudaEventSynchronize(q.ev1));
-        OCLR_CUDA(cudaEventElapsedTime(&stats->deviceMs, q.ev0, q.ev1));
-        stats->launches = launches;
-        stats->traceLaunches = rounds;
-        if (dcnt) OCLR_CUDA(cudaMemcpy(&stats->counters, dcnt, sizeof(Counters), cudaMemcpyDeviceToHost));
-    }
-    return true;
+    return rays.finish(stats, launches, rounds, err);
 }
 
 bool scene_intersect(Scene* s, size_t count, const float* origin4, const float* direction4, const uint32_t* excluded, float* hit4,
@@ -2609,136 +2714,70 @@ bool scene_transmittance(Scene* s, size_t count, const float* origin4, const flo
 }
 
 // ---- radiance along caller rays (rt_query.cuh radiance_start_kernel, then the frame's wf_logic_kernel) ---------------------------------
-// Scratch of one radiance call: the path state of one batch, stream-ordered like QueryScratch.
+// Scratch of one radiance call besides its caller rays: the path state of one batch and its per-ray sums, stream-ordered like them.
 struct RadianceScratch {
-    DeviceBuffer ctl, rng, colour, ring, carry, rayO, rayD, rayExcl, hit, queue, recO, recD, recS0, recS1, order, counters, stats;
-    DeviceBuffer accum, firstHit, inO, inD, inExcl, out, flags;
+    PathState ps;
+    DeviceBuffer accum, firstHit;
     cudaStream_t st = nullptr;
-    int device = 0;
-    cudaEvent_t ev0 = nullptr, ev1 = nullptr;
-    uint32_t* pinned = nullptr;   // the round log, read back once per chunk of rounds
     ~RadianceScratch() {
-        for (DeviceBuffer* b : {&ctl, &rng, &colour, &ring, &carry, &rayO, &rayD, &rayExcl, &hit, &queue, &recO, &recD, &recS0, &recS1, &order,
-                                &counters, &stats, &accum, &firstHit, &inO, &inD, &inExcl, &out, &flags})
-            b->release(st);
-        drop_event(device, ev0, true);
-        drop_event(device, ev1, true);
-        pinned_release(pinned);
+        ps.release(st);
+        accum.release(st);
+        firstHit.release(st);
     }
 };
 
 bool scene_radiance(Scene* s, const Camera* cam, size_t count, const float* origin4, const float* direction4, const uint32_t* excluded,
                     unsigned long long indexBase, uint32_t sampleCount, float* rgb4, uint8_t* flags, bool deviceMemory, bool counting,
                     void* stream, RenderStats* stats, std::string& err) {
-    if (!s) {
-        err = "null scene";
-        return false;
-    }
-    if (stats) *stats = RenderStats();
-    if (sampleCount < 1) {
+    // (a null scene is refused by CallerRays::check)
+    if (s && sampleCount < 1) {
         err = "sampleCount must be at least 1";
         return false;
     }
-    if (!cam && s->hasBump) {
+    if (s && !cam && s->hasBump) {
         err = "null camera: the scene has bump-mapped materials, whose normals read the camera's leftToRight / topToBottom / pixelSizeInv";
         return false;
     }
-    if (count == 0) return true;
-    if (!origin4 || !direction4 || !rgb4) {
-        err = "null origin, direction or output array";
-        return false;
-    }
-    OCLR_CUDA(cudaSetDevice(s->device));
-    if (deviceMemory && (!query_pointer_ok(s, origin4, 16, "origin", err) || !query_pointer_ok(s, direction4, 16, "direction", err) ||
-                         !query_pointer_ok(s, rgb4, 16, "rgb", err) || (excluded && !query_pointer_ok(s, excluded, 4, "excluded", err)) ||
-                         (flags && !query_pointer_ok(s, flags, 1, "flags", err))))
-        return false;
-    const SceneView& S = s->view;
-    if (S.n > 1024) {
-        err = "axesDivCount > 1024 is not supported by the packed walk";
-        return false;
-    }
     cudaStream_t st = (cudaStream_t)stream;
+    CallerRays rays = {s, count, origin4, direction4, excluded, rgb4, flags, deviceMemory, st};
+    if (!rays.check("rgb", stats, err)) return false;
+    if (count == 0) return true;
+    const SceneView& S = s->view;
     RadianceScratch q;
     q.st = st;
-    q.device = s->device;
     const uint32_t B = (uint32_t)std::min<size_t>(count, kRadianceBatch);
     const size_t b = B;
     const uint32_t W = kRadianceRowWidth, Q = (B + W - 1) / W * W;   // paths: the batch as a W-wide image (rt_query.cuh)
-    const size_t qn = Q;
-    if (!q.ctl.alloc(sizeof(uint32_t) * qn, err, st) || !q.rng.alloc(sizeof(uint64_t) * qn, err, st) || !q.colour.alloc(sizeof(float4) * qn, err, st) ||
-        !q.ring.alloc(sizeof(float4) * qn * (size_t)s->ringSlots * kRingParts, err, st) || !q.carry.alloc(sizeof(float4) * qn * kCarryParts, err, st) ||
-        // two ray slots per path (rt_wavefront.cuh: the next segment's closest hit is traced one round ahead)
-        !q.rayO.alloc(sizeof(float4) * 2 * qn, err, st) || !q.rayD.alloc(sizeof(float4) * 2 * qn, err, st) ||
-        !q.rayExcl.alloc(sizeof(uint32_t) * 2 * qn, err, st) || !q.hit.alloc(sizeof(float4) * 2 * qn, err, st) ||
-        !q.queue.alloc(sizeof(uint32_t) * 2 * qn, err, st) || !q.recO.alloc(sizeof(float4) * 2 * qn, err, st) ||
-        !q.recD.alloc(sizeof(float4) * 2 * qn, err, st) || !q.recS0.alloc(sizeof(float4) * 2 * qn, err, st) ||
-        !q.recS1.alloc(sizeof(uint4) * 2 * qn, err, st) || !q.order.alloc(sizeof(uint32_t) * 2 * qn * kLengthClasses, err, st) ||
-        !q.counters.alloc(sizeof(uint32_t) * (2 * kCounterStride + kRoundLogSize), err, st) ||
-        !q.accum.alloc(sizeof(float4) * qn, err, st) || !q.firstHit.alloc(sizeof(uint32_t) * qn, err, st) ||
-        (counting && !q.stats.alloc(sizeof(Counters), err, st)) ||
-        (!deviceMemory && (!q.inO.alloc(sizeof(float4) * b, err, st) || !q.inD.alloc(sizeof(float4) * b, err, st) ||
-                           (excluded && !q.inExcl.alloc(sizeof(uint32_t) * b, err, st)) || !q.out.alloc(sizeof(float4) * b, err, st) ||
-                           (flags && !q.flags.alloc(b, err, st)))))
+    if (!q.ps.reserve(Q, s->ringSlots, st, err) || !q.accum.alloc(sizeof(float4) * Q, err, st) ||
+        !q.firstHit.alloc(sizeof(uint32_t) * Q, err, st) || !rays.begin(b, counting, stats, err))
         return false;
-    if (!(q.pinned = (uint32_t*)pinned_block())) {
+    if (!(rays.pinned = (uint32_t*)pinned_block())) {
         err = "out of pinned host memory";
         return false;
     }
-    Counters* dcnt = counting ? (Counters*)q.stats.p : nullptr;
-    if (dcnt) OCLR_CUDA(cudaMemsetAsync(dcnt, 0, sizeof(Counters), st));
-    if (stats) {
-        OCLR_CUDA(make_event(s->device, &q.ev0, true));
-        OCLR_CUDA(make_event(s->device, &q.ev1, true));
-        OCLR_CUDA(cudaEventRecord(q.ev0, st));
-    }
-    unsigned traceGrid = 0;
-    if (!trace_grid(S, s->smCount, counting, traceGrid, err)) return false;
-    const unsigned setupGrid = (unsigned)std::min<uint64_t>((uint64_t)s->smCount * 8, (2 * qn + 255) / 256);
+    Counters* dcnt = rays.dcnt;
+    RoundDriver drv = {S, s->device, s->smCount, 0u, dcnt, rays.pinned, nullptr, "radiance query"};
+    if (!trace_grid(S, s->smCount, counting, drv.traceGrid, err)) return false;
     const int aheadMode = ahead_mode_for(Q);   // (no camera segments: modes 1 and 2 coincide)
-    uint32_t* counters = (uint32_t*)q.counters.p;
-    const uint32_t cstride = kCounterStride;
-    WfState w = {};
-    w.Q = Q;
-    w.ctl = (uint32_t*)q.ctl.p;
-    w.rng = (uint64_t*)q.rng.p;
-    w.colour = (float4*)q.colour.p;
-    w.ring = (float4*)q.ring.p;
-    w.ringSlots = (uint32_t)s->ringSlots;
-    w.carry = (float4*)q.carry.p;
-    w.rayO = (float4*)q.rayO.p;
-    w.rayD = (float4*)q.rayD.p;
-    w.rayExcl = (uint32_t*)q.rayExcl.p;
-    w.hit = (float4*)q.hit.p;
-    w.queue = (uint32_t*)q.queue.p;
-    w.roundLog = counters + 2 * cstride;
-    WalkRecords rec = {(float4*)q.recO.p, (float4*)q.recD.p, (float4*)q.recS0.p, (uint4*)q.recS1.p, (uint32_t*)q.order.p, nullptr, 2 * Q};
+    uint32_t lastRounds = 4;
+    drv.K = 1;
+    RoundDomain& d = drv.dom[0];
+    d.ps = &q.ps;
+    q.ps.bind(Q, s->ringSlots, d.w, d.rec);
+    d.st = st;
+    d.lastRounds = &lastRounds;
     FrameView F = {};   // the logic kernel's view of a batch: camera vectors, sample count, accumulator, flags (rt_query.cuh)
     if (cam) F.cam = *cam;
     F.cam.width = W;
     F.sampleCount = sampleCount;
     F.accum = (float4*)q.accum.p;
-    uint32_t launches = 0, rounds = 0, lastRounds = 4;
     for (size_t off = 0; off < count; off += b) {
         const uint32_t n = (uint32_t)std::min<size_t>(b, count - off);
         RayBatch R;
         R.count = n;
         R.indexBase = indexBase + off;
-        if (deviceMemory) {
-            R.origin = (const float4*)origin4 + off;
-            R.direction = (const float4*)direction4 + off;
-            R.excluded = excluded ? excluded + off : nullptr;
-        } else {
-            if (!host_to_device(q.inO.p, origin4 + 4 * off, sizeof(float4) * n, st, err) ||
-                !host_to_device(q.inD.p, direction4 + 4 * off, sizeof(float4) * n, st, err) ||
-                (excluded && !host_to_device(q.inExcl.p, excluded + off, sizeof(uint32_t) * n, st, err)))
-                return false;
-            R.origin = (const float4*)q.inO.p;
-            R.direction = (const float4*)q.inD.p;
-            R.excluded = excluded ? (const uint32_t*)q.inExcl.p : nullptr;
-        }
-        float4* result = deviceMemory ? (float4*)rgb4 + off : (float4*)q.out.p;
-        F.flagOut = flags ? (deviceMemory ? flags + off : (uint8_t*)q.flags.p) : nullptr;
+        if (!rays.rays(off, n, R.origin, R.direction, R.excluded, err)) return false;
+        F.flagOut = rays.flag_out(off);
         if (F.flagOut) OCLR_CUDA(cudaMemsetAsync(F.flagOut, 0, n, st));
         const uint32_t rows = (n + W - 1) / W;
         F.cam.height = rows;
@@ -2746,81 +2785,32 @@ bool scene_radiance(Scene* s, const Camera* cam, size_t count, const float* orig
         F.rowEnd = rows;
         const dim3 logicGrid(1, (rows + 7) / 8);
         const unsigned startGrid = (rows * W + 127) / 128, rayGrid = (n + 127) / 128;
-        // Rounds (entry or logic kernel -> setup -> trace) are enqueued ahead in chunks and ended by the round log, as frames do
-        // (launch_wavefront); round 0's entry is radiance_start_kernel instead of the logic kernel's kWfNew.
         for (uint32_t smp = 0; smp < sampleCount; ++smp) {
-            for (uint32_t r = 0;;) {
-                const uint32_t chunk = r == 0 ? std::max<uint32_t>(lastRounds, 2) : 2u;
-                for (uint32_t c = 0; c < chunk; ++c, ++r) {
-                    w.queueCount = counters + cstride * (r & 1u);
-                    w.queueCursor = w.queueCount + 1;
-                    w.roundIndex = r;
-                    rec.classCount = w.queueCount + 2;
-                    const uint32_t* prev = r ? counters + cstride * ((r - 1) & 1u) : nullptr;
-                    OCLR_CUDA(cudaMemsetAsync(w.queueCount, 0, sizeof(uint32_t) * cstride, st));
-                    if (r == 0) {
-                        if (dcnt)
-                            radiance_start_kernel<true><<<startGrid, 128, 0, st>>>(R, w, smp, sampleCount, dcnt);
-                        else
-                            radiance_start_kernel<false><<<startGrid, 128, 0, st>>>(R, w, smp, sampleCount, dcnt);
-                    } else {
-                        if (r == 1 && smp == 0)   // the trace of round 0 holds each ray's own closest hit
-                            radiance_first_hit_kernel<<<rayGrid, 128, 0, st>>>(n, w.hit, (uint32_t*)q.firstHit.p);
-                        if (dcnt)
-                            wf_logic_kernel<true><<<logicGrid, 128, 0, st>>>(S, F, w, smp, 0u, prev, dcnt, aheadMode);
-                        else
-                            wf_logic_kernel<false><<<logicGrid, 128, 0, st>>>(S, F, w, smp, 0u, prev, dcnt, aheadMode);
-                    }
-                    ++launches;
-                    const TailQueue tq = {nullptr, w.queueCount + 2 + kLengthClasses, w.queueCount + 6 + kLengthClasses, 0u,
-                                          nullptr, nullptr, nullptr, nullptr, nullptr};
-                    enqueue_trace(S, w, rec, tq, setupGrid, traceGrid, s->smCount, dcnt, st, launches);
-                    ++rounds;
+            // round 0 enters at radiance_start_kernel instead of the logic kernel's kWfNew
+            const RoundEntry entry = [&](int, uint32_t r, const WfState& w, const uint32_t* prev, cudaStream_t ks) {
+                if (r == 0) {
+                    if (dcnt)
+                        radiance_start_kernel<true><<<startGrid, 128, 0, ks>>>(R, w, smp, sampleCount, dcnt);
+                    else
+                        radiance_start_kernel<false><<<startGrid, 128, 0, ks>>>(R, w, smp, sampleCount, dcnt);
+                    return;
                 }
-                OCLR_CUDA(cudaMemcpyAsync(q.pinned, counters + 2 * cstride, sizeof(uint32_t) * std::min<uint32_t>(r, kRoundLogSize),
-                                          cudaMemcpyDeviceToHost, st));
-                if (r > kRoundLogSize)   // beyond the log: the live counter of the last enqueued round
-                    OCLR_CUDA(cudaMemcpyAsync(q.pinned + kRoundLogSize, counters + cstride * ((r - 1) & 1u), sizeof(uint32_t),
-                                              cudaMemcpyDeviceToHost, st));
-                OCLR_CUDA(cudaStreamSynchronize(st));
-                bool finished = false;
-                uint32_t needed = r;
-                if (r <= kRoundLogSize) {
-                    finished = q.pinned[r - 1] == 0;
-                    for (uint32_t k = 0; k < r; ++k)
-                        if (q.pinned[k] == 0) {   // the first round that queued no ray is the last one that had anything to do
-                            needed = k + 1;
-                            break;
-                        }
-                } else {
-                    finished = q.pinned[kRoundLogSize] == 0;
-                }
-                if (finished) {
-                    lastRounds = needed;
-                    break;
-                }
-                if (r > 100000) {
-                    err = "radiance query did not converge";
-                    return false;
-                }
-            }
+                if (r == 1 && smp == 0)   // the trace of round 0 holds each ray's own closest hit
+                    radiance_first_hit_kernel<<<rayGrid, 128, 0, ks>>>(n, w.hit, (uint32_t*)q.firstHit.p);
+                if (dcnt)
+                    wf_logic_kernel<true><<<logicGrid, 128, 0, ks>>>(S, F, w, smp, 0u, prev, dcnt, aheadMode);
+                else
+                    wf_logic_kernel<false><<<logicGrid, 128, 0, ks>>>(S, F, w, smp, 0u, prev, dcnt, aheadMode);
+            };
+            if (!drv.run(nullptr, entry, err)) return false;
         }
-        radiance_resolve_kernel<<<rayGrid, 128, 0, st>>>(R, (const float4*)q.accum.p, (const uint32_t*)q.firstHit.p, sampleCount, result);
-        ++launches;
+        radiance_resolve_kernel<<<rayGrid, 128, 0, st>>>(R, (const float4*)q.accum.p, (const uint32_t*)q.firstHit.p, sampleCount,
+                                                          rays.result(off));
+        ++drv.launches;
         OCLR_CUDA(cudaGetLastError());
-        if (!deviceMemory && (!device_to_host(rgb4 + 4 * off, q.out.p, sizeof(float4) * n, st, err) ||
-                              (flags && !device_to_host(flags + off, q.flags.p, n, st, err))))
-            return false;
+        if (!rays.download(off, n, err)) return false;
     }
-    if (stats) {
-        OCLR_CUDA(cudaEventRecord(q.ev1, st));
-        OCLR_CUDA(cudaEventSynchronize(q.ev1));
-        OCLR_CUDA(cudaEventElapsedTime(&stats->deviceMs, q.ev0, q.ev1));
-        stats->launches = launches;
-        stats->traceLaunches = rounds;
-        if (dcnt) OCLR_CUDA(cudaMemcpy(&stats->counters, dcnt, sizeof(Counters), cudaMemcpyDeviceToHost));
-    }
-    return true;
+    return rays.finish(stats, drv.launches, drv.rounds, err);
 }
 
 }  // namespace oclr
