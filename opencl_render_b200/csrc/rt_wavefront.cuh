@@ -36,18 +36,18 @@
 namespace oclr {
 
 enum WfStage { kWfDone = 0, kWfNew = 1, kWfWaitClosest = 2, kWfWaitShadow = 3 };
-enum : uint32_t { kCtlSpawned = 1u << 28, kCtlAhead = 1u << 29 };   // ctl = stage | begin << 4 | end << 8 | light << 12 | flags
+enum : uint32_t { kCtlSpawned = 1u << 28, kCtlAhead = 1u << 29 };   // ctl = stage | begin << 4 | end << 8 | flags
 enum { kCarryParts = 7, kRingParts = 3 };
 
 // Path state (device pointers; Q = paths in the launch domain).  All float4 planes are [part][Q].
 struct WfState {
     uint32_t Q;
-    uint32_t* ctl;       // stage | begin << 4 | end << 8 | light << 12
+    uint32_t* ctl;       // stage | begin << 4 | end << 8 | flags
     uint64_t* rng;
     float4* colour;
     float4* ring;        // [slot * 3 + part][Q], slot < ringSlots
     uint32_t ringSlots;  // kRingSize, or 2 for a scene without mirror / glass materials (runtime.cu, Scene::ringSlots)
-    float4* carry;       // [part][Q], part < 7
+    float4* carry;       // [part][Q], part < 7; part 6's w = the light a kWfWaitShadow path waits on (any uint32_t lightCount)
     // two ray slots per path, slot-major [slot * Q + path]: slot 0 = the query the path is suspended on, slot 1 = the closest-hit
     // query of the NEXT ring segment traced one round ahead.  Queue entries are these flat indices (the trace stage knows no paths).
     float4* rayO;        // (o.xyz, minD)
@@ -152,7 +152,7 @@ __global__ void __launch_bounds__(128, OCLR_LOGIC_MIN_CTAS) wf_logic_kernel(Scen
         Counters cnt = {};
         const Camera& cam = F.cam;
         int begin = (int)((ctl >> 4) & 15u), end = (int)((ctl >> 8) & 15u);
-        uint32_t j = (ctl >> 12) & 0xFFFFu;
+        uint32_t j = 0;   // the light loop's index: set by GO_SHADE, or from the carry on a shadow resume
         bool spawned = (ctl & kCtlSpawned) != 0u;   // the current segment's spawn (:656-722) was done ahead of its shadow result
         bool ahead = (ctl & kCtlAhead) != 0u;       // slot 1 holds (or is about to receive) the next segment's closest hit
         uint64_t rng;
@@ -212,6 +212,7 @@ __global__ void __launch_bounds__(128, OCLR_LOGIC_MIN_CTAS) wf_logic_kernel(Scen
                 hitT = k0.w;
                 tex = mk3(k1.x, k1.y, k1.z);
                 const uint32_t shaded = __float_as_uint(k1.w);
+                j = __float_as_uint(k6.w);
                 refl = mk3(k2.x, k2.y, k2.z);
                 transp = mk3(k2.w, k3.x, k3.y);
                 lum = mk3(k3.z, k3.w, k4.x);
@@ -321,7 +322,7 @@ __global__ void __launch_bounds__(128, OCLR_LOGIC_MIN_CTAS) wf_logic_kernel(Scen
                         cp[3 * (size_t)w.Q] = make_float4(transp.y, transp.z, lum.x, lum.y);
                         cp[4 * (size_t)w.Q] = make_float4(lum.z, att.x, att.y, att.z);
                         cp[5 * (size_t)w.Q] = make_float4(face[0].x, face[0].y, face[0].z, 0.f);
-                        cp[6 * (size_t)w.Q] = make_float4(face[1].x, face[1].y, face[1].z, 0.f);
+                        cp[6 * (size_t)w.Q] = make_float4(face[1].x, face[1].y, face[1].z, __uint_as_float(j));
                         stage = kWfWaitShadow;
                         want = true;
                         // last light: spawn now and trace the next segment one round ahead (aheadMode 2: every segment; 1: all but
@@ -466,8 +467,7 @@ __global__ void __launch_bounds__(128, OCLR_LOGIC_MIN_CTAS) wf_logic_kernel(Scen
             w.rng[q] = rng;
             w.colour[q] = make_float4(colour.x, colour.y, colour.z, 0.f);
         }
-        w.ctl[q] = (uint32_t)stage | ((uint32_t)begin << 4) | ((uint32_t)end << 8) | (j << 12) | (spawned ? kCtlSpawned : 0u) |
-                   (ahead ? kCtlAhead : 0u);
+        w.ctl[q] = (uint32_t)stage | ((uint32_t)begin << 4) | ((uint32_t)end << 8) | (spawned ? kCtlSpawned : 0u) | (ahead ? kCtlAhead : 0u);
         if (COUNT) flush_counters(cnt, gcnt);
     }
     enqueue(w, q, want, wantAhead, finished, F.doneCount);
