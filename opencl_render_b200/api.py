@@ -265,7 +265,7 @@ class DeviceScene:
         self._lib = _lib.load()
         scene.normalise()
         if scene.box_min is None:
-            scene.axes_div = axes_div or AXES_DIVISION
+            scene.axes_div = AXES_DIVISION if axes_div is None else axes_div
         d = scene.desc(allow_missing_grid=True)
         self.handle = self._lib.oclr_scene_create(device, C.byref(d))
         if not self.handle:
