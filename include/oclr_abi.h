@@ -270,6 +270,35 @@ oclr_frame* oclr_frame_create_device_lists(oclr_scene* scene, const oclr_camera*
 size_t oclr_frame_camera_list_size(const oclr_frame* frame);
 int oclr_frame_read_camera_lists(oclr_frame* frame, cl_uint* start, cl_uint* end, cl_uint* list);
 
+/* ---- edits of a resident scene and of a frame's camera ----
+ * oclr_scene_update replaces the parts named in `parts` with the arrays of `desc` (same layout as oclr_scene_create; the fields of
+ * other parts are ignored).  Afterwards the scene is byte for byte what oclr_scene_create would make from the new parts plus the
+ * arrays it was created or last updated with: packed arrays, oclr_scene_device_bytes, path ring depth and every render and query result.
+ *   OCLR_SCENE_LIGHTS     lightCount (0 included) and the six light arrays.
+ *   OCLR_SCENE_MATERIALS  materialCount, materialImageSize, materialImageStart, texturesSize and textures, all together.  Without a
+ *                         geometry edit in the same call the resident triangles' material ids are checked against the new count.
+ *   OCLR_SCENE_GEOMETRY   vertices, triangle indices, material ids, UVs and normals at any counts; the grid from desc when given,
+ *                         else built on the device at desc->axesDivCount cells per axis.
+ * memory: OCLR_QUERY_HOST_MEMORY, or OCLR_QUERY_DEVICE_MEMORY -- the geometry arrays (the grid arrays included) are device memory of
+ * the scene's device, read in place (vertex, indices, normals, sceneBoxMin 16-byte aligned, UVs 8, the rest 4).  Lights and
+ * materials are always host arrays.
+ * The call waits for all work already enqueued on the scene's device, builds the new parts into new buffers (a geometry edit can
+ * briefly need twice the geometry's device bytes) and swaps them in only on success: a failed update returns 0 with oclr_last_error()
+ * set and leaves the scene exactly as it was.  It returns with the edit in place; frames and queries see it from their next call.
+ * Planes and float accumulators are not cleared: a progressive job continued across an edit mixes the two scenes.  After a geometry
+ * edit a frame with device-built lists rebuilds them at its next use; a frame with caller lists refuses to render until
+ * oclr_frame_set_camera_lists or oclr_frame_set_camera gives it lists for the new geometry.  Returns 1 on success. */
+enum { OCLR_SCENE_LIGHTS = 1, OCLR_SCENE_MATERIALS = 2, OCLR_SCENE_GEOMETRY = 4 };
+int oclr_scene_update(oclr_scene* scene, const oclr_scene_desc* desc, unsigned parts, int memory);
+/* New camera of the same width x height; lists built on the device from the resident scene.  The frame keeps its planes, path state,
+ * accumulation mode and progress counters; a different image size is refused (make a new frame).  The call waits for all work
+ * enqueued on the frame's device.  A call that fails after the image-size check leaves the frame with the new camera and no lists: it
+ * refuses to render until a camera is set successfully.  Returns 1 on success. */
+int oclr_frame_set_camera(oclr_frame* frame, const oclr_camera* camera);
+/* Same, with the caller's CameraTriangleList::New output (range-checked on the device as in oclr_frame_create). */
+int oclr_frame_set_camera_lists(oclr_frame* frame, const oclr_camera* camera, const cl_uint* start, const cl_uint* end,
+                                const cl_uint* list, size_t listSize);
+
 /* Trace rows [rowBegin,rowEnd) with sampleCount samples per pixel on `cudaStream` (a cudaStream_t, NULL = default
  * stream).  `stats` may be NULL (then the call does not synchronise).  `countEvents` != 0 runs the counting build.
  * Returns 1 on success. */

@@ -82,6 +82,8 @@ EXPORTS = [
     "oclr_set_option", "oclr_frame_push_rows",
     # batched ray queries on a resident scene
     "oclr_scene_intersect", "oclr_scene_transmittance", "oclr_scene_radiance",
+    # edits of a resident scene and of a frame's camera
+    "oclr_scene_update", "oclr_frame_set_camera", "oclr_frame_set_camera_lists",
 ]
 
 _lib = None
@@ -191,6 +193,12 @@ def load() -> C.CDLL:
     lib.oclr_scene_radiance.restype = C.c_int
     lib.oclr_scene_radiance.argtypes = [C.c_void_p, C.POINTER(Camera), C.c_size_t, C.c_void_p, C.c_void_p, C.c_void_p, C.c_ulonglong, C.c_uint32,
                                         C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.POINTER(RenderStats)]
+    lib.oclr_scene_update.restype = C.c_int
+    lib.oclr_scene_update.argtypes = [C.c_void_p, C.POINTER(SceneDesc), C.c_uint, C.c_int]
+    lib.oclr_frame_set_camera.restype = C.c_int
+    lib.oclr_frame_set_camera.argtypes = [C.c_void_p, C.POINTER(Camera)]
+    lib.oclr_frame_set_camera_lists.restype = C.c_int
+    lib.oclr_frame_set_camera_lists.argtypes = [C.c_void_p, C.POINTER(Camera), C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t]
     lib.oclr_set_option.restype = C.c_int
     lib.oclr_set_option.argtypes = [C.c_char_p, C.c_int]
     lib.InitOpenCL.restype = None

@@ -10,6 +10,7 @@ no Python implementation behind any of them.
 from __future__ import annotations
 
 import ctypes as C
+import dataclasses
 from dataclasses import dataclass, field
 
 import numpy as np
@@ -25,6 +26,7 @@ KERNEL_SIMPLE, KERNEL_PIPE, KERNEL_DEFAULT = 0, 2, -1
 ACCUMULATE_REFERENCE_16BIT, ACCUMULATE_FLOAT = 0, 1
 NO_TRIANGLE = 0xFFFFFFFF
 QUERY_HOST_MEMORY, QUERY_DEVICE_MEMORY = 0, 1
+SCENE_LIGHTS, SCENE_MATERIALS, SCENE_GEOMETRY = 1, 2, 4   # parts of oclr_scene_update
 QUERY_BATCH = 1 << 21        # rays per internal batch of a query (runtime.h kQueryBatch)
 RADIANCE_BATCH = 1 << 20     # rays per internal batch of a radiance query (runtime.h kRadianceBatch)
 
@@ -277,6 +279,66 @@ class DeviceScene:
     def device_bytes(self) -> int:
         return int(self._lib.oclr_scene_device_bytes(self.handle))
 
+    def update(self, scene: HostScene, lights: bool = False, materials: bool = False, geometry: bool = False):
+        """Replaces the parts named with those of `scene` (numpy arrays) in place (oclr_scene_update): afterwards the scene is byte for
+        byte what DeviceScene would make from the new parts plus the ones it holds.  geometry=True takes scene's grid when it has one,
+        else builds it on the device at scene.axes_div.  A failed update raises OclrError and leaves the scene as it was."""
+        parts = (SCENE_LIGHTS if lights else 0) | (SCENE_MATERIALS if materials else 0) | (SCENE_GEOMETRY if geometry else 0)
+        if not parts:
+            raise ValueError("update: name at least one part (lights, materials, geometry)")
+        if not isinstance(scene, HostScene):
+            raise ValueError("update: scene must be a HostScene (update_geometry takes bare arrays)")
+        scene.normalise()
+        d = scene.desc(allow_missing_grid=True)
+        if not self._lib.oclr_scene_update(self.handle, C.byref(d), parts, QUERY_HOST_MEMORY):
+            raise OclrError(_lib.last_error())
+        keep = {}
+        if lights:
+            keep.update({k: getattr(scene, k) for k in ("light_type", "light_pos", "light_dir", "light_colour", "light_radius", "light_half")})
+        if materials:
+            keep.update(mat_size=scene.mat_size, mat_start=scene.mat_start, textures=scene.textures)
+        if geometry:
+            keep.update({k: getattr(scene, k) for k in ("vertex", "tri_idx", "tri_mat", "tri_uv", "tri_normal", "axes_div", "box_min",
+                                                         "grid_start", "grid_list")})
+        self.host = dataclasses.replace(self.host, **keep)
+
+    def update_geometry(self, vertex, tri_idx, tri_mat, tri_uv, tri_normal, grid=None, axes_div: int | None = None):
+        """Replaces the geometry in place (oclr_scene_update with OCLR_SCENE_GEOMETRY).  Arrays in HostScene's shapes: vertex [V,4]
+        float32, tri_idx [N,4] int32, tri_mat [N] int32, tri_uv [N,3,2] float32, tri_normal [N,3,4] float32 -- all numpy, or all CUDA
+        torch tensors on the scene's device (read in place, e.g. a simulation's output).  grid = (box_min [n+1,4] float32,
+        grid_start [n^3+1] uint32, grid_list [K] uint32) in the same kind of memory, or None: built on the device at `axes_div` cells
+        per axis (default: the current one).  `host` then holds the arrays given (torch tensors stay tensors)."""
+        arrays = {"vertex": vertex, "tri_idx": tri_idx, "tri_mat": tri_mat, "tri_uv": tri_uv, "tri_normal": tri_normal}
+        if grid is not None:
+            if len(grid) != 3:
+                raise ValueError("grid must be (box_min, grid_start, grid_list)")
+            if axes_div is not None:
+                raise ValueError("axes_div is taken from the grid given (box_min has axes_div + 1 rows)")
+            arrays.update(box_min=grid[0], grid_start=grid[1], grid_list=grid[2])
+        torch = _torch_if_any(arrays.values())
+        if torch is None:
+            a = _geometry_arrays_numpy(arrays, self.host.axes_div if axes_div is None else axes_div)
+            memory, ptr = QUERY_HOST_MEMORY, _ptr
+        else:
+            a = _geometry_arrays_torch(torch, torch.device("cuda", self.device), arrays,
+                                       self.host.axes_div if axes_div is None else axes_div)
+            memory, ptr = QUERY_DEVICE_MEMORY, lambda t: C.c_void_p(t.data_ptr()) if t is not None and t.numel() else None
+        d = _lib.SceneDesc()
+        d.vertexCount, d.vertex = a["vertex"].shape[0], ptr(a["vertex"])
+        d.triangleCount = a["tri_idx"].shape[0]
+        d.triangleVertexIndex, d.triangleMaterialId = ptr(a["tri_idx"]), ptr(a["tri_mat"])
+        d.triangleUv, d.triangleNormal = ptr(a["tri_uv"]), ptr(a["tri_normal"])
+        d.axesDivCount = a["axes_div"]
+        if grid is not None:
+            d.sceneBoxMin, d.scenePixelTriangleListStart, d.scenePixelTriangleList = ptr(a["box_min"]), ptr(a["grid_start"]), ptr(a["grid_list"])
+        if torch is not None:
+            torch.cuda.current_stream(torch.device("cuda", self.device)).synchronize()   # the arrays are complete before the library reads them
+        if not self._lib.oclr_scene_update(self.handle, C.byref(d), SCENE_GEOMETRY, memory):
+            raise OclrError(_lib.last_error())
+        self.host = dataclasses.replace(self.host, vertex=a["vertex"], tri_idx=a["tri_idx"], tri_mat=a["tri_mat"], tri_uv=a["tri_uv"],
+                                        tri_normal=a["tri_normal"], axes_div=a["axes_div"], box_min=a.get("box_min"),
+                                        grid_start=a.get("grid_start"), grid_list=a.get("grid_list"))
+
     def debug_read(self, which: int) -> np.ndarray:
         """Packed device array as bytes (0 triGeo, 1 triShade, 2 bricks, 3 cellRange, 4 planes, 5 cellList)."""
         n = int(self._lib.oclr_scene_debug_read(self.handle, which, None, 0))
@@ -399,6 +461,65 @@ class DeviceScene:
         self.close()
 
 
+_GEOMETRY_SHAPES = {"vertex": ("float32", (4,)), "tri_idx": ("int32", (4,)), "tri_mat": ("int32", ()), "tri_uv": ("float32", (3, 2)),
+                    "tri_normal": ("float32", (3, 4)), "box_min": ("float32", (4,)), "grid_start": ("uint32", ()), "grid_list": ("uint32", ())}
+
+
+def _torch_if_any(arrays):
+    """The torch module when any of `arrays` is a torch tensor (torch is imported only then), else None; numpy and torch do not mix."""
+    kinds = {type(a).__module__.startswith("torch") for a in arrays if a is not None}
+    if kinds == {True, False}:
+        raise ValueError("the geometry arrays mix numpy arrays and torch tensors: give all of them in one kind of memory")
+    if kinds == {True}:
+        import torch
+        return torch
+    return None
+
+
+def _check_geometry_shapes(a: dict, shape_of, axes_div: int | None):
+    """Shapes of the geometry arrays (HostScene's) and their agreement: one triangle count, a grid of axes_div cells per axis."""
+    for name, (_, tail) in _GEOMETRY_SHAPES.items():
+        if name in a and (len(shape_of(a[name])) != 1 + len(tail) or tuple(shape_of(a[name])[1:]) != tail):
+            raise ValueError(f"{name} must be [K{''.join(f',{t}' for t in tail)}], got {tuple(shape_of(a[name]))}")
+    n = shape_of(a["tri_idx"])[0]
+    for name in ("tri_mat", "tri_uv", "tri_normal"):
+        if shape_of(a[name])[0] != n:
+            raise ValueError(f"tri_idx has {n} triangles, {name} {shape_of(a[name])[0]}")
+    if "box_min" in a:
+        axes_div = shape_of(a["box_min"])[0] - 1
+        if shape_of(a["grid_start"])[0] != axes_div ** 3 + 1:
+            raise ValueError(f"box_min has {axes_div + 1} rows (axes_div {axes_div}): grid_start must have {axes_div ** 3 + 1} entries, "
+                             f"got {shape_of(a['grid_start'])[0]}")
+    if isinstance(axes_div, bool) or not isinstance(axes_div, (int, np.integer)) or axes_div < 1 or axes_div & (axes_div - 1) or axes_div > 1024:
+        raise ValueError(f"axes_div must be a power of two <= 1024, got {axes_div!r}")
+    a["axes_div"] = int(axes_div)
+    return a
+
+
+def _geometry_arrays_numpy(arrays: dict, axes_div):
+    a = {k: np.asarray(v) for k, v in arrays.items()}
+    _check_geometry_shapes(a, lambda x: x.shape, axes_div)
+    for name, (dt, _) in _GEOMETRY_SHAPES.items():
+        if name in a:
+            a[name] = np.ascontiguousarray(a[name], dtype=dt)
+    return a
+
+
+def _geometry_arrays_torch(torch, dev, arrays: dict, axes_div):
+    for name, v in arrays.items():
+        if not isinstance(v, torch.Tensor) or v.device != dev:
+            raise ValueError(f"{name} is on {getattr(v, 'device', 'the host')}, the scene is on {dev}: torch geometry is read in place")
+    a = dict(arrays)
+    _check_geometry_shapes(a, lambda x: tuple(x.shape), axes_div)
+    for name, (dt, _) in _GEOMETRY_SHAPES.items():
+        if name in a:
+            want = getattr(torch, dt)
+            if a[name].dtype != want:
+                raise ValueError(f"{name} must be {dt}, got {a[name].dtype}")
+            a[name] = a[name].contiguous()
+    return a
+
+
 def _torch_if_tensor(a):
     """The torch module when `a` is a torch tensor (torch is imported only then), else None."""
     mod = type(a).__module__
@@ -510,6 +631,29 @@ class DeviceFrame:
             lst = _c(lists.list, np.uint32)
             self.handle = self._lib.oclr_frame_create(scene.handle, C.byref(cam), _ptr(start), _ptr(end), _ptr(lst), int(lst.size))
         if not self.handle:
+            raise OclrError(_lib.last_error())
+
+    def set_camera(self, camera: CameraSetup, lists: CameraLists | None = None):
+        """Moves the frame's camera (same width and height): `lists` = CameraTriangleList::New output for the new camera and the
+        scene's current geometry, or None: built on the device.  Planes, path state, accumulation mode and progress stay.  A call that
+        fails in the library (OclrError) leaves the frame with the new camera and no lists: `camera` follows, and the frame refuses to
+        render until a camera is set successfully."""
+        if not isinstance(camera, CameraSetup):
+            raise ValueError("camera must be a CameraSetup (set_camera)")
+        if (camera.width, camera.height) != (self.camera.width, self.camera.height):
+            raise ValueError(f"the camera is {camera.width}x{camera.height}, the frame {self.camera.width}x{self.camera.height}: "
+                             "a frame keeps its image size (make a new DeviceFrame)")
+        cam = camera.c()
+        if lists is None:
+            ok = self._lib.oclr_frame_set_camera(self.handle, C.byref(cam))
+        else:
+            P = camera.width * camera.height
+            start, end, lst = _c(lists.start, np.uint32), _c(lists.end, np.uint32), _c(lists.list, np.uint32)
+            if start.shape != (P,) or end.shape != (P,) or lst.ndim != 1:
+                raise ValueError(f"lists: start and end must be [{P}] (width * height), list 1-D; got {start.shape}, {end.shape}, {lst.shape}")
+            ok = self._lib.oclr_frame_set_camera_lists(self.handle, C.byref(cam), _ptr(start), _ptr(end), _ptr(lst), int(lst.size))
+        self.camera = camera
+        if not ok:
             raise OclrError(_lib.last_error())
 
     @property

@@ -225,6 +225,28 @@ size_t oclr_scene_debug_read(oclr_scene* scene, int which, void* dst, size_t cap
     return scene ? scene_debug_read(scene->impl, which, dst, capacity) : 0;
 }
 size_t oclr_scene_device_bytes(const oclr_scene* scene) { return scene ? scene_device_bytes(scene->impl) : 0; }
+static_assert(OCLR_SCENE_LIGHTS == kSceneLights && OCLR_SCENE_MATERIALS == kSceneMaterials && OCLR_SCENE_GEOMETRY == kSceneGeometry, "part bits");
+int oclr_scene_update(oclr_scene* scene, const oclr_scene_desc* desc, unsigned parts, int memory) {
+    if (parts == 0 || (parts & ~(unsigned)(OCLR_SCENE_LIGHTS | OCLR_SCENE_MATERIALS | OCLR_SCENE_GEOMETRY))) {
+        fail("oclr_scene_update: parts must be a non-empty combination of OCLR_SCENE_LIGHTS, OCLR_SCENE_MATERIALS and OCLR_SCENE_GEOMETRY, "
+             "got " + std::to_string(parts));
+        return 0;
+    }
+    if (memory != OCLR_QUERY_HOST_MEMORY && memory != OCLR_QUERY_DEVICE_MEMORY) {
+        fail("oclr_scene_update: unknown memory kind " + std::to_string(memory));
+        return 0;
+    }
+    if (!scene || !desc) {
+        fail("oclr_scene_update: null scene or description");
+        return 0;
+    }
+    std::string err;
+    if (!scene_update(scene->impl, to_host(desc), parts, memory == OCLR_QUERY_DEVICE_MEMORY, err)) {
+        fail("oclr_scene_update: " + err);
+        return 0;
+    }
+    return 1;
+}
 
 void oclr_set_camera(oclr_camera* out, const cl_float position[3], const cl_float object[3], const cl_float up[3], cl_float fov,
                      cl_uint width, cl_uint height) {
@@ -273,6 +295,27 @@ oclr_frame* oclr_frame_create_device_lists(oclr_scene* scene, const oclr_camera*
     h->impl = f;
     h->scene = scene;
     return h;
+}
+int oclr_frame_set_camera(oclr_frame* frame, const oclr_camera* camera) {
+    std::string err;
+    if (!frame || !camera || !frame_set_camera(frame->impl, to_camera(camera), nullptr, nullptr, nullptr, 0, err)) {
+        fail("oclr_frame_set_camera: " + (err.empty() ? std::string("null frame or camera") : err));
+        return 0;
+    }
+    return 1;
+}
+int oclr_frame_set_camera_lists(oclr_frame* frame, const oclr_camera* camera, const cl_uint* start, const cl_uint* end, const cl_uint* list,
+                                size_t listSize) {
+    std::string err;
+    if (!frame || !camera || !start || !end) {
+        fail("oclr_frame_set_camera_lists: null frame, camera or camera triangle lists");
+        return 0;
+    }
+    if (!frame_set_camera(frame->impl, to_camera(camera), start, end, list, listSize, err)) {
+        fail("oclr_frame_set_camera_lists: " + err);
+        return 0;
+    }
+    return 1;
 }
 size_t oclr_frame_camera_list_size(const oclr_frame* frame) { return frame ? frame_camera_list_size(frame->impl) : 0; }
 int oclr_frame_read_camera_lists(oclr_frame* frame, cl_uint* start, cl_uint* end, cl_uint* list) {

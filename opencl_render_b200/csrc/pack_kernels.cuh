@@ -143,6 +143,24 @@ __global__ void __launch_bounds__(256) face_mask_kernel(const uint32_t* __restri
     faceMask[t] = m;
 }
 
+// Vertex indices of every triangle, checked before the device grid builder gathers vertices by them (the packer checks them too,
+// but runs concurrently with the builder's first kernels).
+__global__ void __launch_bounds__(256) check_indices_kernel(uint32_t triangleCount, uint32_t vertexCount, const int4* __restrict__ triIdx,
+                                                            uint32_t* __restrict__ error) {
+    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= triangleCount) return;
+    const int4 vi = __ldg(triIdx + i);
+    if ((uint32_t)vi.x >= vertexCount || (uint32_t)vi.y >= vertexCount || (uint32_t)vi.z >= vertexCount) atomicOr(error, (uint32_t)kPackBadVertexIndex);
+}
+
+// Material ids of the resident triangles (the .w word of triShade record 0, pack_triangles_kernel) against a new material count:
+// the same rule as the packer's.
+__global__ void __launch_bounds__(256) check_materials_kernel(uint32_t triangleCount, uint32_t materialCount, const float4* __restrict__ shade,
+                                                              uint32_t* __restrict__ error) {
+    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i < triangleCount && __float_as_int(__ldg(shade + 8 * (size_t)i).w) >= (int32_t)materialCount) atomicOr(error, (uint32_t)kPackBadMaterial);
+}
+
 __global__ void __launch_bounds__(256) check_list_kernel(const uint32_t* __restrict__ list, uint32_t total, uint32_t triangleCount,
                                                          uint32_t* __restrict__ error) {
     const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;

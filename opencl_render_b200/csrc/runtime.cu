@@ -660,6 +660,10 @@ struct Scene {
     // instead of kRingSize (576 B)
     int ringSlots = kRingSize;
     bool hasBump = false;   // some material has a BUMP channel: its normals read the camera vectors (radiance queries need a camera)
+    uint64_t geometryGen = 0;   // geometry edits so far (scene_update): camera lists built for an older generation are stale
+    std::array<DeviceBuffer*, 11> buffers() {
+        return {&triGeo, &triShade, &bricks, &cellRange, &cellList, &faceMask, &planes, &matSize, &matStart, &textures, &lights};
+    }
 };
 
 // per-round counters of a launch domain: {ray count, cursor, class counts[4], hand-off count, 0, 0, 0, hand-off cursor}, two sets
@@ -672,15 +676,17 @@ struct PathState {
     DeviceBuffer recO, recD, recS0, recS1, recOrder;   // walk records in queue order + class order (rt_trace.cuh)
     DeviceBuffer counters;                             // kCounterStride counters x 2, alternating between rounds; then the round log
     uint32_t capacity = 0;
+    int ringSlots = 0;   // ring depth the buffers were sized for
     std::array<DeviceBuffer*, 16> buffers() {
         return {&ctl, &rng, &colour, &ring, &carry, &rayO, &rayD, &rayExcl, &hit, &queue, &recO, &recD, &recS0, &recS1, &recOrder, &counters};
     }
-    bool reserve(uint32_t Q, int ringSlots, cudaStream_t st, std::string& err) {
-        if (Q <= capacity) return true;
+    bool reserve(uint32_t Q, int slots, cudaStream_t st, std::string& err) {
+        Q = path_state_regrow(capacity, ringSlots, Q, slots);
+        if (!Q) return true;
         release(st);
         const size_t q = Q;
         if (!ctl.alloc(sizeof(uint32_t) * q, err, st) || !rng.alloc(sizeof(uint64_t) * q, err, st) || !colour.alloc(sizeof(float4) * q, err, st) ||
-            !ring.alloc(sizeof(float4) * q * (size_t)ringSlots * kRingParts, err, st) || !carry.alloc(sizeof(float4) * q * kCarryParts, err, st) ||
+            !ring.alloc(sizeof(float4) * q * (size_t)slots * kRingParts, err, st) || !carry.alloc(sizeof(float4) * q * kCarryParts, err, st) ||
             // two ray slots per path (rt_wavefront.cuh: the next segment's closest hit is traced one round ahead)
             !rayO.alloc(sizeof(float4) * 2 * q, err, st) || !rayD.alloc(sizeof(float4) * 2 * q, err, st) ||
             !rayExcl.alloc(sizeof(uint32_t) * 2 * q, err, st) || !hit.alloc(sizeof(float4) * 2 * q, err, st) ||
@@ -690,11 +696,13 @@ struct PathState {
             !counters.alloc(sizeof(uint32_t) * (2 * kCounterStride + kRoundLogSize), err, st))
             return false;
         capacity = Q;
+        ringSlots = slots;
         return true;
     }
     void release(cudaStream_t st) {
         for (DeviceBuffer* b : buffers()) b->release(st);
         capacity = 0;
+        ringSlots = 0;
     }
     size_t bytes() {
         size_t n = 0;
@@ -725,12 +733,15 @@ struct WfSlice {
     std::array<DeviceBuffer*, 6> tail_buffers() { return {&tailEntries, &tailO, &tailD, &tailS0, &tailS1, &tailOrder}; }
 };
 
+static constexpr uint64_t kNoLists = ~0ull;
 struct Frame {
     Scene* scene = nullptr;
     int device = 0;
     Camera cam = {};
     DeviceBuffer camStart, camEnd, camList, planesRGB, ids, flags, counters;
     DeviceBuffer camCheck;           // range-check flag of caller-supplied camera lists (check_camera_lists_kernel); unset for device-built lists
+    bool deviceLists = false;        // the lists are built on the device (frame_build_camera_lists), again after a geometry edit
+    uint64_t listsGen = 0;           // Scene::geometryGen the lists were made for; kNoLists: the frame has none (a failed frame_set_camera)
     WfSlice slices[kMaxSlices];      // wavefront path state (allocated on first use, sized for the largest slice seen)
     uint32_t* hostCount = nullptr;   // pinned, one per slice
     cudaEvent_t ev0 = nullptr, ev1 = nullptr, evFork = nullptr;
@@ -1044,6 +1055,144 @@ static bool shard_verify(int rank, const ShardArray* arrays, int count, int grou
     return true;
 }
 
+// ---- the stages of a scene build, shared by scene_create (scene_upload) and scene_update ------------------------------------------------
+// Ring depth of a scene's paths and whether its normals read the camera, from the material tables (host arrays).
+static void material_rules(const HostScene& h, int& ringSlots, bool& hasBump) {
+    ringSlots = 2;
+    for (uint32_t m = 0; m < h.materialCount && ringSlots == 2; ++m)
+        for (int ch : {(int)kChReflection, (int)kChTransparency}) {
+            // a channel that is present but black everywhere (the plugin's 1x1 fallback for "no reflection") spawns nothing either: the
+            // segment multiplier is 0 < 3/256 (:684, :703).  Large maps are not scanned: taken as "may be non-zero"
+            const uint2 size = h.matSize[kMaterialChannels * m + ch];
+            const size_t texels = (size_t)size.x * size.y;
+            if (texels == 0) continue;
+            bool black = texels <= ((size_t)1 << 20);
+            const uchar4* t = h.textures + h.matStart[kMaterialChannels * m + ch];
+            for (size_t i = 0; black && i < texels; ++i) black = (t[i].x | t[i].y | t[i].z) == 0;
+            if (!black) ringSlots = kRingSize;
+        }
+    if (const char* v = getenv("OCLR_RING_SLOTS")) ringSlots = std::max(ringSlots, std::min(atoi(v), (int)kRingSize));   // (test knob: more, never fewer)
+    hasBump = false;
+    for (uint32_t m = 0; m < h.materialCount; ++m) hasBump |= h.matSize[kMaterialChannels * m + kChBump].x > 0u;
+}
+
+static std::string pack_error_message(uint32_t flag) {
+    return std::string("scene arrays are inconsistent:") + ((flag & kPackBadVertexIndex) ? " triangleVertexIndex out of range;" : "") +
+           ((flag & kPackBadMaterial) ? " triangleMaterialId out of range;" : "") +
+           ((flag & kPackBadCsr) ? " scenePixelTriangleListStart is not a monotone CSR;" : "") +
+           ((flag & kPackBadListEntry) ? " scenePixelTriangleList entry out of range;" : "") +
+           ((flag & kPackListTooLong) ? " a grid cell lists 131072 triangles or more (unsupported);" : "");
+}
+
+// The kernels' view of the scene's buffers, and the bytes they hold.
+static void bind_view(Scene* s, uint32_t triangleCount, uint32_t materialCount, uint32_t lightCount, int n) {
+    SceneView& v = s->view;
+    v.triGeo = (const float4*)s->triGeo.p;
+    v.triShade = (const float4*)s->triShade.p;
+    v.bricks = (const uint4*)s->bricks.p;
+    v.cellRange = (const uint2*)s->cellRange.p;
+    v.cellList = (const uint32_t*)s->cellList.p;
+    v.faceMask = (const uint32_t*)s->faceMask.p;
+    v.planes = (const float*)s->planes.p;
+    v.matSize = (const uint2*)s->matSize.p;
+    v.matStart = (const int32_t*)s->matStart.p;
+    v.textures = (const uchar4*)s->textures.p;
+    v.lights = (const Light*)s->lights.p;
+    v.triangleCount = triangleCount;
+    v.materialCount = materialCount;
+    v.lightCount = lightCount;
+    v.n = n;
+    v.nb = n >= 4 ? n / 4 : 1;
+    s->bytes = s->triGeo.bytes + s->triShade.bytes + s->bricks.bytes + s->cellRange.bytes + s->cellList.bytes + s->faceMask.bytes + s->planes.bytes +
+               s->matSize.bytes + s->matStart.bytes + s->textures.bytes + s->lights.bytes;
+}
+
+// Triangles: raw reference arrays in device memory -> d->triGeo / d->triShade (pack_triangles_kernel; bad indices and material ids are
+// or-ed into error[0]).  Enqueued on the default stream.
+static bool pack_stage(Scene* d, uint32_t N, uint32_t V, uint32_t materialCount, const float4* vertex, const int4* triIdx, const int32_t* triMat,
+                       const float2* triUv, const float4* triNormal, uint32_t* error, std::string& err) {
+    if (!d->triGeo.alloc(sizeof(float4) * 4 * (size_t)N, err) || !d->triShade.alloc(sizeof(float4) * 8 * (size_t)N, err)) return false;
+    if (N)
+        pack_triangles_kernel<<<(N + 255) / 256, 256>>>(N, V, materialCount, vertex, triIdx, triMat, triUv, triNormal, (float4*)d->triGeo.p,
+                                                        (float4*)d->triShade.p, error);
+    return true;
+}
+
+// The grid: given in device memory (boxMin, gridStart and `total` list entries already in d->cellList), or built on the device at n cells
+// per axis when gridStart is null; repacked into d->bricks / cellRange / faceMask / planes.  Enqueued on the default stream (the
+// builder and the non-empty cell count synchronise it); problems found on the device are or-ed into error[0], which error[1] must
+// be free to use.
+static bool grid_stage(Scene* d, int n, uint32_t V, const float4* vertex, uint32_t N, const int4* triIdx, const float4* boxMin,
+                       const uint32_t* gridStart, uint32_t total, uint32_t* error, std::string& err) {
+    const int nb = n >= 4 ? n / 4 : 1;
+    const size_t nBricks = (size_t)nb * nb * nb;
+    // super-brick records of the three-level walk follow the brick records (rt_walk.h) -- in builds whose trace kernel has that level
+    const int superPolicy = OCLR_SUPER_LEVEL ? super_policy(1) : 0;
+    const int ns = superPolicy > 0 ? super_bricks_per_axis(n) : 0;
+    const size_t nSuper = superPolicy > 0 ? super_brick_records(n) : 0;
+    DeviceGrid grid;
+    DeviceBuffer counts, rankBase, scanTmp, cellIds;
+    auto done = [&](bool ok) {
+        for (DeviceBuffer* b : {&counts, &rankBase, &scanTmp, &cellIds, &grid.boxMin, &grid.start}) b->release();
+        return ok;
+    };
+    if (!gridStart) {
+        // the builder gathers vertices by index before the packer's check has been read: the indices are checked first
+        if (N) check_indices_kernel<<<(N + 255) / 256, 256>>>(N, V, triIdx, error + 1);
+        uint32_t bad = 0;
+        OCLR_CUDA(cudaMemcpy(&bad, error + 1, sizeof(uint32_t), cudaMemcpyDeviceToHost));
+        if (bad) {
+            err = "scene arrays are inconsistent: triangleVertexIndex out of range;";
+            return false;
+        }
+        if (!grid_build_on_device(n, V, vertex, N, triIdx, grid, err)) return false;
+        d->cellList.release();
+        d->cellList = grid.list;   // handed over: the buffer an uploaded list would occupy
+        grid.list = DeviceBuffer();
+        boxMin = (const float4*)grid.boxMin.p;
+        gridStart = (const uint32_t*)grid.start.p;
+        total = grid.total;
+    }
+    if (!d->bricks.alloc(sizeof(uint4) * (nBricks + nSuper), err) || !d->planes.alloc(sizeof(float) * 3 * (n + 1), err) ||
+        !counts.alloc(sizeof(uint32_t) * (nBricks + 1), err) || !rankBase.alloc(sizeof(uint32_t) * (nBricks + 1), err))
+        return done(false);
+    cudaMemsetAsync(counts.p, 0, sizeof(uint32_t) * (nBricks + 1), 0);
+    split_planes_kernel<<<(n + 1 + 127) / 128, 128>>>(boxMin, n, (float*)d->planes.p);
+    brick_count_kernel<<<(unsigned)((nBricks + 127) / 128), 128>>>(gridStart, n, nb, total, (uint32_t*)counts.p, error);
+    size_t tmpBytes = 0;
+    cub::DeviceScan::ExclusiveSum(nullptr, tmpBytes, (const uint32_t*)counts.p, (uint32_t*)rankBase.p, (int)(nBricks + 1));
+    if (!scanTmp.alloc(tmpBytes, err)) return done(false);
+    cub::DeviceScan::ExclusiveSum(scanTmp.p, tmpBytes, (const uint32_t*)counts.p, (uint32_t*)rankBase.p, (int)(nBricks + 1));
+    if (total) check_list_kernel<<<(total + 255) / 256, 256>>>((const uint32_t*)d->cellList.p, total, N, error);
+    uint32_t nonEmpty = 0;
+    cudaMemcpyAsync(&nonEmpty, (const uint32_t*)rankBase.p + nBricks, sizeof(uint32_t), cudaMemcpyDeviceToHost, 0);
+    cudaError_t e = cudaStreamSynchronize(0);
+    if (e != cudaSuccess) {
+        err = std::string("scene repack: ") + cudaGetErrorString(e);
+        return done(false);
+    }
+    if (nonEmpty >= (1u << 29)) {
+        err = "too many non-empty grid cells (>= 2^29)";
+        return done(false);
+    }
+    const size_t ne = nonEmpty ? nonEmpty : 1;
+    if (!d->cellRange.alloc(sizeof(uint2) * ne, err) || !d->faceMask.alloc(sizeof(uint32_t) * 6 * ne, err) || !cellIds.alloc(sizeof(uint32_t) * ne, err))
+        return done(false);
+    brick_write_kernel<<<(unsigned)((nBricks + 127) / 128), 128>>>(gridStart, n, nb, total, (const uint32_t*)rankBase.p, (uint4*)d->bricks.p,
+                                                                  (uint2*)d->cellRange.p, (uint32_t*)cellIds.p, error);
+    if (nSuper) {
+        cudaMemsetAsync((uint4*)d->bricks.p + nBricks, 0, sizeof(uint4) * nSuper, 0);
+        super_brick_kernel<<<(unsigned)(ns * ns * ns), 64>>>((uint4*)d->bricks.p, nb, ns);
+    }
+    if (nonEmpty)
+        face_mask_kernel<<<(unsigned)(((size_t)nonEmpty * 6 + 255) / 256), 256>>>(gridStart, n, total, nonEmpty, (const uint32_t*)cellIds.p,
+                                                                                 (const uint2*)d->cellRange.p, (const uint32_t*)d->cellList.p,
+                                                                                 (uint32_t*)d->faceMask.p);
+    else
+        cudaMemsetAsync(d->faceMask.p, 0xFF, sizeof(uint32_t) * 6, 0);
+    return done(true);   // (the temporaries are freed in stream order behind the kernels that read them)
+}
+
 static bool scene_upload(Scene* s, const HostScene& h, std::string& err, const std::function<void(Scene*)>* early, UploadShare* share) {
     ShardCtx* ctx = share ? share->ctx : nullptr;
     ShardBarriers barriers(ctx);   // (any early return below still passes the barriers the other GPUs' threads wait at)
@@ -1063,29 +1212,10 @@ static bool scene_upload(Scene* s, const HostScene& h, std::string& err, const s
     const bool buildGrid = !h.gridStart;   // no grid given: SceneTriangleList::New runs on the device (grid_builder.cuh)
 
     const size_t N = h.triangleCount;
-    const int n = h.axesDivCount, nb = n >= 4 ? n / 4 : 1;
-    const size_t cells = (size_t)n * n * n, nBricks = (size_t)nb * nb * nb;
-    // super-brick records of the three-level walk follow the brick records (rt_walk.h) -- in builds whose trace kernel has that level
-    const int superPolicy = OCLR_SUPER_LEVEL ? super_policy(1) : 0;
-    const int ns = superPolicy > 0 ? super_bricks_per_axis(n) : 0;
-    const size_t nSuper = superPolicy > 0 ? super_brick_records(n) : 0;
+    const int n = h.axesDivCount;
+    const size_t cells = (size_t)n * n * n;
     // ring depth of this scene's paths (host data only, and decided before the early hook below starts a frame on the scene)
-    s->ringSlots = 2;
-    for (uint32_t m = 0; m < h.materialCount && s->ringSlots == 2; ++m)
-        for (int ch : {(int)kChReflection, (int)kChTransparency}) {
-            // a channel that is present but black everywhere (the plugin's 1x1 fallback for "no reflection") spawns nothing either: the
-            // segment multiplier is 0 < 3/256 (:684, :703).  Large maps are not scanned: taken as "may be non-zero"
-            const uint2 size = h.matSize[kMaterialChannels * m + ch];
-            const size_t texels = (size_t)size.x * size.y;
-            if (texels == 0) continue;
-            bool black = texels <= ((size_t)1 << 20);
-            const uchar4* t = h.textures + h.matStart[kMaterialChannels * m + ch];
-            for (size_t i = 0; black && i < texels; ++i) black = (t[i].x | t[i].y | t[i].z) == 0;
-            if (!black) s->ringSlots = kRingSize;
-        }
-    if (const char* v = getenv("OCLR_RING_SLOTS")) s->ringSlots = std::max(s->ringSlots, std::min(atoi(v), (int)kRingSize));   // (test knob: more, never fewer)
-    s->hasBump = false;
-    for (uint32_t m = 0; m < h.materialCount; ++m) s->hasBump |= h.matSize[kMaterialChannels * m + kChBump].x > 0u;
+    material_rules(h, s->ringSlots, s->hasBump);
     uint32_t total = buildGrid ? 0u : h.gridStart[cells];
     if (total && !h.gridList) {
         err = "scenePixelTriangleList missing";
@@ -1096,7 +1226,7 @@ static bool scene_upload(Scene* s, const HostScene& h, std::string& err, const s
 
     // 1a. everything the primary-ray round needs -- triangles, materials, lights -- goes first: raw reference arrays -> HBM straight
     //     from the caller's memory (async on the default stream), repacked by pack_triangles_kernel
-    DeviceBuffer vertex, triIdx, triMat, triUv, triNormal, boxMin, gridStart, counts, rankBase, scanTmp, errFlag, cellIds;
+    DeviceBuffer vertex, triIdx, triMat, triUv, triNormal, boxMin, gridStart, errFlag;
     std::vector<ShardArray> sharded;   // (kept for the self-test of the second group)
     bool ok;
     if (ctx) {
@@ -1140,27 +1270,14 @@ static bool scene_upload(Scene* s, const HostScene& h, std::string& err, const s
              s->textures.upload(h.textures, sizeof(uchar4) * h.texturesSize, err) &&
              s->lights.upload(lights.data(), sizeof(Light) * lights.size(), err);
     }
-    ok = ok && s->triGeo.alloc(sizeof(float4) * 4 * N, err) && s->triShade.alloc(sizeof(float4) * 8 * N, err) &&
-         errFlag.alloc(sizeof(uint32_t) * 2, err);
+    ok = ok && errFlag.alloc(sizeof(uint32_t) * 2, err);
     if (ok) {
         cudaMemsetAsync(errFlag.p, 0, sizeof(uint32_t) * 2, 0);
-        if (N)
-            pack_triangles_kernel<<<(unsigned)((N + 255) / 256), 256>>>((uint32_t)N, h.vertexCount, h.materialCount, (const float4*)vertex.p,
-                                                                      (const int4*)triIdx.p, (const int32_t*)triMat.p, (const float2*)triUv.p,
-                                                                      (const float4*)triNormal.p, (float4*)s->triGeo.p,
-                                                                      (float4*)s->triShade.p, (uint32_t*)errFlag.p);
-        SceneView& v = s->view;   // the part of the view the logic kernel reads (the grid part follows below)
-        v.triGeo = (const float4*)s->triGeo.p;
-        v.triShade = (const float4*)s->triShade.p;
-        v.matSize = (const uint2*)s->matSize.p;
-        v.matStart = (const int32_t*)s->matStart.p;
-        v.textures = (const uchar4*)s->textures.p;
-        v.lights = (const Light*)s->lights.p;
-        v.triangleCount = h.triangleCount;
-        v.materialCount = h.materialCount;
-        v.lightCount = h.lightCount;
-        v.n = n;
-        v.nb = nb;
+        ok = pack_stage(s, (uint32_t)N, h.vertexCount, h.materialCount, (const float4*)vertex.p, (const int4*)triIdx.p, (const int32_t*)triMat.p,
+                        (const float2*)triUv.p, (const float4*)triNormal.p, (uint32_t*)errFlag.p, err);
+    }
+    if (ok) {
+        bind_view(s, h.triangleCount, h.materialCount, h.lightCount, n);   // the logic kernel's part (the grid part is bound again below)
         // RaytraceAll uploads its camera lists and starts the primary-ray round HERE, on a stream of its own, so that round runs
         // under the upload of the grid (94 of config 2's 133 MB) instead of after it
         if (early && *early) (*early)(s);
@@ -1169,72 +1286,14 @@ static bool scene_upload(Scene* s, const HostScene& h, std::string& err, const s
     ok = ok && (buildGrid || (ctx ? (shard_wait_group(ctx, 1, err) && shard_verify(share->rank, sharded.data(), (int)sharded.size(), 1, err))
                                   : (boxMin.upload(h.boxMin, sizeof(float4) * (n + 1), err) &&
                                      gridStart.upload(h.gridStart, sizeof(uint32_t) * (cells + 1), err) &&
-                                     s->cellList.upload(h.gridList, sizeof(uint32_t) * total, err)))) &&
-         s->bricks.alloc(sizeof(uint4) * (nBricks + nSuper), err) && s->planes.alloc(sizeof(float) * 3 * (n + 1), err) &&
-         counts.alloc(sizeof(uint32_t) * (nBricks + 1), err) && rankBase.alloc(sizeof(uint32_t) * (nBricks + 1), err);
-    uint32_t nonEmpty = 0, flag = 0;
-    if (ok && buildGrid) {
-        for (size_t i = 0; ok && i < N; ++i) {  // the builder gathers vertices by index before the packers have validated them
-            const int32_t* vi = h.triIdx + 4 * i;
-            ok = (uint32_t)vi[0] < h.vertexCount && (uint32_t)vi[1] < h.vertexCount && (uint32_t)vi[2] < h.vertexCount;
-        }
-        if (!ok) err = "scene arrays are inconsistent: triangleVertexIndex out of range;";
-    }
-    if (ok && buildGrid) {
-        DeviceGrid grid;
-        ok = grid_build_on_device(n, h.vertexCount, (const float4*)vertex.p, (uint32_t)N, (const int4*)triIdx.p, grid, err);
-        if (ok) {  // hand the three arrays over: same buffers an uploaded grid would occupy
-            boxMin = grid.boxMin;
-            gridStart = grid.start;
-            s->cellList = grid.list;
-            total = grid.total;
-        }
-    }
-    if (ok) {
-        // 2. repack on the device
-        cudaMemsetAsync(counts.p, 0, sizeof(uint32_t) * (nBricks + 1), 0);
-        split_planes_kernel<<<(n + 1 + 127) / 128, 128>>>((const float4*)boxMin.p, n, (float*)s->planes.p);
-        brick_count_kernel<<<(unsigned)((nBricks + 127) / 128), 128>>>((const uint32_t*)gridStart.p, n, nb, total, (uint32_t*)counts.p,
-                                                                      (uint32_t*)errFlag.p);
-        size_t tmpBytes = 0;
-        cub::DeviceScan::ExclusiveSum(nullptr, tmpBytes, (const uint32_t*)counts.p, (uint32_t*)rankBase.p, (int)(nBricks + 1));
-        ok = scanTmp.alloc(tmpBytes, err);
-        if (ok) {
-            cub::DeviceScan::ExclusiveSum(scanTmp.p, tmpBytes, (const uint32_t*)counts.p, (uint32_t*)rankBase.p, (int)(nBricks + 1));
-            if (total) check_list_kernel<<<(total + 255) / 256, 256>>>((const uint32_t*)s->cellList.p, total, (uint32_t)N, (uint32_t*)errFlag.p);
-            cudaMemcpyAsync(&nonEmpty, (const uint32_t*)rankBase.p + nBricks, sizeof(uint32_t), cudaMemcpyDeviceToHost, 0);
-            cudaError_t e = cudaStreamSynchronize(0);
-            if (e != cudaSuccess) {
-                err = std::string("scene repack: ") + cudaGetErrorString(e);
-                ok = false;
-            }
-        }
-        if (ok && nonEmpty >= (1u << 29)) {
-            err = "too many non-empty grid cells (>= 2^29)";
-            ok = false;
-        }
-        if (ok) ok = s->cellRange.alloc(sizeof(uint2) * (nonEmpty ? nonEmpty : 1), err);
-        if (ok) ok = s->faceMask.alloc(sizeof(uint32_t) * 6 * (size_t)(nonEmpty ? nonEmpty : 1), err);
-        if (ok) ok = cellIds.alloc(sizeof(uint32_t) * (size_t)(nonEmpty ? nonEmpty : 1), err);
-        if (ok) {
-            brick_write_kernel<<<(unsigned)((nBricks + 127) / 128), 128>>>((const uint32_t*)gridStart.p, n, nb, total, (const uint32_t*)rankBase.p,
-                                                                          (uint4*)s->bricks.p, (uint2*)s->cellRange.p, (uint32_t*)cellIds.p,
-                                                                          (uint32_t*)errFlag.p);
-            if (nSuper) {
-                cudaMemsetAsync((uint4*)s->bricks.p + nBricks, 0, sizeof(uint4) * nSuper, 0);
-                super_brick_kernel<<<(unsigned)(ns * ns * ns), 64>>>((uint4*)s->bricks.p, nb, ns);
-            }
-            if (nonEmpty)
-                face_mask_kernel<<<(unsigned)(((size_t)nonEmpty * 6 + 255) / 256), 256>>>((const uint32_t*)gridStart.p, n, total, nonEmpty,
-                                                                                         (const uint32_t*)cellIds.p, (const uint2*)s->cellRange.p,
-                                                                                         (const uint32_t*)s->cellList.p, (uint32_t*)s->faceMask.p);
-            else
-                cudaMemsetAsync(s->faceMask.p, 0xFF, sizeof(uint32_t) * 6, 0);
-            cudaMemcpyAsync(&flag, errFlag.p, sizeof(uint32_t), cudaMemcpyDeviceToHost, 0);
-        }
-    }
+                                     s->cellList.upload(h.gridList, sizeof(uint32_t) * total, err))));
+    // 2. repack on the device
+    ok = ok && grid_stage(s, n, h.vertexCount, (const float4*)vertex.p, (uint32_t)N, (const int4*)triIdx.p, (const float4*)boxMin.p,
+                          (const uint32_t*)gridStart.p, total, (uint32_t*)errFlag.p, err);
+    uint32_t flag = 0;
+    if (ok) cudaMemcpyAsync(&flag, errFlag.p, sizeof(uint32_t), cudaMemcpyDeviceToHost, 0);
     cudaError_t e = cudaStreamSynchronize(0);
-    DeviceBuffer* tmp[] = {&vertex, &triIdx, &triMat, &triUv, &triNormal, &boxMin, &gridStart, &counts, &rankBase, &scanTmp, &errFlag, &cellIds};
+    DeviceBuffer* tmp[] = {&vertex, &triIdx, &triMat, &triUv, &triNormal, &boxMin, &gridStart, &errFlag};
     for (DeviceBuffer* b : tmp) b->release();
     if (!ok) return false;
     if (e != cudaSuccess || (e = cudaGetLastError()) != cudaSuccess) {
@@ -1242,32 +1301,10 @@ static bool scene_upload(Scene* s, const HostScene& h, std::string& err, const s
         return false;
     }
     if (flag) {
-        err = std::string("scene arrays are inconsistent:") + ((flag & kPackBadVertexIndex) ? " triangleVertexIndex out of range;" : "") +
-              ((flag & kPackBadMaterial) ? " triangleMaterialId out of range;" : "") +
-              ((flag & kPackBadCsr) ? " scenePixelTriangleListStart is not a monotone CSR;" : "") +
-              ((flag & kPackBadListEntry) ? " scenePixelTriangleList entry out of range;" : "") +
-              ((flag & kPackListTooLong) ? " a grid cell lists 131072 triangles or more (unsupported);" : "");
+        err = pack_error_message(flag);
         return false;
     }
-    SceneView& v = s->view;
-    v.triGeo = (const float4*)s->triGeo.p;
-    v.triShade = (const float4*)s->triShade.p;
-    v.bricks = (const uint4*)s->bricks.p;
-    v.cellRange = (const uint2*)s->cellRange.p;
-    v.cellList = (const uint32_t*)s->cellList.p;
-    v.faceMask = (const uint32_t*)s->faceMask.p;
-    v.planes = (const float*)s->planes.p;
-    v.matSize = (const uint2*)s->matSize.p;
-    v.matStart = (const int32_t*)s->matStart.p;
-    v.textures = (const uchar4*)s->textures.p;
-    v.lights = (const Light*)s->lights.p;
-    v.triangleCount = h.triangleCount;
-    v.materialCount = h.materialCount;
-    v.lightCount = h.lightCount;
-    v.n = n;
-    v.nb = nb;
-    s->bytes = s->triGeo.bytes + s->triShade.bytes + s->bricks.bytes + s->cellRange.bytes + s->cellList.bytes + s->faceMask.bytes + s->planes.bytes +
-               s->matSize.bytes + s->matStart.bytes + s->textures.bytes + s->lights.bytes;
+    bind_view(s, h.triangleCount, h.materialCount, h.lightCount, n);
     return true;
 }
 
@@ -1290,9 +1327,7 @@ Scene* scene_create(int device, const HostScene& h, std::string& err, const std:
 void scene_destroy(Scene* s) {
     if (!s) return;
     cudaSetDevice(s->device);
-    DeviceBuffer* all[] = {&s->triGeo, &s->triShade, &s->bricks, &s->cellRange, &s->cellList, &s->faceMask, &s->planes, &s->matSize,
-                           &s->matStart, &s->textures, &s->lights};
-    for (DeviceBuffer* b : all) b->release();
+    for (DeviceBuffer* b : s->buffers()) b->release();
     delete s;
 }
 
@@ -1341,8 +1376,9 @@ static bool frame_setup_common(Frame* f, std::string& err, bool sync = true) {
     return true;
 }
 
-static bool frame_setup(Frame* f, const uint32_t* camStart, const uint32_t* camEnd, const uint32_t* camList, size_t listSize,
-                        std::string& err, bool sync, StagedCamLists* staged) {
+// Caller-supplied (or staged) camera lists into the frame, range-checked on the device.
+static bool frame_upload_lists(Frame* f, const uint32_t* camStart, const uint32_t* camEnd, const uint32_t* camList, size_t listSize,
+                               std::string& err, StagedCamLists* staged) {
     OCLR_CUDA(cudaSetDevice(f->scene->device));
     const size_t P = (size_t)f->cam.width * f->cam.height;
     if (staged && staged->start && !staged->adopted) {   // already in HBM (uploaded together with the scene, shard_upload)
@@ -1376,13 +1412,19 @@ static bool frame_setup(Frame* f, const uint32_t* camStart, const uint32_t* camE
     check_camera_lists_kernel<<<(unsigned)std::min<size_t>((std::max(P, listSize) + 255) / 256, (size_t)f->scene->smCount * 8), 256>>>(
         (const uint32_t*)f->camStart.p, (const uint32_t*)f->camEnd.p, (const uint32_t*)f->camList.p, (uint32_t)P, (uint32_t)listSize,
         f->scene->view.triangleCount, (uint32_t*)f->camCheck.p);
-    return frame_setup_common(f, err, sync);
+    f->deviceLists = false;
+    f->listsGen = f->scene->geometryGen;
+    return true;
 }
 
 // CameraTriangleList::New on the device (cam_builder.cuh): the frame's camera lists are built from the resident scene.
 static bool frame_build_camera_lists(Frame* f, std::string& err) {
     Scene* s = f->scene;
     OCLR_CUDA(cudaSetDevice(s->device));
+    for (DeviceBuffer* b : {&f->camStart, &f->camEnd, &f->camList, &f->camCheck}) b->release();   // (a rebuild: the old lists go)
+    f->camListSize = 0;
+    f->deviceLists = true;
+    f->listsGen = kNoLists;
     const uint32_t W = f->cam.width, H = f->cam.height, N = s->view.triangleCount;
     const uint32_t P = W * H;
     if ((uint64_t)W * H >= 0xFFFFFFFFull) {
@@ -1488,7 +1530,19 @@ static bool frame_build_camera_lists(Frame* f, std::string& err) {
         err = std::string("camera-list builder: ") + cudaGetErrorString(e);
         return done(false);
     }
+    f->listsGen = s->geometryGen;
     return done(true);
+}
+
+// Lists for the scene's current geometry, before anything reads them: device-built lists are rebuilt after a geometry edit; caller
+// lists made for older geometry may name triangles that no longer exist, so the frame refuses until it is given new ones.
+static bool frame_lists_current(Frame* f, std::string& err) {
+    if (f->listsGen == f->scene->geometryGen) return true;
+    if (f->deviceLists) return frame_build_camera_lists(f, err);
+    err = f->listsGen == kNoLists ? "the frame has no camera triangle lists (its last camera change failed): set a camera again"
+                                  : "the scene's geometry changed since the frame's camera triangle lists were made: give the frame new lists "
+                                    "(oclr_frame_set_camera_lists) or let the device build them (oclr_frame_set_camera)";
+    return false;
 }
 
 void staged_release(StagedCamLists& st) {
@@ -1513,8 +1567,9 @@ Frame* frame_create(Scene* s, const Camera& cam, const uint32_t* camStart, const
     f->scene = s;
     f->device = s->device;
     f->cam = cam;
-    const bool ok = (camStart || (staged && staged->start)) ? frame_setup(f, camStart, camEnd, camList, camListSize, err, sync, staged)
-                             : (frame_build_camera_lists(f, err) && frame_setup_common(f, err));   // no lists given: build them on the device
+    const bool ok = (camStart || (staged && staged->start))
+                        ? frame_upload_lists(f, camStart, camEnd, camList, camListSize, err, staged) && frame_setup_common(f, err, sync)
+                        : (frame_build_camera_lists(f, err) && frame_setup_common(f, err));   // no lists given: build them on the device
     if (!ok) {
         frame_destroy(f);
         return nullptr;
@@ -1522,7 +1577,10 @@ Frame* frame_create(Scene* s, const Camera& cam, const uint32_t* camStart, const
     return f;
 }
 
-size_t frame_camera_list_size(const Frame* f) { return f ? f->camListSize : 0; }
+size_t frame_camera_list_size(Frame* f) {
+    std::string ignored;   // (frame_read_camera_lists reports why stale lists cannot be read)
+    return f && frame_lists_current(f, ignored) ? f->camListSize : 0;
+}
 
 bool frame_read_camera_lists(Frame* f, uint32_t* start, uint32_t* end, uint32_t* list, std::string& err) {
     if (!f) {
@@ -1530,6 +1588,7 @@ bool frame_read_camera_lists(Frame* f, uint32_t* start, uint32_t* end, uint32_t*
         return false;
     }
     OCLR_CUDA(cudaSetDevice(f->scene->device));
+    if (!frame_lists_current(f, err)) return false;
     const size_t P = (size_t)f->cam.width * f->cam.height;
     OCLR_CUDA(cudaMemcpy(start, f->camStart.p, sizeof(uint32_t) * P, cudaMemcpyDeviceToHost));
     OCLR_CUDA(cudaMemcpy(end, f->camEnd.p, sizeof(uint32_t) * P, cudaMemcpyDeviceToHost));
@@ -1902,12 +1961,12 @@ static bool launch_wavefront(Frame* f, const SceneView& S, const FrameView& Fall
             return false;
         }
         const uint32_t Q = (uint32_t)Q64;
-        if (Q > sl.ps.capacity) {
+        if (path_state_regrow(sl.ps.capacity, sl.ps.ringSlots, Q, f->scene->ringSlots)) {
             for (DeviceBuffer* b : sl.tail_buffers()) b->release(st);
             if (!sl.ps.reserve(Q, f->scene->ringSlots, st, err)) return false;
             sl.tailCapacity = 0;
-            if (handoff_domain(Q)) {   // small launch domain: its trace tail is handed to wf_tail_kernel (rt_tail.cuh)
-                sl.tailCapacity = 2 * Q;   // (every ray of a round could be given up: the list cannot overflow)
+            if (handoff_domain(sl.ps.capacity)) {   // small launch domain: its trace tail is handed to wf_tail_kernel (rt_tail.cuh)
+                sl.tailCapacity = 2 * sl.ps.capacity;   // (every ray of a round could be given up: the list cannot overflow)
                 const size_t c = sl.tailCapacity;
                 if (!sl.tailEntries.alloc(sizeof(uint4) * c, err, st) || !sl.tailO.alloc(sizeof(float4) * c, err, st) ||
                     !sl.tailD.alloc(sizeof(float4) * c, err, st) || !sl.tailS0.alloc(sizeof(float4) * c, err, st) ||
@@ -2122,6 +2181,7 @@ bool frame_render(Frame* f, uint32_t sampleCount, uint32_t sampleBegin, uint32_t
         err = "empty render request";
         return false;
     }
+    if (!frame_lists_current(f, err)) return false;
     FrameView F = {};
     F.sampleCount = sampleCount;
     F.sampleBegin = sampleBegin;
@@ -2147,6 +2207,7 @@ bool frame_render_bands(Frame* f, uint32_t sampleCount, uint32_t sampleBegin, ui
         return false;
     }
     if (world == 1) return frame_render(f, sampleCount, sampleBegin, sampleEnd, 0, f->cam.height, variant, count, stream, stats, err);
+    if (!frame_lists_current(f, err)) return false;
     FrameView F = {};
     F.sampleCount = sampleCount;
     F.sampleBegin = sampleBegin;
@@ -2174,6 +2235,7 @@ bool frame_prelaunch(Frame* f, uint32_t sampleCount, uint32_t bandRows, uint32_t
         return false;
     }
     OCLR_CUDA(cudaSetDevice(f->scene->device));
+    if (!frame_lists_current(f, err)) return false;
     FrameView F = {};
     F.sampleCount = sampleCount;
     F.sampleBegin = 0;
@@ -2811,6 +2873,202 @@ bool scene_radiance(Scene* s, const Camera* cam, size_t count, const float* orig
         if (!rays.download(off, n, err)) return false;
     }
     return rays.finish(stats, drv.launches, drv.rounds, err);
+}
+
+// ---- edits of a resident scene and of a frame's camera -----------------------------------------------------------------------------------
+bool frame_set_camera(Frame* f, const Camera& cam, const uint32_t* camStart, const uint32_t* camEnd, const uint32_t* camList, size_t listSize,
+                      std::string& err) {
+    if (!f) {
+        err = "null frame";
+        return false;
+    }
+    if (cam.width != f->cam.width || cam.height != f->cam.height) {
+        err = "the new camera is " + std::to_string(cam.width) + "x" + std::to_string(cam.height) + ", the frame " + std::to_string(f->cam.width) +
+              "x" + std::to_string(f->cam.height) + ": a frame keeps its image size (create a new frame)";
+        return false;
+    }
+    // From here on the frame holds the new camera; whatever fails below leaves it without lists (it refuses to render until a camera is
+    // set successfully), never with the old camera's lists under the new camera.
+    f->cam = cam;
+    f->deviceLists = false;
+    f->listsGen = kNoLists;
+    OCLR_CUDA(cudaSetDevice(f->device));
+    // every launch that may read the old lists has finished (a round started ahead included) before they are replaced
+    OCLR_CUDA(cudaDeviceSynchronize());
+    f->prelaunched = false;
+    for (DeviceBuffer* b : {&f->camStart, &f->camEnd, &f->camList, &f->camCheck}) b->release();
+    f->camListSize = 0;
+    if (!camStart) return frame_build_camera_lists(f, err);
+    if (!frame_upload_lists(f, camStart, camEnd, camList, listSize, err, nullptr)) {
+        f->listsGen = kNoLists;
+        return false;
+    }
+    OCLR_CUDA(cudaStreamSynchronize(0));   // (the caller's arrays may go once the call returns)
+    return true;
+}
+
+// The device arrays of a geometry update: caller device memory used in place, or host arrays uploaded.
+struct GeometryInputs {
+    DeviceBuffer vertex, triIdx, triMat, triUv, triNormal, boxMin, gridStart;
+    const void* p[7] = {};   // the arrays in that order, in device memory
+    ~GeometryInputs() {
+        for (DeviceBuffer* b : {&vertex, &triIdx, &triMat, &triUv, &triNormal, &boxMin, &gridStart}) b->release();
+    }
+};
+
+bool scene_update(Scene* s, const HostScene& h, unsigned parts, bool deviceMemory, std::string& err) {
+    if (!s) {
+        err = "null scene";
+        return false;
+    }
+    const bool lights = parts & kSceneLights, materials = parts & kSceneMaterials, geometry = parts & kSceneGeometry;
+    // The arrays of the parts named, checked like a scene of their own (the resident grid size stands in when the geometry stays).
+    HostScene v;
+    if (geometry) {
+        v.vertexCount = h.vertexCount;
+        v.vertex = h.vertex;
+        v.triangleCount = h.triangleCount;
+        v.triIdx = h.triIdx;
+        v.triMat = h.triMat;
+        v.triUv = h.triUv;
+        v.triNormal = h.triNormal;
+        v.axesDivCount = h.axesDivCount;
+        v.boxMin = h.boxMin;
+        v.gridStart = h.gridStart;
+        v.gridList = h.gridList;
+    } else {
+        v.axesDivCount = s->view.n;
+    }
+    if (materials) {
+        v.materialCount = h.materialCount;
+        v.matSize = h.matSize;
+        v.matStart = h.matStart;
+        v.texturesSize = h.texturesSize;
+        v.textures = h.textures;
+    }
+    if (lights) {
+        v.lightCount = h.lightCount;
+        v.lightType = h.lightType;
+        v.lightPos = h.lightPos;
+        v.lightDir = h.lightDir;
+        v.lightColour = h.lightColour;
+        v.lightRadius = h.lightRadius;
+        v.lightHalf = h.lightHalf;
+    }
+    if (!validate_scene(v, err, true)) return false;
+    OCLR_CUDA(cudaSetDevice(s->device));
+    const int n = v.axesDivCount;
+    const size_t N = v.triangleCount, cells = (size_t)n * n * n;
+    const bool buildGrid = geometry && !v.gridStart;
+    if (geometry && deviceMemory) {
+        const struct {
+            const void* p;
+            size_t align;
+            const char* what;
+        } arrays[] = {{v.vertex, 16, "vertex"}, {v.triIdx, 16, "triangleVertexIndex"}, {v.triMat, 4, "triangleMaterialId"},
+                      {v.triUv, 8, "triangleUv"}, {v.triNormal, 16, "triangleNormal"}, {v.boxMin, 16, "sceneBoxMin"},
+                      {v.gridStart, 4, "scenePixelTriangleListStart"}, {v.gridList, 4, "scenePixelTriangleList"}};
+        for (const auto& a : arrays)
+            if (a.p && !query_pointer_ok(s, a.p, a.align, a.what, err)) return false;
+    }
+    // every piece of work already enqueued on the device (renders and queries on this scene among it) ends before anything changes
+    OCLR_CUDA(cudaDeviceSynchronize());
+    stage_reset(s->device);
+    // The new parts are built beside the resident ones and swapped in on success.  The scratch owns whatever it holds when the call
+    // ends: the new buffers after a failure (whichever way it returns), the replaced ones after a success.
+    struct Scratch {
+        Scene t;
+        DeviceBuffer errFlag;
+        ~Scratch() {
+            cudaDeviceSynchronize();   // (staged copies and kernels that touch the buffers have ended)
+            for (DeviceBuffer* b : t.buffers()) b->release();
+            errFlag.release();
+        }
+    } x;
+    Scene& t = x.t;
+    t.device = s->device;
+    GeometryInputs in;
+    std::vector<Light> packed;
+    if (!x.errFlag.alloc(sizeof(uint32_t) * 2, err)) return false;
+    OCLR_CUDA(cudaMemsetAsync(x.errFlag.p, 0, sizeof(uint32_t) * 2, 0));
+    uint32_t* flagDev = (uint32_t*)x.errFlag.p;
+    if (lights) {
+        pack_lights(v, packed);
+        if (!t.lights.upload(packed.data(), sizeof(Light) * packed.size(), err)) return false;
+    }
+    const uint32_t M = materials ? v.materialCount : s->view.materialCount;
+    if (materials) {
+        material_rules(v, t.ringSlots, t.hasBump);
+        if (!t.matSize.upload(v.matSize, sizeof(uint2) * kMaterialChannels * M, err) ||
+            !t.matStart.upload(v.matStart, sizeof(int32_t) * (kMaterialChannels * M + (M ? 1 : 0)), err) ||
+            !t.textures.upload(v.textures, sizeof(uchar4) * v.texturesSize, err))
+            return false;
+        if (!geometry && s->view.triangleCount)   // the resident triangles against the new material count
+            check_materials_kernel<<<(s->view.triangleCount + 255) / 256, 256>>>(s->view.triangleCount, M, s->view.triShade, flagDev);
+    }
+    if (geometry) {
+        uint32_t total = 0;
+        if (!buildGrid) {
+            if (deviceMemory)
+                OCLR_CUDA(cudaMemcpy(&total, v.gridStart + cells, sizeof(uint32_t), cudaMemcpyDeviceToHost));
+            else
+                total = v.gridStart[cells];
+            if (total && !v.gridList) {
+                err = "scenePixelTriangleList missing";
+                return false;
+            }
+        }
+        const size_t bytes[7] = {sizeof(float4) * v.vertexCount, sizeof(int4) * N, sizeof(int32_t) * N, sizeof(float2) * 3 * N,
+                                 sizeof(float4) * 3 * N, buildGrid ? 0 : sizeof(float4) * (n + 1), buildGrid ? 0 : sizeof(uint32_t) * (cells + 1)};
+        const void* src[7] = {v.vertex, v.triIdx, v.triMat, v.triUv, v.triNormal, v.boxMin, v.gridStart};
+        DeviceBuffer* dst[7] = {&in.vertex, &in.triIdx, &in.triMat, &in.triUv, &in.triNormal, &in.boxMin, &in.gridStart};
+        for (int i = 0; i < 7; ++i) {
+            if (deviceMemory) {
+                in.p[i] = src[i];
+            } else {
+                if (!dst[i]->upload(src[i], bytes[i], err)) return false;
+                in.p[i] = bytes[i] ? dst[i]->p : nullptr;
+            }
+        }
+        if (!buildGrid && !t.cellList.alloc(sizeof(uint32_t) * total, err)) return false;
+        if (total) {
+            if (deviceMemory)
+                OCLR_CUDA(cudaMemcpyAsync(t.cellList.p, v.gridList, sizeof(uint32_t) * total, cudaMemcpyDeviceToDevice, 0));
+            else if (!host_to_device(t.cellList.p, v.gridList, sizeof(uint32_t) * total, 0, err))
+                return false;
+        }
+        if (!pack_stage(&t, (uint32_t)N, v.vertexCount, M, (const float4*)in.p[0], (const int4*)in.p[1], (const int32_t*)in.p[2],
+                        (const float2*)in.p[3], (const float4*)in.p[4], flagDev, err) ||
+            !grid_stage(&t, n, v.vertexCount, (const float4*)in.p[0], (uint32_t)N, (const int4*)in.p[1], (const float4*)in.p[5],
+                        (const uint32_t*)in.p[6], total, flagDev, err))
+            return false;
+    }
+    uint32_t flag = 0;
+    cudaMemcpyAsync(&flag, flagDev, sizeof(uint32_t), cudaMemcpyDeviceToHost, 0);
+    cudaError_t e = cudaStreamSynchronize(0);
+    if (e != cudaSuccess || (e = cudaGetLastError()) != cudaSuccess) {
+        err = std::string("scene update: ") + cudaGetErrorString(e);
+        return false;
+    }
+    if (flag) {
+        err = pack_error_message(flag);
+        return false;
+    }
+    // success: the new parts in, the old ones out
+    if (lights) std::swap(s->lights, t.lights);
+    if (materials) {
+        for (DeviceBuffer Scene::*b : {&Scene::matSize, &Scene::matStart, &Scene::textures}) std::swap(s->*b, t.*b);
+        s->ringSlots = t.ringSlots;
+        s->hasBump = t.hasBump;
+    }
+    if (geometry) {
+        for (DeviceBuffer Scene::*b : {&Scene::triGeo, &Scene::triShade, &Scene::bricks, &Scene::cellRange, &Scene::cellList, &Scene::faceMask,
+                                       &Scene::planes})
+            std::swap(s->*b, t.*b);
+        ++s->geometryGen;
+    }
+    bind_view(s, geometry ? v.triangleCount : s->view.triangleCount, M, lights ? v.lightCount : s->view.lightCount, n);
+    return true;   // (the scratch releases the replaced buffers)
 }
 
 }  // namespace oclr

@@ -62,6 +62,14 @@ void pack_lights(const HostScene& h, std::vector<Light>& out);
 bool validate_scene(const HostScene& h, std::string& err, bool gridMayBeMissing = false);
 
 // ---- device runtime (runtime.cu) -----------------------------------------------------------------------------------
+// Path state of a launch domain (runtime.cu PathState): the capacity to reallocate at before a domain of Q paths with a ring of `slots`
+// slots runs on buffers sized for `capacity` paths and `ringSlots` slots, or 0 when they serve it as they are.  A new ring depth (a
+// materials edit changed the scene's) reallocates in both directions, at no smaller capacity.
+inline uint32_t path_state_regrow(uint32_t capacity, int ringSlots, uint32_t Q, int slots) {
+    if (Q <= capacity && slots == ringSlots) return 0;
+    return Q > capacity ? Q : capacity;
+}
+
 struct Scene;
 struct Frame;
 
@@ -112,9 +120,16 @@ Frame* frame_create(Scene* s, const Camera& cam, const uint32_t* camStart, const
                     size_t camListSize, std::string& err, bool sync = true,   // sync = false: the host arrays outlive the copies
                     StagedCamLists* staged = nullptr);
 void frame_destroy(Frame* f);
+// Edits of a resident scene (semantics in include/oclr_abi.h, oclr_scene_update): the parts named are rebuilt from `h` by the stages
+// scene_create runs, into new buffers swapped in on success.  deviceMemory: the geometry arrays are device memory of the scene's device.
+enum { kSceneLights = 1, kSceneMaterials = 2, kSceneGeometry = 4 };
+bool scene_update(Scene* s, const HostScene& h, unsigned parts, bool deviceMemory, std::string& err);
+// A new camera of the same image size for a frame: caller lists (camStart != nullptr) or lists built on the device.
+bool frame_set_camera(Frame* f, const Camera& cam, const uint32_t* camStart, const uint32_t* camEnd, const uint32_t* camList, size_t listSize,
+                      std::string& err);
 // camStart == nullptr: CameraTriangleList::New runs on the device from the resident scene (cam_builder.cuh).  The lists a frame
 // holds (uploaded or device-built) can be copied back: `list` needs frame_camera_list_size() entries.
-size_t frame_camera_list_size(const Frame* f);
+size_t frame_camera_list_size(Frame* f);
 bool frame_read_camera_lists(Frame* f, uint32_t* start, uint32_t* end, uint32_t* list, std::string& err);
 
 enum KernelVariant { kKernelSimple = 0, kKernelPipe = 2 };   // (1 was the lane-owned wavefront kernel, retired)
