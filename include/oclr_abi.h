@@ -341,7 +341,9 @@ int oclr_write_ppm16(const char* path, cl_uint width, cl_uint height, const cl_u
 int oclr_write_png16(const char* path, cl_uint width, cl_uint height, const cl_ushort* red, const cl_ushort* green, const cl_ushort* blue);
 
 /* Run-time options.  "slices": how many slices a launch domain is cut into (0 = automatic).  "ahead": tracing one round ahead
- * (0 never, 1 all segments but the camera's, 2 all, -1 automatic).  "devices": the "all devices" computation type
+ * (0 never, 1 all segments but the camera's, 2 all, -1 automatic).  "cull_hidden_lights": 1 (default) skips the shadow rays of lights
+ * on the side of a surface its segment does not see, whose contribution the shading never reads; 0 traces them all.  The planes are
+ * the same either way.  "devices": the "all devices" computation type
  * (RaytraceAll(deviceCount + 1, ...), the analogue of the reference's multi-device tile loop raytrace.c:507-556) renders on the first
  * `value` GPUs of the box (0 = all of them).  Returns 1 if the option is known. */
 int oclr_set_option(const char* name, int value);

@@ -165,6 +165,10 @@ int oclr_set_option(const char* name, int value) {
         set_ahead_mode(value);
         return 1;
     }
+    if (name && strcmp(name, "cull_hidden_lights") == 0) {
+        set_cull_hidden_lights(value);
+        return 1;
+    }
     if (name && strcmp(name, "devices") == 0) {   // the "all devices" computation type uses the first `value` GPUs (0 = all)
         g_allDevicesLimit.store(value < 0 ? 0 : value);
         return 1;

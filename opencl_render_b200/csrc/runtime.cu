@@ -1654,6 +1654,11 @@ static int ahead_mode_for(uint32_t paths) {
     return paths < 3000000u ? 2 : 1;
 }
 
+// Shadow rays of lights on the side of the surface the segment does not see (rt_wavefront.cuh, GO_LIGHTS): skipped (1, default) or traced
+// like the reference (0).  The planes are the same either way; 0 is for A/B runs.
+static std::atomic<bool> g_cullHidden(true);
+void set_cull_hidden_lights(int on) { g_cullHidden.store(on != 0); }
+
 static std::atomic<int> g_sliceCount(-1);   // -1: not yet read from OCLR_SLICES; 0: automatic
 void set_slice_count(int k) { g_sliceCount.store(std::max(0, std::min(k, (int)kMaxSlices))); }
 static int slice_count_for(uint32_t rows, uint32_t width) {
@@ -1952,6 +1957,7 @@ static bool launch_wavefront(Frame* f, const SceneView& S, const FrameView& Fall
     drv.K = K;
     dim3 logicGrid[kMaxSlices];
     int aheadMode[kMaxSlices];
+    const bool cull = g_cullHidden.load();
     for (int k = 0; k < K; ++k) {
         WfSlice& sl = f->slices[k];
         const uint32_t rows = launch_rows(FV[k]);
@@ -2013,7 +2019,7 @@ static bool launch_wavefront(Frame* f, const SceneView& S, const FrameView& Fall
         OCLR_CUDA(cudaEventRecord(f->preReady, st));
         OCLR_CUDA(cudaStreamWaitEvent(f->preStream, f->preReady, 0));
         OCLR_CUDA(cudaMemsetAsync(w.queueCount, 0, sizeof(uint32_t) * kCounterStride, f->preStream));
-        wf_logic_kernel<false><<<logicGrid[0], 128, 0, f->preStream>>>(S, FV[0], w, Fall.sampleBegin, 1u, nullptr, nullptr, aheadMode[0]);
+        wf_logic_kernel<false><<<logicGrid[0], 128, 0, f->preStream>>>(S, FV[0], w, Fall.sampleBegin, 1u, nullptr, nullptr, aheadMode[0], cull);
         OCLR_CUDA(cudaGetLastError());
         OCLR_CUDA(cudaEventRecord(f->preDone, f->preStream));
         f->prelaunched = true;
@@ -2029,9 +2035,9 @@ static bool launch_wavefront(Frame* f, const SceneView& S, const FrameView& Fall
     for (uint32_t s = Fall.sampleBegin; s < Fall.sampleEnd; ++s) {
         const RoundEntry logic = [&](int k, uint32_t r, const WfState& w, const uint32_t* prev, cudaStream_t ks) {
             if (dcnt)
-                wf_logic_kernel<true><<<logicGrid[k], 128, 0, ks>>>(S, FV[k], w, s, r == 0 ? 1u : 0u, prev, dcnt, aheadMode[k]);
+                wf_logic_kernel<true><<<logicGrid[k], 128, 0, ks>>>(S, FV[k], w, s, r == 0 ? 1u : 0u, prev, dcnt, aheadMode[k], false);
             else
-                wf_logic_kernel<false><<<logicGrid[k], 128, 0, ks>>>(S, FV[k], w, s, r == 0 ? 1u : 0u, prev, dcnt, aheadMode[k]);
+                wf_logic_kernel<false><<<logicGrid[k], 128, 0, ks>>>(S, FV[k], w, s, r == 0 ? 1u : 0u, prev, dcnt, aheadMode[k], cull);
         };
         // the first logic round of the request may already be running (or done) on the frame's own stream: frame_prelaunch
         const cudaEvent_t resume = resumePre && s == Fall.sampleBegin ? f->preDone : nullptr;
@@ -2821,6 +2827,7 @@ bool scene_radiance(Scene* s, const Camera* cam, size_t count, const float* orig
     RoundDriver drv = {S, s->device, s->smCount, 0u, dcnt, rays.pinned, nullptr, "radiance query"};
     if (!trace_grid(S, s->smCount, counting, drv.traceGrid, err)) return false;
     const int aheadMode = ahead_mode_for(Q);   // (no camera segments: modes 1 and 2 coincide)
+    const bool cull = g_cullHidden.load();
     uint32_t lastRounds = 4;
     drv.K = 1;
     RoundDomain& d = drv.dom[0];
@@ -2860,9 +2867,9 @@ bool scene_radiance(Scene* s, const Camera* cam, size_t count, const float* orig
                 if (r == 1 && smp == 0)   // the trace of round 0 holds each ray's own closest hit
                     radiance_first_hit_kernel<<<rayGrid, 128, 0, ks>>>(n, w.hit, (uint32_t*)q.firstHit.p);
                 if (dcnt)
-                    wf_logic_kernel<true><<<logicGrid, 128, 0, ks>>>(S, F, w, smp, 0u, prev, dcnt, aheadMode);
+                    wf_logic_kernel<true><<<logicGrid, 128, 0, ks>>>(S, F, w, smp, 0u, prev, dcnt, aheadMode, false);
                 else
-                    wf_logic_kernel<false><<<logicGrid, 128, 0, ks>>>(S, F, w, smp, 0u, prev, dcnt, aheadMode);
+                    wf_logic_kernel<false><<<logicGrid, 128, 0, ks>>>(S, F, w, smp, 0u, prev, dcnt, aheadMode, cull);
             };
             if (!drv.run(nullptr, entry, err)) return false;
         }

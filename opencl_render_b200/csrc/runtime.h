@@ -165,6 +165,8 @@ bool frame_progress(Frame* f, unsigned long long* done, unsigned long long* tota
 void set_slice_count(int k);
 // Tracing one round ahead (rt_wavefront.cuh): 0 never, 1 all segments but the camera's, 2 all, -1 automatic.
 void set_ahead_mode(int m);
+// Skipping the shadow rays of lights on the unseen side of a surface (rt_wavefront.cuh): 1 (default) or 0.  The planes are the same.
+void set_cull_hidden_lights(int on);
 uint32_t band_owned_rows(uint32_t height, uint32_t bandRows, uint32_t rank, uint32_t world);
 // Device -> host copy of ALL rows `rank` owns (bands of bandRows dealt round-robin over world): compacted on the device, one transfer
 // into a pinned staging block, scattered to the caller's (pageable) planes by the calling thread.
