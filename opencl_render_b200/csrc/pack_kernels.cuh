@@ -54,49 +54,61 @@ __global__ void __launch_bounds__(256) pack_triangles_kernel(uint32_t triangleCo
     s[7] = make_float4(u2.x, u2.y, 0.f, 0.f);
 }
 
+// Reference cell id of cell (x, y, z) of the grid being packed, or -1 when it has none.  map == nullptr: the reference grid itself; else a
+// walk grid (rt_types.h): cell j of axis a stands for reference cell map[a * n + j], -1 past the axis' extent (scene_pack.cpp walk_cell_map).
+__device__ __forceinline__ long long grid_ref_id(const int32_t* __restrict__ map, int n, int x, int y, int z) {
+    if ((unsigned)x >= (unsigned)n || (unsigned)y >= (unsigned)n || (unsigned)z >= (unsigned)n) return -1;
+    if (map) {
+        x = __ldg(map + x);
+        y = __ldg(map + n + y);
+        z = __ldg(map + 2 * n + z);
+        if ((x | y | z) < 0) return -1;
+    }
+    return (long long)x + (long long)n * y + (long long)n * n * z;
+}
+
 // Pass 1 over the reference CSR (n^3 + 1 starts): one thread per 4x4x4 brick builds its occupancy mask and counts its
 // non-empty cells.  Pass 2 (after an exclusive scan of the counts) writes {mask, rank base} and the {begin,end} ranges.
 __device__ __forceinline__ uint64_t brick_mask(const uint32_t* __restrict__ start, int n, int nb, uint32_t total, int b, uint32_t* error,
-                                               uint2* ranges /* nullable */, uint32_t* cellIds = nullptr /* linear cell id per non-empty cell */) {
+                                               const int32_t* __restrict__ map, uint2* ranges /* nullable */,
+                                               uint32_t* cellIds = nullptr /* linear cell id (of this grid) per non-empty cell */) {
     const int side = n >= 4 ? 4 : n;
     const int bx = b % nb, by = (b / nb) % nb, bz = b / (nb * nb);
     uint64_t mask = 0;
     int k = 0;
     for (int z = 0; z < side; ++z)
-        for (int y = 0; y < side; ++y) {
-            const size_t row = (size_t)(bx * 4) + (size_t)n * (by * 4 + y) + (size_t)n * n * (bz * 4 + z);
-            uint32_t s = __ldg(start + row);
+        for (int y = 0; y < side; ++y)
             for (int x = 0; x < side; ++x) {
-                const uint32_t e = __ldg(start + row + x + 1);
+                const long long id = grid_ref_id(map, n, bx * 4 + x, by * 4 + y, bz * 4 + z);
+                if (id < 0) continue;
+                const uint32_t s = __ldg(start + id), e = __ldg(start + id + 1);
                 if (e < s || e > total) atomicOr(error, (uint32_t)kPackBadCsr);
                 else if (e - s >= (uint32_t)kMaxCellListLength) atomicOr(error, (uint32_t)kPackListTooLong);
                 if (s < e) {
                     mask |= 1ull << (x | (y << 2) | (z << 4));
                     if (ranges) ranges[k] = make_uint2(s, e);
-                    if (cellIds) cellIds[k] = (uint32_t)(row + x);
+                    if (cellIds) cellIds[k] = (uint32_t)((bx * 4 + x) + (size_t)n * (by * 4 + y) + (size_t)n * n * (bz * 4 + z));
                     ++k;
                 }
-                s = e;
             }
-        }
     return mask;
 }
 
 __global__ void __launch_bounds__(128) brick_count_kernel(const uint32_t* __restrict__ start, int n, int nb, uint32_t total,
-                                                          uint32_t* __restrict__ counts, uint32_t* __restrict__ error) {
+                                                          const int32_t* __restrict__ map, uint32_t* __restrict__ counts, uint32_t* __restrict__ error) {
     const int b = blockIdx.x * blockDim.x + threadIdx.x;
     if (b >= nb * nb * nb) return;
-    counts[b] = (uint32_t)__popcll(brick_mask(start, n, nb, total, b, error, nullptr));
+    counts[b] = (uint32_t)__popcll(brick_mask(start, n, nb, total, b, error, map, nullptr));
 }
 
 __global__ void __launch_bounds__(128) brick_write_kernel(const uint32_t* __restrict__ start, int n, int nb, uint32_t total,
-                                                          const uint32_t* __restrict__ rankBase, uint4* __restrict__ bricks,
+                                                          const int32_t* __restrict__ map, const uint32_t* __restrict__ rankBase, uint4* __restrict__ bricks,
                                                           uint2* __restrict__ cellRange, uint32_t* __restrict__ cellIds,
                                                           uint32_t* __restrict__ error) {
     const int b = blockIdx.x * blockDim.x + threadIdx.x;
     if (b >= nb * nb * nb) return;
     const uint32_t base = rankBase[b];
-    const uint64_t mask = brick_mask(start, n, nb, total, b, error, cellRange + base, cellIds + base);
+    const uint64_t mask = brick_mask(start, n, nb, total, b, error, map, cellRange + base, cellIds + base);
     bricks[b] = make_uint4((uint32_t)mask, (uint32_t)(mask >> 32), mask ? base : 0u, 0u);   // (.z of an empty brick: flags of the three-level walk, rt_walk.h)
 }
 
@@ -113,12 +125,14 @@ __global__ void __launch_bounds__(64) super_brick_kernel(uint4* __restrict__ bri
     if (!any) bricks[b].z = 1u;
 }
 
-// Face masks (rt_types.h): bit e set = list entry e of the cell is absent from the list of the neighbour the walk comes from.
-// One thread per (non-empty cell, face): the work of the face masks sits in the ~10 % of bricks that hold triangles, so it is
-// spread over cells x faces instead of being done by the brick's thread.  Both lists are ascending: one merge pass.
+// Face masks (rt_types.h): bit e set = list entry e of the cell is absent from the list of the neighbour the walk comes from (in the
+// grid being packed: map as in grid_ref_id).  One thread per (non-empty cell, face): the work of the face masks sits in the ~10 % of
+// bricks that hold triangles, so it is spread over cells x faces instead of being done by the brick's thread.  Both lists are
+// ascending: one merge pass.
 __global__ void __launch_bounds__(256) face_mask_kernel(const uint32_t* __restrict__ start, int n, uint32_t total, uint32_t nonEmpty,
-                                                        const uint32_t* __restrict__ cellIds, const uint2* __restrict__ cellRange,
-                                                        const uint32_t* __restrict__ list, uint32_t* __restrict__ faceMask) {
+                                                        const int32_t* __restrict__ map, const uint32_t* __restrict__ cellIds,
+                                                        const uint2* __restrict__ cellRange, const uint32_t* __restrict__ list,
+                                                        uint32_t* __restrict__ faceMask) {
     const uint32_t t = blockIdx.x * blockDim.x + threadIdx.x;
     if (t >= nonEmpty * 6u) return;
     const uint32_t k = t / 6u, face = t - 6u * k;   // face = axis*2 + (entered moving towards +axis)
@@ -126,8 +140,8 @@ __global__ void __launch_bounds__(256) face_mask_kernel(const uint32_t* __restri
     int q[3] = {(int)(id % (uint32_t)n), (int)((id / (uint32_t)n) % (uint32_t)n), (int)(id / ((uint32_t)n * (uint32_t)n))};
     q[face >> 1] += (face & 1) ? -1 : 1;
     uint32_t m = 0xFFFFFFFFu;
-    if (q[face >> 1] >= 0 && q[face >> 1] < n) {
-        const size_t nid = (size_t)q[0] + (size_t)n * q[1] + (size_t)n * n * q[2];
+    const long long nid = grid_ref_id(map, n, q[0], q[1], q[2]);
+    if (nid >= 0) {
         const uint32_t ns = __ldg(start + nid), ne = __ldg(start + nid + 1);
         const uint2 r = cellRange[k];
         if (ns < ne && ne <= total && r.y <= total) {
@@ -141,6 +155,29 @@ __global__ void __launch_bounds__(256) face_mask_kernel(const uint32_t* __restri
         }
     }
     faceMask[t] = m;
+}
+
+// Walk grid (rt_types.h): does run `r` (zero-width cells first .. first + count - 1 of its axis) collapse?  One thread per column across
+// the other two axes compares the lists of the run's cells with the first one's; a difference sets bit 0 of differs[r].  Same rule as
+// scene_pack.cpp walk_run_collapses.  The grid may be the caller's and is not known to be a CSR yet (brick_mask's flag is read later):
+// a cell whose range is not inside the list (end < begin or end > total) counts as a difference, and no entry of it is read.
+__global__ void __launch_bounds__(256) run_check_kernel(const uint32_t* __restrict__ start, const uint32_t* __restrict__ list, int n,
+                                                        uint32_t total, const int3* __restrict__ runs, uint32_t* __restrict__ differs) {
+    const int3 r = runs[blockIdx.y];   // (axis, first, count)
+    const uint32_t col = blockIdx.x * blockDim.x + threadIdx.x;
+    if (col >= (uint32_t)n * (uint32_t)n) return;
+    const size_t stride[3] = {1, (size_t)n, (size_t)n * n};
+    const int u = r.x == 0 ? 1 : 0, v = r.x == 2 ? 1 : 2;
+    const size_t first = (size_t)r.y * stride[r.x] + (size_t)(col % (uint32_t)n) * stride[u] + (size_t)(col / (uint32_t)n) * stride[v];
+    const uint32_t s0 = __ldg(start + first), e0 = __ldg(start + first + 1);
+    bool same = s0 <= e0 && e0 <= total;
+    for (int k = 1; same && k < r.z; ++k) {
+        const size_t id = first + (size_t)k * stride[r.x];
+        const uint32_t s = __ldg(start + id), e = __ldg(start + id + 1);
+        same = s <= e && e <= total && e - s == e0 - s0;
+        for (uint32_t q = 0; same && q < e0 - s0; ++q) same = __ldg(list + s + q) == __ldg(list + s0 + q);
+    }
+    if (!same) atomicOr(differs + blockIdx.y, 1u);
 }
 
 // Vertex indices of every triangle, checked before the device grid builder gathers vertices by them (the packer checks them too,

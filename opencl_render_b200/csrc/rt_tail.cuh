@@ -70,7 +70,7 @@ __global__ void __launch_bounds__(128) wf_tail_kernel(SceneView S, WfState w, Ta
         ray.r = r;
         {   // the end cell, as wf_setup_kernel computed it (raytrace_opencl.c:357-361)
             PackedWalk s;
-            pwalk_setup(s, n, nb, px, py, pz, o, r, minD, maxD);
+            pwalk_setup(s, n, nb, S.walkTrim, px, py, pz, o, r, minD, maxD);
             ray.epk = s.epk;
         }
         ray.c0[0] = pk_get(e.y, 0);
@@ -287,7 +287,7 @@ __global__ void __launch_bounds__(128) wf_tail_brick_kernel(SceneView S, WfState
         uint32_t epk;
         {
             PackedWalk s;
-            pwalk_setup(s, n, nb, px, py, pz, o, r, minD, maxD);
+            pwalk_setup(s, n, nb, S.walkTrim, px, py, pz, o, r, minD, maxD);
             epk = s.epk;
         }
         const uint32_t endBrickPk = epk == (uint32_t)kPkNone ? (uint32_t)kPkNone : ((epk >> 2) & 0x0FF3FCFFu);
@@ -363,7 +363,7 @@ __global__ void __launch_bounds__(128) wf_tail_brick_kernel(SceneView S, WfState
                     int axis, up;
                     float tE;
                     bool crossed;
-                    if (!pwalk_step(g, n, nbShift, shPlanes, axis, up, tE, crossed)) break;   // left the grid (the exit crossing says "finished")
+                    if (!pwalk_step(g, n, S.walkTrim, nbShift, shPlanes, axis, up, tE, crossed)) break;   // left the grid (the exit crossing says "finished")
                     if (crossed) break;                                                          // left the brick: the next slot's business
                     face = axis * 2 + up;
                 }

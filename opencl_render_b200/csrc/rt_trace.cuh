@@ -72,7 +72,8 @@ struct WalkRecords {
 
 // Estimated number of cells between the start cell and the end cell (finite rays) or the cell where the ray leaves the grid.
 // Only used to ORDER the work, never for a result: approximate arithmetic is fine here.
-__device__ __forceinline__ int walk_length_estimate(const PackedWalk& g, int n, const float* px, const float* py, const float* pz) {
+// On a walk grid (trim != 0, SceneView::walkTrim) the exit cell is clamped to the extents like pwalk_setup's cells.
+__device__ __forceinline__ int walk_length_estimate(const PackedWalk& g, int n, uint32_t trim, const float* px, const float* py, const float* pz) {
     int ex, ey, ez;
     if (g.epk != kPkNone) {
         ex = pk_get(g.epk, 0);
@@ -86,6 +87,9 @@ __device__ __forceinline__ int walk_length_estimate(const PackedWalk& g, int n, 
         if (g.r.z != 0.f) t = fminf(t, (bz - g.o.z) / g.r.z);
         if (!(t < OCLR_INF) || t < 0.f) t = 0.f;
         box_address(n, px, py, pz, mk3(g.o.x + t * g.r.x, g.o.y + t * g.r.y, g.o.z + t * g.r.z), ex, ey, ez);
+        ex = pwalk_clamp_cell(ex, n, trim, 0);
+        ey = pwalk_clamp_cell(ey, n, trim, 1);
+        ez = pwalk_clamp_cell(ez, n, trim, 2);
     }
     const int sh = 2 * g.level;   // (level 1: brick coordinates, level 2: super-brick coordinates)
     return abs(ex - (pk_get(g.cpk, 0) << sh)) + abs(ey - (pk_get(g.cpk, 1) << sh)) + abs(ez - (pk_get(g.cpk, 2) << sh));
@@ -103,6 +107,7 @@ __global__ void __launch_bounds__(256) wf_setup_kernel(SceneView S, WfState w, W
     const float* px = shPlanes;
     const float* py = shPlanes + (n + 1);
     const float* pz = shPlanes + 2 * (n + 1);
+    const int span = n - (int)min(S.walkTrim & kPkMask, min((S.walkTrim >> kPkBits) & kPkMask, (S.walkTrim >> (2 * kPkBits)) & kPkMask));
     for (uint32_t base = blockIdx.x * blockDim.x; base < count; base += gridDim.x * blockDim.x) {
         const uint32_t idx = base + threadIdx.x;
         const bool valid = idx < count;
@@ -111,14 +116,15 @@ __global__ void __launch_bounds__(256) wf_setup_kernel(SceneView S, WfState w, W
             const uint32_t path = w.queue[idx];
             const float4 ro = w.rayO[path], rd = w.rayD[path];
             PackedWalk g;
-            pwalk_setup(g, n, S.nb, px, py, pz, mk3(ro.x, ro.y, ro.z), mk3(rd.x, rd.y, rd.z), ro.w, rd.w);
+            pwalk_setup(g, n, S.nb, S.walkTrim, px, py, pz, mk3(ro.x, ro.y, ro.z), mk3(rd.x, rd.y, rd.z), ro.w, rd.w);
             rec.o[idx] = ro;
             rec.d[idx] = rd;
             rec.s0[idx] = make_float4(g.tx, g.ty, g.tz, __uint_as_float(g.cpk));
             rec.s1[idx] = make_uint4(g.epk, w.rayExcl[path], path, g.coarseOk ? 1u : 0u);
-            const int len = walk_length_estimate(g, n, px, py, pz);
-            // classes by quarters of n, longest first (a walk can be up to 3n cells long; 8 classes measured no better than 4)
-            cls = kLengthClasses - 1 - min(kLengthClasses - 1, (len * kLengthClasses) / (n > 0 ? n : 1));
+            const int len = walk_length_estimate(g, n, S.walkTrim, px, py, pz);
+            // classes by quarters of the longest extent (n on the reference grid), longest first (a walk can be up to 3n cells long; 8
+            // classes measured no better than 4)
+            cls = kLengthClasses - 1 - min(kLengthClasses - 1, (len * kLengthClasses) / (span > 0 ? span : 1));
         }
         // one global atomic per CTA, class and iteration (the warps' counts are first summed in shared memory)
         if (threadIdx.x < kLengthClasses) shCount[threadIdx.x] = 0u;
@@ -221,7 +227,9 @@ __device__ __forceinline__ uint32_t next_entry(uint32_t begin, uint32_t end, uin
     return k < end ? k : end;
 }
 
-template <bool COUNT, bool SPLIT, bool HANDOFF = false>
+// WALKGRID: the scene view is a walk grid (rt_types.h, SceneView::walkTrim != 0) and a step's exit test reads the axis' extent; without it
+// the test is the reference grid's `cn >= n >> level`, so a scene that has no walk grid runs the instructions it ran before walk grids.
+template <bool COUNT, bool SPLIT, bool HANDOFF = false, bool WALKGRID = false>
 __global__ void __launch_bounds__(128, OCLR_TRACE_MIN_CTAS) wf_pipe_kernel(SceneView S, WfState w, WalkRecords rec, TraceTuning tune,
                                                                             Counters* gcnt, TailQueue tq) {
     extern __shared__ float shPlanes[];
@@ -291,7 +299,7 @@ __global__ void __launch_bounds__(128, OCLR_TRACE_MIN_CTAS) wf_pipe_kernel(Scene
                     g.o = mk3(P.ray[0][lane], P.ray[1][lane], P.ray[2][lane]);   // (the estimate and the plan below read the ray from the walk state)
                     g.r = mk3(P.ray[3][lane], P.ray[4][lane], P.ray[5][lane]);
 #endif
-                    best = walk_length_estimate(g, n, px, py, pz);
+                    best = walk_length_estimate(g, n, WALKGRID ? S.walkTrim : 0u, px, py, pz);
                 }
 #pragma unroll
                 for (int off = 16; off; off >>= 1) {
@@ -516,9 +524,9 @@ __global__ void __launch_bounds__(128, OCLR_TRACE_MIN_CTAS) wf_pipe_kernel(Scene
 #if OCLR_RAY_IN_SMEM
                     lastAxis = pwalk_step_axis(g, lastE);
                     up = (int)((sgn >> lastAxis) & 1u);
-                    const bool inside = pwalk_step_along(g, n, nbShift, shPlanes, lastAxis, P.ray[lastAxis][lane], P.ray[3 + lastAxis][lane], up, crossed);
+                    const bool inside = pwalk_step_along(g, n, WALKGRID ? S.walkTrim : 0u, nbShift, shPlanes, lastAxis, P.ray[lastAxis][lane], P.ray[3 + lastAxis][lane], up, crossed);
 #else
-                    const bool inside = pwalk_step(g, n, nbShift, shPlanes, lastAxis, up, lastE, crossed);
+                    const bool inside = pwalk_step(g, n, WALKGRID ? S.walkTrim : 0u, nbShift, shPlanes, lastAxis, up, lastE, crossed);
 #endif
                     if (!inside) {
                         ws = kWsFinished;

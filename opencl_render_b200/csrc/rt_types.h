@@ -25,6 +25,16 @@
 //             from cell N into cell C has already examined every triangle of N, so only the masked-in entries of C
 //             can be new to it -- the trace kernel jumps straight to them instead of scanning the whole list.
 //   planes    3 x (n+1) floats (x planes, y planes, z planes) -- copied to shared memory by each CTA.
+//
+// Walk grid.  The reference puts split plane i at a vertex quantile, so a scene whose vertices sit on few distinct heights (config 2:
+// 36 UV spheres, 26 ring heights) repeats planes: 229 of its 256 y layers have zero width, in runs of 8-9.  Where every cell of such a
+// run has the same list as the run's first cell in every column (checked at pack time, scene_pack.cpp walk_cell_map), crossing the run
+// cell by cell only revisits one list.  The production trace stage therefore walks a second grid over the cells it keeps per axis --
+// every positive-width cell, one cell per collapsed run (plus up to 3 duplicates, to make the extent a multiple of 4), every cell of a
+// run that did not collapse -- with its own bricks / cellRange / faceMask / planes and the same cellList; planes past the extent repeat
+// the last one.  The walk's crossing sequence
+// on it is the reference's with runs of equal crossing values shortened, which the tie rule merges in the same order, so it visits the
+// same lists in the same order with repeats dropped: the same first hit.  A scene without a collapsible run walks the reference grid.
 #pragma once
 #include <stdint.h>
 
@@ -111,6 +121,10 @@ struct SceneView {
     uint32_t lightCount;
     int32_t n;                // axesDivCount (power of two)
     int32_t nb;               // bricks per axis = max(n/4, 1)
+    // Extents of the grid the packed walk runs on (rt_walk.h): n minus `walkTrim`'s field of the axis, packed like a cell coordinate
+    // (pk_make).  0 = the reference grid (the default, so that a view built without knowing of walk grids is one); non-zero only in a
+    // walk grid's view (see the top of this file).  Index space, brick addressing and plane stride stay those of n.
+    uint32_t walkTrim = 0;
 };
 
 struct Camera {

@@ -84,7 +84,15 @@ OCLR_HD int pwalk_end_key(uint32_t epk, int nbShift) {
 }
 
 // Ray -> initial walk state: raytrace_opencl.c:350-362 (BindInCube on start and end, GetBoxAddress) + the first three crossing values.
-OCLR_HD void pwalk_setup(PackedWalk& w, int n, int nb, const float* px, const float* py, const float* pz, f3 o, f3 r, float minD,
+// Cell index along `axis` on a grid of n - (trim's field) cells per axis (SceneView::walkTrim).  On a walk grid the planes past its
+// extent repeat its last plane, so a point beyond that plane addresses a padded cell: the grid's last cell stands for it (its list is
+// the list of every reference cell past the last kept plane, a collapsed run).  The reference grid: box_address's own answer.
+OCLR_HD int pwalk_clamp_cell(int c, int n, uint32_t trim, int axis) {
+    const int last = n - 1 - (int)((trim >> (axis * kPkBits)) & kPkMask);
+    return c < last ? c : last;
+}
+
+OCLR_HD void pwalk_setup(PackedWalk& w, int n, int nb, uint32_t trim, const float* px, const float* py, const float* pz, f3 o, f3 r, float minD,
                          float maxD) {
     w.o = o;
     w.r = r;
@@ -94,6 +102,9 @@ OCLR_HD void pwalk_setup(PackedWalk& w, int n, int nb, const float* px, const fl
     bind_in_cube(start, r, lo, hi);
     int cx, cy, cz;
     box_address(n, px, py, pz, start, cx, cy, cz);
+    cx = pwalk_clamp_cell(cx, n, trim, 0);
+    cy = pwalk_clamp_cell(cy, n, trim, 1);
+    cz = pwalk_clamp_cell(cz, n, trim, 2);
     w.cpk = pk_make(cx, cy, cz);
     w.epk = kPkNone;
     w.endBrick = (int)kEndNone;
@@ -102,6 +113,9 @@ OCLR_HD void pwalk_setup(PackedWalk& w, int n, int nb, const float* px, const fl
         bind_in_cube(end, r, lo, hi);
         int ex, ey, ez;
         box_address(n, px, py, pz, end, ex, ey, ez);
+        ex = pwalk_clamp_cell(ex, n, trim, 0);
+        ey = pwalk_clamp_cell(ey, n, trim, 1);
+        ez = pwalk_clamp_cell(ez, n, trim, 2);
         w.epk = pk_make(ex, ey, ez);
         w.endBrick = ((ex >> 2) + nb * ((ey >> 2) + nb * (ez >> 2))) | (pwalk_bit(w.epk) << kEndBitShift);
     }
@@ -150,15 +164,17 @@ OCLR_HD int pwalk_step_axis(const PackedWalk& w, float& tEvent) {
     return xmin ? 0 : (ymin ? 1 : 2);
 }
 // Second half: the step along `axis` (oo, rr = origin / direction component of that axis, up = (0 <= rr)).  Returns false when the walk
-// left the grid; `crossed` is set when the step entered another brick (always above level 0).
-OCLR_HD bool pwalk_step_along(PackedWalk& w, int n, int nbShift, const float* planes, int axis, float oo, float rr, int up, bool& crossed) {
+// left the grid -- n - (trim's field of the axis) cells, SceneView::walkTrim; a multiple of 4 whenever the brick level runs;
+// `crossed` is set when the step entered another brick (always above level 0).
+OCLR_HD bool pwalk_step_along(PackedWalk& w, int n, uint32_t trim, int nbShift, const float* planes, int axis, float oo, float rr, int up,
+                              bool& crossed) {
     const int sh = axis * kPkBits;
     const int c = (int)((w.cpk >> sh) & kPkMask);
     const int dir = up ? 1 : -1;
     const int cn = c + dir;
     const int lsh = 2 * w.level;
     crossed = false;
-    if ((uint32_t)cn >= (uint32_t)(n >> lsh)) return false;
+    if ((uint32_t)cn >= (uint32_t)((n - (int)((trim >> sh) & kPkMask)) >> lsh)) return false;
     const float t = (planes[axis * (n + 1) + ((cn + up) << lsh)] - oo) / rr;
     w.cpk += (uint32_t)dir << sh;   // two's complement: -1 << sh subtracts one from the axis' field
     w.tx = axis == 0 ? t : w.tx;
@@ -169,12 +185,12 @@ OCLR_HD bool pwalk_step_along(PackedWalk& w, int n, int nbShift, const float* pl
     return true;
 }
 // Both halves, the ray taken from the walk state.  `axis`, `up` and `tEvent` describe the crossing taken.
-OCLR_HD bool pwalk_step(PackedWalk& w, int n, int nbShift, const float* planes, int& axis, int& up, float& tEvent, bool& crossed) {
+OCLR_HD bool pwalk_step(PackedWalk& w, int n, uint32_t trim, int nbShift, const float* planes, int& axis, int& up, float& tEvent, bool& crossed) {
     axis = pwalk_step_axis(w, tEvent);
     const float rr = axis == 0 ? w.r.x : (axis == 1 ? w.r.y : w.r.z);
     const float oo = axis == 0 ? w.o.x : (axis == 1 ? w.o.y : w.o.z);
     up = (0 <= rr) ? 1 : 0;
-    return pwalk_step_along(w, n, nbShift, planes, axis, oo, rr, up, crossed);
+    return pwalk_step_along(w, n, trim, nbShift, planes, axis, oo, rr, up, crossed);
 }
 
 // After a successful step along `axis`: did the walk just cross into the cell index at which this part ends?
@@ -449,7 +465,7 @@ OCLR_HD uint32_t grid_walk_packed(const SceneView& S, const float* planes, Packe
         bool crossed;
         if (COUNT && w.level) cnt->coarseSteps++;
         if (COUNT && w.level == 2) cnt->superSteps++;
-        if (!pwalk_step(w, n, nbShift, planes, lastAxis, up, lastE, crossed)) break;
+        if (!pwalk_step(w, n, S.walkTrim, nbShift, planes, lastAxis, up, lastE, crossed)) break;
         if (pwalk_stopped(w, lastAxis, up)) break;   // this part of the walk ends here; the cell belongs to the next part
         face = w.level ? (int)kFaceNone : lastAxis * 2 + up;
         if (crossed) {
@@ -466,7 +482,7 @@ OCLR_HD uint32_t grid_trace_packed(const SceneView& S, const float* planes, f3 o
                                    float& outT, float& outAB, float& outAC, Counters* cnt) {
     const int n = S.n;
     PackedWalk w;
-    pwalk_setup(w, n, S.nb, planes, planes + (n + 1), planes + 2 * (n + 1), o, r, minD, maxD);
+    pwalk_setup(w, n, S.nb, S.walkTrim, planes, planes + (n + 1), planes + 2 * (n + 1), o, r, minD, maxD);
     if (COUNT) cnt->gridRays++;
     return grid_walk_packed<COUNT>(S, planes, w, minD, maxD, excl, outT, outAB, outAC, cnt);
 }
@@ -492,7 +508,7 @@ OCLR_HD uint32_t grid_trace_split(const SceneView& S, const float* planes, f3 o,
     const float* py = planes + (n + 1);
     const float* pz = planes + 2 * (n + 1);
     PackedWalk first;
-    pwalk_setup(first, n, S.nb, px, py, pz, o, r, minD, maxD);
+    pwalk_setup(first, n, S.nb, S.walkTrim, px, py, pz, o, r, minD, maxD);
     if (COUNT) cnt->gridRays++;
     const bool splittable = (n >= 4) & (r.x != 0.f) & (r.y != 0.f) & (r.z != 0.f);
     if (!splittable) return grid_walk_packed<COUNT>(S, planes, first, minD, maxD, excl, outT, outAB, outAC, cnt);
@@ -596,7 +612,7 @@ OCLR_HD uint32_t grid_trace_split_mid(const SceneView& S, const float* planes, f
     const float* py = planes + (n + 1);
     const float* pz = planes + 2 * (n + 1);
     PackedWalk first;
-    pwalk_setup(first, n, S.nb, px, py, pz, o, r, minD, maxD);
+    pwalk_setup(first, n, S.nb, S.walkTrim, px, py, pz, o, r, minD, maxD);
     if (COUNT) cnt->gridRays++;
     WalkPause pause;
     uint32_t hit = grid_walk_packed<COUNT>(S, planes, first, minD, maxD, excl, outT, outAB, outAC, cnt, walkFirst, &pause);
@@ -728,7 +744,7 @@ OCLR_HD uint32_t grid_trace_coop(const SceneView& S, const float* planes, f3 o, 
                                  float& outAB, float& outAC, Counters* cnt) {
     const int n = S.n;
     PackedWalk w;
-    pwalk_setup(w, n, S.nb, planes, planes + (n + 1), planes + 2 * (n + 1), o, r, minD, maxD);
+    pwalk_setup(w, n, S.nb, S.walkTrim, planes, planes + (n + 1), planes + 2 * (n + 1), o, r, minD, maxD);
     if (!w.coarseOk) return grid_trace_packed<COUNT>(S, planes, o, r, minD, maxD, excl, outT, outAB, outAC, cnt);
     if (COUNT) cnt->gridRays++;
     auto test_cell = [&](uint32_t cpk, int face, uint32_t& closest) {
@@ -802,7 +818,7 @@ OCLR_HD uint32_t grid_trace_coop_bricks(const SceneView& S, const float* planes,
     const float* py = planes + (n + 1);
     const float* pz = planes + 2 * (n + 1);
     PackedWalk start;
-    pwalk_setup(start, n, nb, px, py, pz, o, r, minD, maxD);
+    pwalk_setup(start, n, nb, S.walkTrim, px, py, pz, o, r, minD, maxD);
     if (!start.coarseOk) return grid_trace_packed<COUNT>(S, planes, o, r, minD, maxD, excl, outT, outAB, outAC, cnt);
     if (COUNT) cnt->gridRays++;
     int nbShift = 0;
@@ -849,7 +865,7 @@ OCLR_HD uint32_t grid_trace_coop_bricks(const SceneView& S, const float* planes,
             int axis, upA;
             float tE;
             bool crossed;
-            if (!pwalk_step(g, n, nbShift, planes, axis, upA, tE, crossed)) return;
+            if (!pwalk_step(g, n, S.walkTrim, nbShift, planes, axis, upA, tE, crossed)) return;
             if (crossed) return;
             face = axis * 2 + upA;
         }

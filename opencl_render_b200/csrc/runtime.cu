@@ -651,7 +651,11 @@ bool run_on_devices(int world, bool shareUpload, const std::function<void(int ra
 struct Scene {
     int device = 0;
     DeviceBuffer triGeo, triShade, bricks, cellRange, cellList, faceMask, planes, matSize, matStart, textures, lights;
+    // the walk grid (rt_types.h), when a run of coincident planes collapses; else empty and walkView == view
+    DeviceBuffer walkBricks, walkCellRange, walkFaceMask, walkPlanes;
+    uint32_t walkTrim = 0;
     SceneView view = {};
+    SceneView walkView = {};   // what the production trace stage walks (enqueue_trace)
     size_t bytes = 0;
     int smCount = 148;
     // Ring slots a path of this scene can occupy (rt_wavefront.cuh): only mirror / glass segments (raytrace_opencl.c:682-722) push the
@@ -661,8 +665,9 @@ struct Scene {
     int ringSlots = kRingSize;
     bool hasBump = false;   // some material has a BUMP channel: its normals read the camera vectors (radiance queries need a camera)
     uint64_t geometryGen = 0;   // geometry edits so far (scene_update): camera lists built for an older generation are stale
-    std::array<DeviceBuffer*, 11> buffers() {
-        return {&triGeo, &triShade, &bricks, &cellRange, &cellList, &faceMask, &planes, &matSize, &matStart, &textures, &lights};
+    std::array<DeviceBuffer*, 15> buffers() {
+        return {&triGeo, &triShade, &bricks, &cellRange, &cellList, &faceMask, &planes, &matSize, &matStart, &textures, &lights,
+                &walkBricks, &walkCellRange, &walkFaceMask, &walkPlanes};
     }
 };
 
@@ -1103,8 +1108,17 @@ static void bind_view(Scene* s, uint32_t triangleCount, uint32_t materialCount, 
     v.lightCount = lightCount;
     v.n = n;
     v.nb = n >= 4 ? n / 4 : 1;
-    s->bytes = s->triGeo.bytes + s->triShade.bytes + s->bricks.bytes + s->cellRange.bytes + s->cellList.bytes + s->faceMask.bytes + s->planes.bytes +
-               s->matSize.bytes + s->matStart.bytes + s->textures.bytes + s->lights.bytes;
+    s->walkView = v;
+    if (s->walkTrim) {
+        SceneView& w = s->walkView;
+        w.bricks = (const uint4*)s->walkBricks.p;
+        w.cellRange = (const uint2*)s->walkCellRange.p;
+        w.faceMask = (const uint32_t*)s->walkFaceMask.p;
+        w.planes = (const float*)s->walkPlanes.p;
+        w.walkTrim = s->walkTrim;
+    }
+    s->bytes = 0;
+    for (DeviceBuffer* b : s->buffers()) s->bytes += b->bytes;
 }
 
 // Triangles: raw reference arrays in device memory -> d->triGeo / d->triShade (pack_triangles_kernel; bad indices and material ids are
@@ -1118,22 +1132,68 @@ static bool pack_stage(Scene* d, uint32_t N, uint32_t V, uint32_t materialCount,
     return true;
 }
 
-// The grid: given in device memory (boxMin, gridStart and `total` list entries already in d->cellList), or built on the device at n cells
-// per axis when gridStart is null; repacked into d->bricks / cellRange / faceMask / planes.  Enqueued on the default stream (the
-// builder and the non-empty cell count synchronise it); problems found on the device are or-ed into error[0], which error[1] must
-// be free to use.
-static bool grid_stage(Scene* d, int n, uint32_t V, const float4* vertex, uint32_t N, const int4* triIdx, const float4* boxMin,
-                       const uint32_t* gridStart, uint32_t total, uint32_t* error, std::string& err) {
+// Bricks, ranges and face masks of one grid over the reference CSR -- the reference grid (map == nullptr) or a walk grid (map: see
+// pack_kernels.cuh grid_ref_id) -- into bricks / cellRange / faceMask, behind `nSuper` zeroed super-brick records.  Synchronises the
+// default stream once (the non-empty cell count sizes the ranges).
+static bool pack_cells_on_device(int n, const uint32_t* gridStart, uint32_t total, const uint32_t* list, const int32_t* map, size_t nSuper,
+                                 DeviceBuffer& bricks, DeviceBuffer& cellRange, DeviceBuffer& faceMask, uint32_t* error, std::string& err) {
     const int nb = n >= 4 ? n / 4 : 1;
     const size_t nBricks = (size_t)nb * nb * nb;
+    DeviceBuffer counts, rankBase, scanTmp, cellIds;
+    auto done = [&](bool ok) {
+        for (DeviceBuffer* b : {&counts, &rankBase, &scanTmp, &cellIds}) b->release();
+        return ok;
+    };
+    if (!bricks.alloc(sizeof(uint4) * (nBricks + nSuper), err) || !counts.alloc(sizeof(uint32_t) * (nBricks + 1), err) ||
+        !rankBase.alloc(sizeof(uint32_t) * (nBricks + 1), err))
+        return done(false);
+    cudaMemsetAsync(counts.p, 0, sizeof(uint32_t) * (nBricks + 1), 0);
+    brick_count_kernel<<<(unsigned)((nBricks + 127) / 128), 128>>>(gridStart, n, nb, total, map, (uint32_t*)counts.p, error);
+    size_t tmpBytes = 0;
+    cub::DeviceScan::ExclusiveSum(nullptr, tmpBytes, (const uint32_t*)counts.p, (uint32_t*)rankBase.p, (int)(nBricks + 1));
+    if (!scanTmp.alloc(tmpBytes, err)) return done(false);
+    cub::DeviceScan::ExclusiveSum(scanTmp.p, tmpBytes, (const uint32_t*)counts.p, (uint32_t*)rankBase.p, (int)(nBricks + 1));
+    uint32_t nonEmpty = 0;
+    cudaMemcpyAsync(&nonEmpty, (const uint32_t*)rankBase.p + nBricks, sizeof(uint32_t), cudaMemcpyDeviceToHost, 0);
+    cudaError_t e = cudaStreamSynchronize(0);
+    if (e != cudaSuccess) {
+        err = std::string("scene repack: ") + cudaGetErrorString(e);
+        return done(false);
+    }
+    if (nonEmpty >= (1u << 29)) {
+        err = "too many non-empty grid cells (>= 2^29)";
+        return done(false);
+    }
+    const size_t ne = nonEmpty ? nonEmpty : 1;
+    if (!cellRange.alloc(sizeof(uint2) * ne, err) || !faceMask.alloc(sizeof(uint32_t) * 6 * ne, err) || !cellIds.alloc(sizeof(uint32_t) * ne, err))
+        return done(false);
+    brick_write_kernel<<<(unsigned)((nBricks + 127) / 128), 128>>>(gridStart, n, nb, total, map, (const uint32_t*)rankBase.p, (uint4*)bricks.p,
+                                                                  (uint2*)cellRange.p, (uint32_t*)cellIds.p, error);
+    if (nonEmpty)
+        face_mask_kernel<<<(unsigned)(((size_t)nonEmpty * 6 + 255) / 256), 256>>>(gridStart, n, total, nonEmpty, map, (const uint32_t*)cellIds.p,
+                                                                                 (const uint2*)cellRange.p, list, (uint32_t*)faceMask.p);
+    else
+        cudaMemsetAsync(faceMask.p, 0xFF, sizeof(uint32_t) * 6, 0);
+    return done(true);   // (the temporaries are freed in stream order behind the kernels that read them)
+}
+
+// The grid: given in device memory (boxMin, gridStart and `total` list entries already in d->cellList), or built on the device at n cells
+// per axis when gridStart is null; repacked into d->bricks / cellRange / faceMask / planes, and into the walk grid (rt_types.h) when
+// a run of coincident planes collapses: the runs are found on the host from the planes, checked on the device (the grid may be the
+// caller's), and the walk grid is packed on the device from the cell map of scene_pack.cpp walk_cell_map.  Enqueued on the default
+// stream (the builder and the non-empty cell counts synchronise it); problems found on the device are or-ed into error[0], which
+// error[1] must be free to use.
+static bool grid_stage(Scene* d, int n, uint32_t V, const float4* vertex, uint32_t N, const int4* triIdx, const float4* boxMin,
+                       const uint32_t* gridStart, uint32_t total, uint32_t* error, std::string& err) {
     // super-brick records of the three-level walk follow the brick records (rt_walk.h) -- in builds whose trace kernel has that level
     const int superPolicy = OCLR_SUPER_LEVEL ? super_policy(1) : 0;
+    const int nb = n >= 4 ? n / 4 : 1;
     const int ns = superPolicy > 0 ? super_bricks_per_axis(n) : 0;
     const size_t nSuper = superPolicy > 0 ? super_brick_records(n) : 0;
     DeviceGrid grid;
-    DeviceBuffer counts, rankBase, scanTmp, cellIds;
+    DeviceBuffer runsDev, differs, mapDev;
     auto done = [&](bool ok) {
-        for (DeviceBuffer* b : {&counts, &rankBase, &scanTmp, &cellIds, &grid.boxMin, &grid.start}) b->release();
+        for (DeviceBuffer* b : {&grid.boxMin, &grid.start, &runsDev, &differs, &mapDev}) b->release();
         return ok;
     };
     if (!gridStart) {
@@ -1153,44 +1213,54 @@ static bool grid_stage(Scene* d, int n, uint32_t V, const float4* vertex, uint32
         gridStart = (const uint32_t*)grid.start.p;
         total = grid.total;
     }
-    if (!d->bricks.alloc(sizeof(uint4) * (nBricks + nSuper), err) || !d->planes.alloc(sizeof(float) * 3 * (n + 1), err) ||
-        !counts.alloc(sizeof(uint32_t) * (nBricks + 1), err) || !rankBase.alloc(sizeof(uint32_t) * (nBricks + 1), err))
-        return done(false);
-    cudaMemsetAsync(counts.p, 0, sizeof(uint32_t) * (nBricks + 1), 0);
+    if (!d->planes.alloc(sizeof(float) * 3 * (n + 1), err)) return done(false);
     split_planes_kernel<<<(n + 1 + 127) / 128, 128>>>(boxMin, n, (float*)d->planes.p);
-    brick_count_kernel<<<(unsigned)((nBricks + 127) / 128), 128>>>(gridStart, n, nb, total, (uint32_t*)counts.p, error);
-    size_t tmpBytes = 0;
-    cub::DeviceScan::ExclusiveSum(nullptr, tmpBytes, (const uint32_t*)counts.p, (uint32_t*)rankBase.p, (int)(nBricks + 1));
-    if (!scanTmp.alloc(tmpBytes, err)) return done(false);
-    cub::DeviceScan::ExclusiveSum(scanTmp.p, tmpBytes, (const uint32_t*)counts.p, (uint32_t*)rankBase.p, (int)(nBricks + 1));
     if (total) check_list_kernel<<<(total + 255) / 256, 256>>>((const uint32_t*)d->cellList.p, total, N, error);
-    uint32_t nonEmpty = 0;
-    cudaMemcpyAsync(&nonEmpty, (const uint32_t*)rankBase.p + nBricks, sizeof(uint32_t), cudaMemcpyDeviceToHost, 0);
+    std::vector<float> planes(3 * (size_t)(n + 1));
+    cudaMemcpyAsync(planes.data(), d->planes.p, sizeof(float) * planes.size(), cudaMemcpyDeviceToHost, 0);   // (read after the next sync)
+    if (!pack_cells_on_device(n, gridStart, total, (const uint32_t*)d->cellList.p, nullptr, nSuper, d->bricks, d->cellRange, d->faceMask,
+                              error, err))
+        return done(false);
+    if (nSuper) {
+        cudaMemsetAsync((uint4*)d->bricks.p + (size_t)nb * nb * nb, 0, sizeof(uint4) * nSuper, 0);
+        super_brick_kernel<<<(unsigned)(ns * ns * ns), 64>>>((uint4*)d->bricks.p, nb, ns);
+    }
+    // the walk grid
+    for (DeviceBuffer* b : {&d->walkBricks, &d->walkCellRange, &d->walkFaceMask, &d->walkPlanes}) b->release();
+    d->walkTrim = 0;
+    const std::vector<WalkRun> runs = walk_runs(planes.data(), n);
+    if (runs.empty()) return done(true);
+    std::vector<int3> runs3(runs.size());
+    for (size_t i = 0; i < runs.size(); ++i) runs3[i] = make_int3(runs[i].axis, runs[i].first, runs[i].count);
+    if (!runsDev.upload(runs3.data(), sizeof(int3) * runs3.size(), err) || !differs.alloc(sizeof(uint32_t) * runs.size(), err)) return done(false);
+    cudaMemsetAsync(differs.p, 0, sizeof(uint32_t) * runs.size(), 0);
+    run_check_kernel<<<dim3((unsigned)(((size_t)n * n + 255) / 256), (unsigned)runs.size()), 256>>>(
+        gridStart, (const uint32_t*)d->cellList.p, n, total, (const int3*)runsDev.p, (uint32_t*)differs.p);
+    std::vector<uint32_t> differ(runs.size());
+    cudaMemcpyAsync(differ.data(), differs.p, sizeof(uint32_t) * runs.size(), cudaMemcpyDeviceToHost, 0);
+    uint32_t packErrors = 0;   // a grid the packers flagged (bad CSR, ...) is refused by the caller: no walk grid is built over it
+    cudaMemcpyAsync(&packErrors, error, sizeof(uint32_t), cudaMemcpyDeviceToHost, 0);
     cudaError_t e = cudaStreamSynchronize(0);
     if (e != cudaSuccess) {
         err = std::string("scene repack: ") + cudaGetErrorString(e);
         return done(false);
     }
-    if (nonEmpty >= (1u << 29)) {
-        err = "too many non-empty grid cells (>= 2^29)";
+    if (packErrors) return done(true);
+    std::vector<uint8_t> collapses(runs.size());
+    bool any = false;
+    for (size_t i = 0; i < runs.size(); ++i) any |= (collapses[i] = differ[i] ? 0 : 1) != 0;
+    if (!any) return done(true);
+    std::vector<int32_t> map;
+    const uint32_t trim = walk_cell_map(n, runs, collapses, map);
+    if (!trim) return done(true);   // the padding kept every cell again
+    std::vector<float> wplanes(planes.size());
+    walk_planes(planes.data(), n, map.data(), wplanes.data());
+    if (!mapDev.upload(map.data(), sizeof(int32_t) * map.size(), err) || !d->walkPlanes.upload(wplanes.data(), sizeof(float) * wplanes.size(), err) ||
+        !pack_cells_on_device(n, gridStart, total, (const uint32_t*)d->cellList.p, (const int32_t*)mapDev.p, 0, d->walkBricks, d->walkCellRange,
+                              d->walkFaceMask, error, err))
         return done(false);
-    }
-    const size_t ne = nonEmpty ? nonEmpty : 1;
-    if (!d->cellRange.alloc(sizeof(uint2) * ne, err) || !d->faceMask.alloc(sizeof(uint32_t) * 6 * ne, err) || !cellIds.alloc(sizeof(uint32_t) * ne, err))
-        return done(false);
-    brick_write_kernel<<<(unsigned)((nBricks + 127) / 128), 128>>>(gridStart, n, nb, total, (const uint32_t*)rankBase.p, (uint4*)d->bricks.p,
-                                                                  (uint2*)d->cellRange.p, (uint32_t*)cellIds.p, error);
-    if (nSuper) {
-        cudaMemsetAsync((uint4*)d->bricks.p + nBricks, 0, sizeof(uint4) * nSuper, 0);
-        super_brick_kernel<<<(unsigned)(ns * ns * ns), 64>>>((uint4*)d->bricks.p, nb, ns);
-    }
-    if (nonEmpty)
-        face_mask_kernel<<<(unsigned)(((size_t)nonEmpty * 6 + 255) / 256), 256>>>(gridStart, n, total, nonEmpty, (const uint32_t*)cellIds.p,
-                                                                                 (const uint2*)d->cellRange.p, (const uint32_t*)d->cellList.p,
-                                                                                 (uint32_t*)d->faceMask.p);
-    else
-        cudaMemsetAsync(d->faceMask.p, 0xFF, sizeof(uint32_t) * 6, 0);
-    return done(true);   // (the temporaries are freed in stream order behind the kernels that read them)
+    d->walkTrim = trim;
+    return done(true);
 }
 
 static bool scene_upload(Scene* s, const HostScene& h, std::string& err, const std::function<void(Scene*)>* early, UploadShare* share) {
@@ -1343,10 +1413,18 @@ size_t frame_state_bytes(Frame* f) {
     return n;
 }
 
-// Debug/test door: copies one packed device array back (0 triGeo, 1 triShade, 2 bricks, 3 cellRange, 4 planes, 5 cellList).
+// Debug/test door: copies one packed device array back (0 triGeo, 1 triShade, 2 bricks, 3 cellRange, 4 planes, 5 cellList, 6 faceMask;
+// the walk grid: 7 bricks, 8 cellRange, 9 faceMask, 10 planes -- empty when the scene walks the reference grid -- and 11 its extents,
+// three uint32).
 size_t scene_debug_read(Scene* s, int which, void* dst, size_t cap) {
-    DeviceBuffer* all[] = {&s->triGeo, &s->triShade, &s->bricks, &s->cellRange, &s->planes, &s->cellList, &s->faceMask};
-    if (which < 0 || which > 6) return 0;
+    DeviceBuffer* all[] = {&s->triGeo, &s->triShade, &s->bricks, &s->cellRange, &s->planes, &s->cellList, &s->faceMask,
+                           &s->walkBricks, &s->walkCellRange, &s->walkFaceMask, &s->walkPlanes};
+    if (which == 11) {
+        const uint32_t ext[3] = {s->view.n - ((s->walkTrim) & 1023u), s->view.n - ((s->walkTrim >> 10) & 1023u), s->view.n - ((s->walkTrim >> 20) & 1023u)};
+        if (dst && cap >= sizeof(ext)) memcpy(dst, ext, sizeof(ext));
+        return sizeof(ext);
+    }
+    if (which < 0 || which > 10) return 0;
     cudaSetDevice(s->device);
     const size_t n = all[which]->bytes;
     if (dst && n && n <= cap) cudaMemcpy(dst, all[which]->p, n, cudaMemcpyDeviceToHost);
@@ -1722,27 +1800,33 @@ static bool trace_grid(const SceneView& S, int smCount, bool counting, unsigned&
 
 // Enqueues one round of the trace stage on `ks`: walk records of the rays queued in w (wf_setup_kernel), the trace (wf_pipe_kernel,
 // instantiation chosen from the tuning), and the hand-off of its tail when `tq` has room (tq.capacity != 0).  Every kernel reads the ray
-// count from device memory, so a round with nothing queued costs only its launches.
-static void enqueue_trace(const SceneView& S, const WfState& w, const WalkRecords& rec, const TailQueue& tq, unsigned setupGrid, unsigned traceGrid,
-                          int smCount, Counters* dcnt, cudaStream_t ks, uint32_t& launches) {
+// count from device memory, so a round with nothing queued costs only its launches.  The production instantiations walk `walkGrid`
+// (Scene::walkView); the off-by-default experiments -- run-time split, tail hand-off, super-brick level -- the reference grid `S`.
+static void enqueue_trace(const SceneView& reference, const SceneView& walkGrid, const WfState& w, const WalkRecords& rec, const TailQueue& tq,
+                          unsigned setupGrid, unsigned traceGrid, int smCount, Counters* dcnt, cudaStream_t ks, uint32_t& launches) {
     const TraceTuning& tune = trace_tuning();
-    const size_t shBytes = sizeof(float) * 3 * (S.n + 1);
-    wf_setup_kernel<<<setupGrid, 256, shBytes, ks>>>(S, w, rec);
-    ++launches;
     // (the run-time split of long walks is an instantiation of its own: compiled into the production kernel it cost
     // 10 % through register pressure even when switched off)
     // (so is the hand-off of the tail to wf_tail_kernel: only the launches of small domains run that instantiation)
     const bool handoff = tq.capacity != 0 && tune.splitMin <= 0;
+    const SceneView& S = (OCLR_SUPER_LEVEL || tune.splitMin > 0 || handoff) ? reference : walkGrid;
+    const size_t shBytes = sizeof(float) * 3 * (S.n + 1);
+    wf_setup_kernel<<<setupGrid, 256, shBytes, ks>>>(S, w, rec);
+    ++launches;
     if (dcnt && tune.splitMin > 0)
         wf_pipe_kernel<true, true><<<traceGrid, 128, shBytes, ks>>>(S, w, rec, tune, dcnt, tq);
     else if (dcnt && handoff)
         wf_pipe_kernel<true, false, true><<<traceGrid, 128, shBytes, ks>>>(S, w, rec, tune, dcnt, tq);
+    else if (dcnt && S.walkTrim)
+        wf_pipe_kernel<true, false, false, true><<<traceGrid, 128, shBytes, ks>>>(S, w, rec, tune, dcnt, tq);
     else if (dcnt)
         wf_pipe_kernel<true, false><<<traceGrid, 128, shBytes, ks>>>(S, w, rec, tune, dcnt, tq);
     else if (tune.splitMin > 0)
         wf_pipe_kernel<false, true><<<traceGrid, 128, shBytes, ks>>>(S, w, rec, tune, dcnt, tq);
     else if (handoff)
         wf_pipe_kernel<false, false, true><<<traceGrid, 128, shBytes, ks>>>(S, w, rec, tune, dcnt, tq);
+    else if (S.walkTrim)
+        wf_pipe_kernel<false, false, false, true><<<traceGrid, 128, shBytes, ks>>>(S, w, rec, tune, dcnt, tq);
     else
         wf_pipe_kernel<false, false><<<traceGrid, 128, shBytes, ks>>>(S, w, rec, tune, dcnt, tq);
     if (handoff && tune.handoffMode == 2) {   // second pass: the same kernel over the rays given up, as their own little queue
@@ -1791,6 +1875,7 @@ struct RoundDomain {
 using RoundEntry = std::function<void(int k, uint32_t r, const WfState& w, const uint32_t* prev, cudaStream_t ks)>;
 struct RoundDriver {
     const SceneView& S;
+    const SceneView& walkS;   // the grid the production trace stage walks (Scene::walkView)
     int device, smCount;
     unsigned traceGrid;
     Counters* dcnt;
@@ -1850,7 +1935,7 @@ bool RoundDriver::run(cudaEvent_t resume, const RoundEntry& entry, std::string& 
                     }
                     OCLR_CUDA(cudaEventRecord((*d.traceEvents)[*d.traceEventsUsed], d.st));
                 }
-                enqueue_trace(S, d.w, d.rec, d.tail, setupGrid[k], traceGrid, smCount, dcnt, d.st, launches);
+                enqueue_trace(S, walkS, d.w, d.rec, d.tail, setupGrid[k], traceGrid, smCount, dcnt, d.st, launches);
                 if (d.traceEvents) {
                     OCLR_CUDA(cudaEventRecord((*d.traceEvents)[*d.traceEventsUsed + 1], d.st));
                     *d.traceEventsUsed += 2;
@@ -1953,7 +2038,7 @@ static bool launch_wavefront(Frame* f, const SceneView& S, const FrameView& Fall
     }
     if (prelaunchOnly && K != 1) return true;   // (only the one-slice case is started ahead)
 
-    RoundDriver drv = {S, f->device, smCount, 0u, dcnt, nullptr, Fall.camBad, "wavefront"};
+    RoundDriver drv = {S, f->scene->walkView, f->device, smCount, 0u, dcnt, nullptr, Fall.camBad, "wavefront"};
     drv.K = K;
     dim3 logicGrid[kMaxSlices];
     int aheadMode[kMaxSlices];
@@ -2747,7 +2832,7 @@ static bool scene_query(Scene* s, bool transmit, size_t count, const float* orig
                 rec.classCount = w.queueCount + 2;
                 const TailQueue tq = {nullptr, w.queueCount + 2 + kLengthClasses, w.queueCount + 6 + kLengthClasses, 0u,
                                       nullptr, nullptr, nullptr, nullptr, nullptr};
-                enqueue_trace(S, w, rec, tq, setupGrid, traceGrid, s->smCount, dcnt, st, launches);
+                enqueue_trace(S, s->walkView, w, rec, tq, setupGrid, traceGrid, s->smCount, dcnt, st, launches);
                 ++rounds;
                 if (!transmit) break;
                 WfState next = w;
@@ -2824,7 +2909,7 @@ bool scene_radiance(Scene* s, const Camera* cam, size_t count, const float* orig
         return false;
     }
     Counters* dcnt = rays.dcnt;
-    RoundDriver drv = {S, s->device, s->smCount, 0u, dcnt, rays.pinned, nullptr, "radiance query"};
+    RoundDriver drv = {S, s->walkView, s->device, s->smCount, 0u, dcnt, rays.pinned, nullptr, "radiance query"};
     if (!trace_grid(S, s->smCount, counting, drv.traceGrid, err)) return false;
     const int aheadMode = ahead_mode_for(Q);   // (no camera segments: modes 1 and 2 coincide)
     const bool cull = g_cullHidden.load();
@@ -3070,8 +3155,9 @@ bool scene_update(Scene* s, const HostScene& h, unsigned parts, bool deviceMemor
     }
     if (geometry) {
         for (DeviceBuffer Scene::*b : {&Scene::triGeo, &Scene::triShade, &Scene::bricks, &Scene::cellRange, &Scene::cellList, &Scene::faceMask,
-                                       &Scene::planes})
+                                       &Scene::planes, &Scene::walkBricks, &Scene::walkCellRange, &Scene::walkFaceMask, &Scene::walkPlanes})
             std::swap(s->*b, t.*b);
+        s->walkTrim = t.walkTrim;
         ++s->geometryGen;
     }
     bind_view(s, geometry ? v.triangleCount : s->view.triangleCount, M, lights ? v.lightCount : s->view.lightCount, n);

@@ -49,9 +49,26 @@ struct PackedGrid {
     std::vector<uint32_t> faceMask;
     std::vector<float> planes;
     int32_t n = 0, nb = 0;
+    // a walk grid (rt_types.h) only: walk cell j of axis a stands for reference cell cellMap[a * n + j] (-1 past the extent);
+    // cells each axis has fewer than n (SceneView::walkTrim).  cellList stays empty: the ranges point into the reference's list.
+    std::vector<int32_t> cellMap;
+    uint32_t walkTrim = 0;
 };
 void pack_triangles(const HostScene& h, float4* triGeo /*4N*/, float4* triShade /*8N*/, int threads);
 bool pack_grid(const HostScene& h, PackedGrid& out, std::string& err);
+// Walk grid (rt_types.h) of a scene and its packed reference grid `ref`; walk.n == 0 when no run collapses or the padding to a multiple of
+// 4 keeps every cell again (the walk runs on `ref`).
+// The device builds it from the same pieces: walk_runs and walk_cell_map on the host, the run check and the packing on the device.
+struct WalkRun {
+    int axis, first, count;   // zero-width cells first .. first + count - 1 of `axis` (count >= 2): count + 1 equal planes
+};
+std::vector<WalkRun> walk_runs(const float* planes /* 3 x (n+1) */, int n);
+// every cell of the run has, in every column across the other two axes, the list of the run's first cell (same length, same entries)
+bool walk_run_collapses(const uint32_t* gridStart, const uint32_t* gridList, int n, const WalkRun& r);
+// kept cells per axis -> map (3 x n, -1 past each extent); returns the cells removed per axis, packed (SceneView::walkTrim)
+uint32_t walk_cell_map(int n, const std::vector<WalkRun>& runs, const std::vector<uint8_t>& collapses, std::vector<int32_t>& map);
+void walk_planes(const float* planes, int n, const int32_t* map, float* out /* 3 x (n+1) */);
+bool pack_walk_grid(const HostScene& h, const PackedGrid& ref, PackedGrid& walk, std::string& err);
 // super-brick level of the three-level walk (rt_walk.h): records appended to the brick array, flags in the empty bricks' .w
 int super_bricks_per_axis(int n);   // n / 16 for power-of-two grids of >= 32 cells per axis, else 0 (no super-brick level)
 size_t super_brick_records(int n);  // records behind the nb^3 brick records (super-brick records sit at the brick strides)

@@ -105,33 +105,23 @@ void pack_triangles(const HostScene& h, float4* geo, float4* shade, int threads)
     for (auto& t : pool) t.join();
 }
 
-// CSR over n^3 cells  ->  4x4x4 bricks {mask, rank base} + ranges of the non-empty cells + list in brick-major order.
-bool pack_grid(const HostScene& h, PackedGrid& out, std::string& err) {
-    const int n = h.axesDivCount;
+// Bricks {mask, rank base}, ranges and face masks of the cells of a grid over the reference CSR.  map == nullptr: the reference grid.
+// Otherwise a walk grid (rt_types.h): walk cell j of axis a stands for reference cell map[a * n + j] (-1: past the axis' extent, no
+// cell); face masks are taken against the neighbour in the walk grid.  Same order and arithmetic as the device packers (pack_kernels.cuh).
+static bool pack_cells(const HostScene& h, int n, const int32_t* map, PackedGrid& out, std::string& err) {
     const int nb = n >= 4 ? n / 4 : 1;
-    const size_t cells = (size_t)n * n * n;
-    const uint32_t total = h.gridStart[cells];
-    if (total && !h.gridList) {
-        err = "scenePixelTriangleList missing";
-        return false;
-    }
-    out.n = n;
-    out.nb = nb;
-    out.planes.resize(3 * (size_t)(n + 1));
-    for (int i = 0; i <= n; ++i) {
-        out.planes[i] = h.boxMin[i].x;
-        out.planes[(n + 1) + i] = h.boxMin[i].y;
-        out.planes[2 * (n + 1) + i] = h.boxMin[i].z;
-    }
+    const uint32_t total = h.gridStart[(size_t)n * n * n];
+    auto ref_id = [&](const int c[3]) -> long long {   // reference cell id of a cell of this grid, or -1
+        int q[3] = {c[0], c[1], c[2]};
+        for (int a = 0; a < 3; ++a) {
+            if (q[a] < 0 || q[a] >= n) return -1;
+            if (map && (q[a] = map[a * n + q[a]]) < 0) return -1;
+        }
+        return (long long)q[0] + (long long)n * q[1] + (long long)n * n * q[2];
+    };
     out.bricks.assign((size_t)nb * nb * nb, make_uint4(0, 0, 0, 0));
     out.cellRange.clear();
     out.faceMask.clear();
-    out.cellList.assign(h.gridList, h.gridList + total);   // list kept in the reference's order; ranges point into it
-    for (uint32_t k = 0; k < total; ++k)
-        if (out.cellList[k] >= h.triangleCount) {
-            err = "scenePixelTriangleList entry out of range";
-            return false;
-        }
     const int side = n >= 4 ? 4 : n;
     for (int bz = 0; bz < nb; ++bz)
         for (int by = 0; by < nb; ++by)
@@ -141,7 +131,9 @@ bool pack_grid(const HostScene& h, PackedGrid& out, std::string& err) {
                 for (int z = 0; z < side; ++z)
                     for (int y = 0; y < side; ++y)
                         for (int x = 0; x < side; ++x) {
-                            const size_t id = (size_t)(bx * 4 + x) + (size_t)n * (by * 4 + y) + (size_t)n * n * (bz * 4 + z);
+                            const int c[3] = {bx * 4 + x, by * 4 + y, bz * 4 + z};
+                            const long long id = ref_id(c);
+                            if (id < 0) continue;
                             const uint32_t s = h.gridStart[id], e = h.gridStart[id + 1];
                             if (e < s || e > total) {
                                 err = "scenePixelTriangleListStart is not a monotone CSR";
@@ -150,13 +142,12 @@ bool pack_grid(const HostScene& h, PackedGrid& out, std::string& err) {
                             if (s < e) {
                                 mask |= 1ull << (x | (y << 2) | (z << 4));
                                 out.cellRange.push_back(make_uint2(s, e));
-                                const int c[3] = {bx * 4 + x, by * 4 + y, bz * 4 + z};
                                 for (int face = 0; face < 6; ++face) {  // face = axis*2 + (entered moving towards +axis)
                                     int q[3] = {c[0], c[1], c[2]};
                                     q[face >> 1] += (face & 1) ? -1 : 1;  // the cell the walk came from
                                     uint32_t m = 0xFFFFFFFFu;
-                                    if (q[face >> 1] >= 0 && q[face >> 1] < n) {
-                                        const size_t nid = (size_t)q[0] + (size_t)n * q[1] + (size_t)n * n * q[2];
+                                    const long long nid = ref_id(q);
+                                    if (nid >= 0) {
                                         const uint32_t ns = h.gridStart[nid], ne = h.gridStart[nid + 1];
                                         for (uint32_t k = 0; k < 32 && s + k < e; ++k) {
                                             bool found = false;
@@ -175,8 +166,129 @@ bool pack_grid(const HostScene& h, PackedGrid& out, std::string& err) {
         out.cellRange.push_back(make_uint2(0, 0));
         out.faceMask.assign(6, 0xFFFFFFFFu);
     }
+    return true;
+}
+
+// CSR over n^3 cells  ->  4x4x4 bricks {mask, rank base} + ranges of the non-empty cells + list in brick-major order.
+bool pack_grid(const HostScene& h, PackedGrid& out, std::string& err) {
+    const int n = h.axesDivCount;
+    const int nb = n >= 4 ? n / 4 : 1;
+    const size_t cells = (size_t)n * n * n;
+    const uint32_t total = h.gridStart[cells];
+    if (total && !h.gridList) {
+        err = "scenePixelTriangleList missing";
+        return false;
+    }
+    out.n = n;
+    out.nb = nb;
+    out.planes.resize(3 * (size_t)(n + 1));
+    for (int i = 0; i <= n; ++i) {
+        out.planes[i] = h.boxMin[i].x;
+        out.planes[(n + 1) + i] = h.boxMin[i].y;
+        out.planes[2 * (n + 1) + i] = h.boxMin[i].z;
+    }
+    out.cellList.assign(h.gridList, h.gridList + total);   // list kept in the reference's order; ranges point into it
+    for (uint32_t k = 0; k < total; ++k)
+        if (out.cellList[k] >= h.triangleCount) {
+            err = "scenePixelTriangleList entry out of range";
+            return false;
+        }
+    if (!pack_cells(h, n, nullptr, out, err)) return false;
     append_super_bricks(out.bricks, n, nb, super_policy(0));   // (the production kernel has no super-brick level: nothing is appended unless asked)
     return true;
+}
+
+// ---- walk grid (rt_types.h) -----------------------------------------------------------------------------------------------------
+std::vector<WalkRun> walk_runs(const float* planes, int n) {
+    std::vector<WalkRun> runs;
+    if (n < 4) return runs;   // (no brick level to keep the extent a multiple of 4 for; nothing worth collapsing)
+    for (int a = 0; a < 3; ++a) {
+        const float* p = planes + (size_t)a * (n + 1);
+        for (int c = 0; c < n;) {
+            int e = c;
+            while (e < n && p[e] == p[e + 1]) ++e;   // cells c .. e-1 have zero width
+            if (e - c >= 2) runs.push_back({a, c, e - c});
+            c = e > c ? e : c + 1;
+        }
+    }
+    return runs;
+}
+
+bool walk_run_collapses(const uint32_t* start, const uint32_t* list, int n, const WalkRun& r) {
+    const size_t stride[3] = {1, (size_t)n, (size_t)n * n};
+    const uint32_t total = start[(size_t)n * n * n];
+    const int u = r.axis == 0 ? 1 : 0, v = r.axis == 2 ? 1 : 2;   // the other two axes
+    for (int j = 0; j < n; ++j)
+        for (int i = 0; i < n; ++i) {
+            const size_t first = (size_t)r.first * stride[r.axis] + (size_t)i * stride[u] + (size_t)j * stride[v];
+            const uint32_t s0 = start[first], len = start[first + 1] - s0;
+            if (start[first + 1] < s0 || start[first + 1] > total) return false;   // (as run_check_kernel: no entry of a bad range is read)
+            for (int k = 1; k < r.count; ++k) {
+                const size_t id = first + (size_t)k * stride[r.axis];
+                const uint32_t s = start[id];
+                if (start[id + 1] < s || start[id + 1] > total || start[id + 1] - s != len) return false;
+                for (uint32_t q = 0; q < len; ++q)
+                    if (list[s + q] != list[s0 + q]) return false;
+            }
+        }
+    return true;
+}
+
+uint32_t walk_cell_map(int n, const std::vector<WalkRun>& runs, const std::vector<uint8_t>& collapses, std::vector<int32_t>& map) {
+    std::vector<uint8_t> keep(3 * (size_t)n, 1);
+    int removed[3] = {0, 0, 0};
+    for (size_t i = 0; i < runs.size(); ++i)
+        if (collapses[i]) {
+            const WalkRun& r = runs[i];
+            for (int k = 1; k < r.count; ++k) keep[(size_t)r.axis * n + r.first + k] = 0;
+            removed[r.axis] += r.count - 1;
+        }
+    // extent up to a multiple of 4 (n is one): cells of collapsed runs kept again, in run order -- each only revisits its run's list
+    for (size_t i = 0; i < runs.size(); ++i) {
+        const WalkRun& r = runs[i];
+        for (int k = 1; collapses[i] && k < r.count && removed[r.axis] % 4 != 0; ++k) {
+            keep[(size_t)r.axis * n + r.first + k] = 1;
+            removed[r.axis] -= 1;
+        }
+    }
+    map.assign(3 * (size_t)n, -1);
+    for (int a = 0; a < 3; ++a) {
+        int m = 0;
+        for (int c = 0; c < n; ++c)
+            if (keep[(size_t)a * n + c]) map[(size_t)a * n + m++] = c;
+    }
+    return pk_make(removed[0], removed[1], removed[2]);
+}
+
+void walk_planes(const float* planes, int n, const int32_t* map, float* out) {
+    for (int a = 0; a < 3; ++a) {
+        const float* p = planes + (size_t)a * (n + 1);
+        float* w = out + (size_t)a * (n + 1);
+        int j = 0;
+        for (; j < n && map[a * n + j] >= 0; ++j) w[j] = p[map[a * n + j]];   // lower plane of the kept cell
+        for (; j <= n; ++j) w[j] = p[n];   // the extent's upper plane, repeated up to the plane stride
+    }
+}
+
+bool pack_walk_grid(const HostScene& h, const PackedGrid& ref, PackedGrid& walk, std::string& err) {
+    const int n = ref.n;
+    const std::vector<WalkRun> runs = walk_runs(ref.planes.data(), n);
+    std::vector<uint8_t> collapses(runs.size());
+    bool any = false;
+    for (size_t i = 0; i < runs.size(); ++i) any |= (collapses[i] = walk_run_collapses(h.gridStart, h.gridList, n, runs[i]) ? 1 : 0) != 0;
+    walk = PackedGrid();
+    if (!any) return true;
+    const uint32_t trim = walk_cell_map(n, runs, collapses, walk.cellMap);
+    if (!trim) {   // the padding kept every cell again (a run of < 4 cells on a small grid): nothing to walk faster
+        walk = PackedGrid();
+        return true;
+    }
+    walk.n = n;
+    walk.nb = ref.nb;
+    walk.walkTrim = trim;
+    walk.planes.resize(ref.planes.size());
+    walk_planes(ref.planes.data(), n, walk.cellMap.data(), walk.planes.data());
+    return pack_cells(h, n, walk.cellMap.data(), walk, err);
 }
 
 // Super-brick level of the three-level walk (rt_walk.h).  Behind the nb^3 brick records: the record {non-empty, 0, 0, 0} of super-brick
